@@ -2,13 +2,19 @@
 """bench.py — MVOC composition hot path on B200: video frames/s of the 50-step DDIM composition.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl mvoc|reference] [--workload config2]
+                    [--dump-outputs DIR]
 
 One "step" = one DDIM composition step (latent fusion + concat, one UNet forward over
 [bg, obj_1..obj_n, uncond, cond], CFG + DDIM update) of BASELINE.json configs[1]:
 full i2vgen-xl-architecture UNet (random init), 16 frames x 64x64 latents (512x512 px), bg + 2 objects,
 boat_surf injection schedule.  The timed region starts at step 0 of the schedule (fusion step, conv
-injection on the first 10 % of the steps) and runs K steps; with K = 50 (default) it is the whole run.
+injection on the first 10 % of the steps) and runs K steps; with K = 50 (default) it is the whole run, and a
+larger K starts the schedule again from the initial latents.
 value = n_frames / (50 * mean step time).
+
+--dump-outputs DIR writes the latents of the timed region's last step as DIR/latents.npy (float32; the inversion
+workloads write DIR/latents_video<v>.npy per video); the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 
 Prints ONE JSON line (see README / DESIGN.md §Measurement for every key).
 """
@@ -145,6 +151,42 @@ def workload_description(wl) -> str:
             f"spatial/temporal attn injection {wl.pnp_spatial_attn_t}/{wl.pnp_temp_attn_t}")
 
 
+def schedule_passes(steps: int, schedule_len: int) -> list:
+    """Step counts of the passes over a schedule of `schedule_len` steps that make `steps` steps in all.  A count
+    past the end of the schedule starts it again from the initial latents, so --steps is the number of steps timed
+    whatever the length of the schedule."""
+    full, rest = divmod(steps, schedule_len)
+    return [schedule_len] * full + ([rest] if rest else [])
+
+
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def _dump_dtype(t):
+    import torch
+
+    return torch.float64 if t.dtype == torch.float64 else torch.float32
+
+
+def check_dump_size(arrays: dict) -> None:
+    """Refuses outputs of more than DUMP_LIMIT_BYTES.  The benchmark also calls it before the warm-up, with tensors
+    of the outputs' shapes and dtypes (the initial latents), so that an oversized dump fails before any step runs."""
+    total = sum(t.numel() * _dump_dtype(t).itemsize for t in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+
+
+def dump_outputs(outdir: str, arrays: dict) -> None:
+    """--dump-outputs: every tensor as <outdir>/<name>.npy, float64 kept and any other dtype as float32, so that
+    two builds of the project can be compared output for output on the same seeded inputs."""
+    import numpy as np
+
+    check_dump_size(arrays)
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), t.detach().to("cpu", _dump_dtype(t)).numpy())
+
+
 def dist_env():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -279,6 +321,8 @@ def run_mvoc(args):
         return run_inversion(args, wl, par, dev, rank, world, local)
     sched = DDIMSchedule(wl.n_steps)
     inputs = synthetic.make_inputs(wl, sched.timesteps, sched.alphas_cumprod)
+    if args.dump_outputs:
+        check_dump_size({"latents": inputs["init_latents"]})
     torch.backends.cudnn.benchmark = True
     unet = build_unet(wl.unet, seed=0, device=dev)
     pipe = I2VGenXLPipeline(unet, dev, parallel=par, use_cuda_graphs=not args.no_graphs)
@@ -297,12 +341,17 @@ def run_mvoc(args):
             random_noise_ratio=wl.random_noise_ratio, obj_random_noise_fusion=wl.obj_random_noise_fusion,
             start_step=start, max_steps=steps, host_io=host_io)
 
+    def run(steps, host_io=False):
+        lat = None
+        for n in schedule_passes(steps, wl.n_steps - wl.ddim_init_latents_t_idx):
+            lat = loop(0, n, host_io)
+        return lat
+
     K, W = args.steps, max(args.warmup, 0)
-    K = min(K, wl.n_steps)
     # warm-up: W steps from the start of the schedule, plus one step of every other hook configuration that
     # occurs in the timed range, so that cuDNN autotuning and CUDA-graph capture happen outside the timing
     if W > 0:
-        loop(0, min(W, wl.n_steps))
+        run(W)
     for i in pipe.step_kinds(sched.timesteps[:K], masks):
         if i >= W:
             loop(i, 1)
@@ -320,7 +369,7 @@ def run_mvoc(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.nvtx.range_push("mvoc_timed_region")   # `ncu --nvtx --nvtx-include "mvoc_timed_region/"`
     ev0.record()
-    final = loop(0, K)
+    final = run(K)
     ev1.record()
     barrier()
     torch.cuda.nvtx.range_pop()
@@ -334,7 +383,7 @@ def run_mvoc(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_wall0 = time.perf_counter()
     e0.record()
-    final_e2e = loop(0, K, host_io=True)
+    final_e2e = run(K, host_io=True)
     e1.record()
     barrier()
     wall_ms = (time.perf_counter() - t_wall0) * 1e3
@@ -354,7 +403,7 @@ def run_mvoc(args):
     ops.set_timer(timer)
     k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     k0.record()
-    loop(0, K)
+    run(K)
     k1.record()
     barrier()
     ops.set_timer(None)
@@ -523,6 +572,8 @@ def run_mvoc(args):
         line["parity"] = parity
     print(json.dumps(line))
     sys.stdout.flush()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latents": final})   # every rank holds all frames of the latents
     _finish(pipe, par)
     if parity is not None and not parity["ok"]:
         raise SystemExit(f"multi-rank parity failed: rel L2 {parity['rel_l2_vs_n1']:.3e} > {PARITY_BAR}")
@@ -550,18 +601,21 @@ def run_inversion(args, wl, par, dev, rank, world, local):
         inv = synthetic.make_inversion_inputs(wl, v)
         pe, ie, il, fps = bf(inv["prompt_embeds"]), bf(inv["image_embeddings"]), bf(inv["image_latents"]), inv["fps"].to(dev)
         vids.append((inv["latents"].to(dev), pe, ie, il, fps, Conditioning(pe, ie, il, il, fps)))
-    K, W = min(args.steps, wl.inversion_steps), max(args.warmup, 0)
+    if args.dump_outputs:
+        check_dump_size({f"latents_video{v}": vid[0] for v, vid in zip(mine, vids)})
+    K, W = args.steps, max(args.warmup, 0)
 
     pinned = [torch.empty(v[0].shape, dtype=v[0].dtype).pin_memory() for v in vids]   # once, outside the timing
 
     def steps(n, host_io=False):
-        out = None
+        outs = []
         for (lat, pe, ie, il, fps, cond), host in zip(vids, pinned):
-            x = host.copy_(lat.cpu()).to(dev, non_blocking=True) if host_io else lat.clone()
-            pipe.invert(x, pe, ie, il, fps, num_inference_steps=wl.inversion_steps, max_steps=n, keep=False, cond=cond,
-                        on_step=(lambda t, z: host.copy_(z, non_blocking=False)) if host_io else None)
-            out = x
-        return out
+            for m in schedule_passes(n, wl.inversion_steps):
+                x = host.copy_(lat.cpu()).to(dev, non_blocking=True) if host_io else lat.clone()
+                pipe.invert(x, pe, ie, il, fps, num_inference_steps=wl.inversion_steps, max_steps=m, keep=False,
+                            cond=cond, on_step=(lambda t, z: host.copy_(z, non_blocking=False)) if host_io else None)
+            outs.append(x)
+        return outs
 
     if W > 0:
         steps(W)
@@ -578,7 +632,7 @@ def run_inversion(args, wl, par, dev, rank, world, local):
         clocks.start()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
-    steps(K)
+    outs = steps(K)
     ev1.record()
     barrier()
     clk = clocks.stop() if rank == 0 else None
@@ -616,6 +670,8 @@ def run_inversion(args, wl, par, dev, rank, world, local):
         }
         print(json.dumps(line))
         sys.stdout.flush()
+    if args.dump_outputs:      # every rank writes the videos it inverted
+        dump_outputs(args.dump_outputs, {f"latents_video{v}": x for v, x in zip(mine, outs)})
     _finish(pipe, par)
 
 
@@ -641,16 +697,28 @@ def _finish(pipe, par):
         par.shutdown()
 
 
+def positive_int(text: str) -> int:
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, not {v}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=positive_int, default=50,
+                    help="timed steps; past the end of the schedule it starts again from the initial latents")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="mvoc", choices=["mvoc", "reference"])
     ap.add_argument("--workload", default="config2")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graphs", action="store_true", help="launch every kernel from Python instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the latents they computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the CUDA path computes; --impl reference times a reduced CPU sample")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -26,6 +26,7 @@ from __future__ import annotations
 import importlib.util
 import logging
 import os
+import shutil
 import sys
 import types
 from types import SimpleNamespace
@@ -179,6 +180,12 @@ def main():
     torch.save(lat.detach().clone(), os.path.join(d, f"ddim_latents_{torch.tensor(981)}.pt"))
     back = ref_utils.load_ddim_latents_at_t(torch.tensor(981), d)
     assert torch.equal(back, lat)
+
+    # the reference's own config files, byte for byte (a few KB): the config loader is tested on them
+    for sub in ("group_composite", "group_inversion"):
+        os.makedirs(os.path.join(HERE, "reference_configs", sub), exist_ok=True)
+        for name in ("template.yaml", "group_config.json"):
+            shutil.copyfile(os.path.join(REF, "configs", sub, name), os.path.join(HERE, "reference_configs", sub, name))
     print("wrote goldens")
 
 

@@ -1,4 +1,5 @@
 """CPU-side tests: C-ABI surface, host logic (scheduler, config, injection sites), oracle unit pins."""
+import argparse
 import ctypes
 import json
 import os
@@ -433,10 +434,11 @@ def test_latent_bank_and_wire_format(tmp_path):
 
 
 # ------------------------------------------------------------------ script / config contract
-REF_CFG = "/root/reference/i2vgen-xl/configs"
+REF_CFG = os.path.join(ROOT, "tests", "golden", "reference_configs")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference configs only exist in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="the reference's config files are not stored under "
+                    "tests/golden/reference_configs (tests/golden/make_golden.py copies them from a reference checkout)")
 def test_reference_config_files_load_unchanged():
     """The reference's own template.yaml + group_config.json go through the loader and the path joins of
     composite.py:97-106 / inverse.py:143-150 without edits."""
@@ -459,6 +461,40 @@ def test_reference_config_files_load_unchanged():
     assert inv and inv[0].inverse_config.n_steps == 500 and inv[0].inverse_config.cfg == 1.0
     assert inv[0].inverse_config.image_size == [1280, 720]          # ${image_size} keeps the list type
     assert inv[0].inverse_config.output_dir == "../inversions/i2vgen-xl/boat_surf/ddim_latents"
+    assert inv[0].recon_config.ddim_latents_path == inv[0].inverse_config.output_dir
+
+
+CFG = os.path.join(ROOT, "configs")
+
+
+def test_shipped_config_files_load():
+    """The template.yaml + group_config.json pairs under configs/ (the CLI defaults) go through the loader and the
+    path joins of composite.py:97-106 / inverse.py:143-150 without edits."""
+    from mvoc_b200 import composite, config as cfgmod
+
+    entries = list(cfgmod.iter_configs(f"{CFG}/group_composite/template.yaml",
+                                       f"{CFG}/group_composite/group_config.json"))
+    assert len(entries) == 1                                        # the inactive entry is dropped
+    c = composite.resolve_paths(entries[0])
+    j = lambda *p: os.path.join(c.data_dir, *p)
+    assert c.video_name == "synthetic_small" and c.image_size == [256, 128]
+    assert c.obj_mask_path == [j("demo/synthetic_small/obj1_mask"), j("demo/synthetic_small/obj2_mask")]
+    assert c.obj_ddim_latents_path == [j("inversions/i2vgen-xl/obj1/ddim_latents"),
+                                       j("inversions/i2vgen-xl/obj2/ddim_latents")]
+    assert c.bg_ddim_latents_path == j("inversions/i2vgen-xl/synthetic_small/ddim_latents")
+    assert c.edited_first_frame_path == j("demo/synthetic_small/edited_first_frame/00000.png")
+    assert c.video_path == j("demo", "synthetic_small.mp4")
+    assert c.output_dir == f"{c.data_dir}/Results/MVOC-B200/i2vgen-xl/synthetic_small/bg plus two objects/"
+    assert composite.latent_geometry(c) == (8, 16, 32)
+    assert (c.pnp_f_t, c.pnp_spatial_attn_t, c.pnp_temp_attn_t, c.fusion_step) == (0.1, 1.0, 1.0, [0, 1])
+    assert (c.n_steps, c.cfg, c.ddim_init_latents_t_idx, c.random_noise_ratio) == (50, 9.0, 0, 0.0)
+    inv = list(cfgmod.iter_configs(f"{CFG}/group_inversion/template.yaml",
+                                   f"{CFG}/group_inversion/group_config.json"))
+    assert len(inv) == 1 and inv[0].video_name == "synthetic_small"
+    assert inv[0].inverse_config.n_steps == 500 and inv[0].inverse_config.cfg == 1.0
+    assert inv[0].inverse_config.image_size == [256, 128]           # ${image_size} keeps the list type
+    assert inv[0].inverse_config.n_frames == 8                      # the entry's override reaches the nested key
+    assert inv[0].inverse_config.output_dir == f"{inv[0].data_dir}/inversions/i2vgen-xl/synthetic_small/ddim_latents"
     assert inv[0].recon_config.ddim_latents_path == inv[0].inverse_config.output_dir
 
 
@@ -534,6 +570,35 @@ def test_bench_reference_arm_contract(monkeypatch, capsys):
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] == 4
     assert line["e2e"] == {"value": pytest.approx(0.002), "unit": "frames/s", "h2d_bytes_per_step": 0,
                            "d2h_bytes_per_step": 0}
+
+
+def test_bench_steps_past_the_schedule_start_it_again():
+    import bench
+
+    assert bench.schedule_passes(3, 50) == [3]
+    assert bench.schedule_passes(50, 50) == [50]
+    assert bench.schedule_passes(120, 50) == [50, 50, 20]
+    assert sum(bench.schedule_passes(1001, 500)) == 1001
+    assert bench.positive_int("1") == 1
+    with pytest.raises(argparse.ArgumentTypeError):
+        bench.positive_int("0")
+
+
+def test_bench_dump_outputs(tmp_path):
+    import numpy as np
+
+    import bench
+
+    lat = torch.randn(1, 4, 2, 8, 8)
+    bench.dump_outputs(str(tmp_path / "out"), {"latents": lat.bfloat16(), "exact": lat.double()})
+    a = np.load(tmp_path / "out" / "latents.npy")
+    b = np.load(tmp_path / "out" / "exact.npy")
+    assert a.dtype == np.float32 and a.shape == (1, 4, 2, 8, 8)
+    assert np.array_equal(a, lat.bfloat16().float().numpy())
+    assert b.dtype == np.float64 and np.array_equal(b, lat.double().numpy())
+    with pytest.raises(SystemExit, match="limit"):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": torch.empty(bench.DUMP_LIMIT_BYTES // 4 + 1)})
+    assert not (tmp_path / "big").exists()
 
 
 # ------------------------------------------------------------------ round-2 advisor findings

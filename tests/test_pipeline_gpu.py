@@ -6,6 +6,7 @@ oracle's own module tree in bf16 on the GPU (torch SDPA / ATen GroupNorm); the p
 1.5x of that envelope (plus a small absolute floor).
 """
 import copy
+import os
 from types import SimpleNamespace
 
 import pytest
@@ -207,3 +208,33 @@ def test_unet_forward_vs_reference_golden(cuda_device, case_name):
     comp = rel_l2(out[3:], ref[3:])
     print(f"[golden {case_name}] rel L2 all {err:.4e}, composite branches {comp:.4e}")
     assert err <= 3e-2 and comp <= 3e-2
+
+
+def test_bench_steps_and_dump_outputs(cuda_device, tmp_path, monkeypatch, capsys):
+    """bench.py --steps K times exactly K steps: past the end of the schedule (47 steps here, it starts at index 3)
+    it starts again from the initial latents, so 48 steps end where 1 step does.  --dump-outputs writes those
+    latents after the JSON line."""
+    import dataclasses
+    import json
+    import sys
+
+    import numpy as np
+
+    import bench
+    from mvoc_b200 import synthetic
+
+    wl = dataclasses.replace(synthetic.WORKLOADS["config1"], name="config1_from_idx3", ddim_init_latents_t_idx=3)
+    monkeypatch.setitem(synthetic.WORKLOADS, wl.name, wl)
+    monkeypatch.setattr(torch.backends.cudnn, "benchmark", torch.backends.cudnn.benchmark)   # restored afterwards
+    out = {}
+    for k in (1, 48):
+        d = tmp_path / f"k{k}"
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--workload", wl.name, "--steps", str(k), "--warmup", "1",
+                                          "--no-cpu-baseline", "--dump-outputs", str(d)])
+        bench.main()
+        line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+        assert line["steps"] == k
+        assert sorted(os.listdir(d)) == ["latents.npy"]
+        out[k] = np.load(d / "latents.npy")
+    assert out[1].dtype == np.float32 and out[1].shape == (1, 4, wl.n_frames, wl.latent_h, wl.latent_w)
+    assert rel_l2(torch.from_numpy(out[48]), torch.from_numpy(out[1])) <= 1e-3
