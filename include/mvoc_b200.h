@@ -107,6 +107,22 @@ int mvoc_attn_fwd_trace(const void* q, const void* k, const void* v, void* o, in
                         long long* trace, void* stream);
 
 /*
+ * Single-head attention of width 512, O = softmax(Q K^T * scale) V.
+ * Replaces the mid-block Attention of the AutoencoderKL decoder (one head over the 512 channels of the latent-
+ * resolution map, diffusers' Attention with group_norm and residual_connection), reached from decode_latents,
+ * i2vgen-xl/pipelines/pipeline_i2vgen_xl.py:771-791.
+ *
+ * q,k,v,o: [B, N, D], D == 512 innermost and contiguous; strides in ELEMENTS for (batch, token), so q/k/v may be
+ * the three column slices of one fused QKV projection output [B*N, 1536].  Any N >= 1 (no multiple of 128 needed).
+ * Tensor-core path (tcgen05.mma, accumulators in TMEM, operands staged by TMA); bf16 or fp16 (P is rounded to the
+ * storage type).  Requirements: base pointers 16-byte aligned, strides non-negative multiples of 8.
+ */
+int mvoc_attn_d512_fwd(const void* q, const void* k, const void* v, void* o, int B, int N, int D,
+                       int64_t q_sb, int64_t q_sn, int64_t k_sb, int64_t k_sn,
+                       int64_t v_sb, int64_t v_sn, int64_t o_sb, int64_t o_sn,
+                       float scale, int dtype, void* stream);
+
+/*
  * Short-sequence attention (tokens = frames), one warp per (pixel, head).
  * Replaces F.scaled_dot_product_attention at i2vgen-xl/pnp_utils.py:862-864
  * (injected temporal attn1) and the stock processor on the temporal attn2,

@@ -38,6 +38,8 @@ SIGNATURES = {
     ),
     "mvoc_attn_fwd_trace": (
         c_int, [c_void_p] * 4 + [c_int] * 5 + [ctypes.POINTER(c_int64), c_int, c_float, c_int, c_int, c_void_p, c_void_p]),
+    "mvoc_attn_d512_fwd": (
+        c_int, [c_void_p] * 4 + [c_int] * 3 + [c_int64] * 8 + [c_float, c_int, c_void_p]),
     "mvoc_attn_temporal_fwd": (
         c_int,
         [c_void_p] * 4 + [c_int64, c_int, c_int, c_int] + [c_int64] * 12 + [c_float, c_int, c_void_p],

@@ -10,7 +10,7 @@ masks (utils.mask_preprocess) and runs the 50-step composition loop
 (pipelines/pipeline_i2vgen_xl.py:1636-1734) on the GPU.  The final latents are written to
 `<output_dir>/composite_latents.pt`.
 
-Out of scope here (SURVEY §2 #9, #10): CLIP / VAE.  The tensors those stages produce are read from
+Out of scope here (SURVEY §2 #9, #10): CLIP / VAE encode.  The tensors those stages produce are read from
 `--conditioning file.pt` (a dict with prompt_embeds [n+3,77,1024], image_embeddings [n+3,T,1024],
 image_latents_first / image_latents [n+3,4,T,h,w]); the path may contain `{video_name}` / `{edited_video_name}`
 so that every config entry gets its own file.  Missing inverted latents, masks or conditioning are ERRORS, like
@@ -18,6 +18,11 @@ the reference's asserts (utils.py:34, composite.py:246).  Only with `--synthetic
 of the right shape substituted (mvoc_b200.synthetic) — the offline end-to-end exercise of the config → hooks →
 loop path; the output is then written as `composite_latents.synthetic.pt`.  UNet weights come from
 `--unet_state_dict` (a diffusers I2VGenXLUNet state dict) or, with `--synthetic`, are random-initialised.
+
+With `--vae_state_dict` (a diffusers AutoencoderKL state dict, .safetensors or a torch file) the final latents are
+also decoded (decode_latents, pipelines/pipeline_i2vgen_xl.py:771-791) and written as one PNG per frame to
+`<output_dir>/composite_frames/` (`composite_frames.synthetic/` under `--synthetic`).  `--synthetic` never invents
+decoder weights: without the flag nothing is decoded.
 """
 from __future__ import annotations
 
@@ -123,9 +128,10 @@ def run_entry(pipe, config, device, conditioning=None, allow_synthetic: bool = F
 
 
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, conditioning: str = None,
-         device: str = None, max_entries: int = None, synthetic_inputs: bool = False):
+         device: str = None, max_entries: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None):
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
+    from .vae import load_vae_decoder, save_frames
 
     template = cfgmod.load_template(template_config)
     device = torch.device(device or template.get("device", "cuda:0"))
@@ -138,7 +144,8 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
     elif not synthetic_inputs:
         raise FileNotFoundError("--unet_state_dict is required (pass --synthetic to run on random-init weights)")
     unet = prepare(unet.to(device=device, dtype=torch.bfloat16))
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True)
+    vae = load_vae_decoder(vae_state_dict, device) if vae_state_dict else None
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae=vae)
     done = 0
     for config in cfgmod.iter_configs(template_config, configs_json):
         config = resolve_paths(config)
@@ -155,6 +162,11 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
                            "composite_latents.synthetic.pt" if synthetic_inputs else "composite_latents.pt")
         torch.save(latents.detach().cpu(), out)
         logger.info("saved %s", out)
+        if vae is not None:
+            frames_dir = os.path.join(config.output_dir,
+                                      "composite_frames.synthetic" if synthetic_inputs else "composite_frames")
+            save_frames(pipe.decode_latents(latents)[0], frames_dir)
+            logger.info("saved %s", frames_dir)
         done += 1
         if max_entries is not None and done >= max_entries:
             break
@@ -167,6 +179,8 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--configs_json", type=str, default="./configs/group_composite/group_config.json")
     ap.add_argument("--unet_state_dict", type=str, default=None)
     ap.add_argument("--conditioning", type=str, default=None)
+    ap.add_argument("--vae_state_dict", type=str, default=None,
+                    help="diffusers AutoencoderKL state dict: also decode the latents and write PNG frames")
     ap.add_argument("--device", type=str, default=None)
     ap.add_argument("--max_entries", type=int, default=None)
     ap.add_argument("--synthetic", action="store_true",
@@ -179,4 +193,4 @@ if __name__ == "__main__":
     logging.basicConfig(level=logging.INFO)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # composite.py:246
     main(args.template_config, args.configs_json, args.unet_state_dict, args.conditioning, args.device,
-         args.max_entries, args.synthetic)
+         args.max_entries, args.synthetic, args.vae_state_dict)

@@ -153,6 +153,38 @@ def attention(
     return out
 
 
+WIDE_HEAD_DIM = 512
+
+
+def _bn_strides(t: torch.Tensor, what: str, B: int, N: int):
+    """(batch, token) element strides of a [B, N, 512] tensor with a contiguous last dim."""
+    if tuple(t.shape) != (B, N, WIDE_HEAD_DIM) or t.stride(-1) != 1:
+        raise ValueError(f"attention_d512: {what} must be [{B}, {N}, {WIDE_HEAD_DIM}] with a contiguous last dim, "
+                         f"got {tuple(t.shape)} strides {t.stride()}")
+    return t.stride(0), t.stride(1)
+
+
+def attention_d512(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: Optional[float] = None,
+                   out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Single-head softmax(Q K^T * scale) V with head_dim 512 (the VAE decoder's mid-block attention):
+    q, k, v [B, N, 512] (any batch / token strides, e.g. column slices of a fused QKV output) -> [B, N, 512]."""
+    _need_cuda(q, k, v, out)
+    if q.dim() != 3:
+        raise ValueError(f"attention_d512: need q, k, v [B, N, 512], got {tuple(q.shape)}")
+    B, N = q.shape[0], q.shape[1]
+    if out is None:
+        out = torch.empty((B, N, WIDE_HEAD_DIM), dtype=q.dtype, device=q.device)
+    st = [s for t, nm in ((q, "q"), (k, "k"), (v, "v"), (out, "out")) for s in _bn_strides(t, nm, B, N)]
+    if scale is None:
+        scale = WIDE_HEAD_DIM ** -0.5
+    with _Timed(("attn_d512", B, N), 4.0 * B * N * N * WIDE_HEAD_DIM):
+        rc = _cabi.load().mvoc_attn_d512_fwd(q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), B, N,
+                                             WIDE_HEAD_DIM, *st, float(scale), _dt(q), _stream())
+    _cabi.check(rc, "mvoc_attn_d512_fwd")
+    _count()
+    return out
+
+
 def temporal_attention(
     q: torch.Tensor,
     k: torch.Tensor,

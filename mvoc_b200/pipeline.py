@@ -98,10 +98,11 @@ class Conditioning:
 
 
 class I2VGenXLPipeline:
-    def __init__(self, unet, device="cuda", parallel=None, use_cuda_graphs: bool = False):
+    def __init__(self, unet, device="cuda", parallel=None, use_cuda_graphs: bool = False, vae=None):
         from .parallel import FrameParallel
 
         self.unet = unet
+        self.vae = vae             # mvoc_b200.vae.AutoencoderKLDecoder for decode_latents, or None
         self.device = torch.device(device)
         self.parallel = parallel or FrameParallel.single(self.device)
         # A UNet forward is ~2700 launches; enqueuing them from Python takes about as long as the GPU needs
@@ -116,6 +117,23 @@ class I2VGenXLPipeline:
         self.scheduler: Optional[DDIMSchedule] = None
         self._cond_caches = {}     # id(cond) -> {"key": cond (strong ref), "ctx", "il", "fps_emb"}; a few conditionings
 
+
+    @torch.no_grad()
+    def decode_latents(self, latents: torch.Tensor, decode_chunk_size: int = 4) -> torch.Tensor:
+        """pipelines/pipeline_i2vgen_xl.py:771-791: latents [b, 4, T, h, w] -> video [b, 3, T, 8h, 8w] fp32, the
+        frames decoded `decode_chunk_size` at a time (which bounds the decoder's activation memory)."""
+        from .vae import SCALING_FACTOR
+
+        if self.vae is None:
+            raise RuntimeError("decode_latents: this pipeline was built without a VAE decoder (vae=None)")
+        if decode_chunk_size < 1:
+            raise ValueError(f"decode_latents: decode_chunk_size={decode_chunk_size} must be >= 1")
+        latents = 1 / SCALING_FACTOR * latents.float()
+        b, c, f, h, w = latents.shape
+        flat = latents.permute(0, 2, 1, 3, 4).reshape(b * f, c, h, w)
+        frames = [self.vae(flat[i:i + decode_chunk_size]) for i in range(0, flat.shape[0], decode_chunk_size)]
+        image = torch.cat(frames, dim=0)
+        return image.reshape((b, f) + image.shape[1:]).permute(0, 2, 1, 3, 4).float()
 
     def drop_graphs(self) -> None:
         """Forget every captured graph.  The private pool goes with them: torch asserts when a capture re-uses a

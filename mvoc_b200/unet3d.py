@@ -437,13 +437,14 @@ class TransformerTemporalModel(nn.Module):
 
 # ------------------------------------------------------------------ conv blocks
 class ResnetBlock2D(nn.Module):
-    """Stock ResnetBlock2D forward == the closure at pnp_utils.py:902-1020 without the injection block."""
+    """Stock ResnetBlock2D forward == the closure at pnp_utils.py:902-1020 without the injection block.
+    temb_channels=None builds the VAE's resnet: no time_emb_proj, called as forward(x, None)."""
 
     def __init__(self, in_channels, out_channels, temb_channels, groups=32, eps=1e-5):
         super().__init__()
         self.norm1 = GroupNormAct(groups, in_channels, eps=eps, affine=True)
         self.conv1 = nn.Conv2d(in_channels, out_channels, 3, padding=1)
-        self.time_emb_proj = nn.Linear(temb_channels, out_channels)
+        self.time_emb_proj = nn.Linear(temb_channels, out_channels) if temb_channels is not None else None
         self.norm2 = GroupNormAct(groups, out_channels, eps=eps, affine=True)
         self.dropout = nn.Dropout(0.0)
         self.conv2 = nn.Conv2d(out_channels, out_channels, 3, padding=1)
@@ -458,7 +459,7 @@ class ResnetBlock2D(nn.Module):
         n, H, W, cin = input_tensor.shape
         h = self.norm1(input_tensor, silu=True)                                 # :909-910
         h = conv_nhwc(h, self.conv1)                                            # :939
-        t = self.time_emb_proj(F.silu(temb))                                    # :941-948
+        t = None if self.time_emb_proj is None else self.time_emb_proj(F.silu(temb))   # :941-948
         h = self.norm2(h, silu=True, add=t, out=h)                              # `+ temb` :952 fused into norm2 :953, :965
         if self.conv_shortcut is None:
             if self.feature_hook is None:
