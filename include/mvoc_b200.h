@@ -66,8 +66,9 @@ int mvoc_device_check(int device);
  * q,o: [B, Nq, H, D]   k,v: [B, Nk, H, D]   D innermost and contiguous, D == 64.
  * Strides are in ELEMENTS for (batch, token, head).  Tensor-core path
  * (tcgen05.mma, accumulators in TMEM, operands staged by TMA); bf16 or fp16 (P is rounded to the storage type).
- * Requirements: base pointers 16-byte aligned, strides non-negative multiples of 8 (a batch stride of 0
- * broadcasts one Q / K / V to every batch).
+ * Requirements: base pointers 16-byte aligned, strides non-negative multiples of 8, and positive along every
+ * dimension of extent > 1 (q, k and v are read through TMA, which cannot broadcast: a zero stride there returns
+ * MVOC_ERR_UNSUPPORTED).
  * variant: 0 = default (currently 4).  1, 2 = all exp2 on the MUFU; 3 / 4 / 5 = 2 / 3 / 4 of every
  *          8 exp2 pairs evaluated by a degree-3 polynomial on the FMA pipe.  Same results up to the exp2
  *          approximation (<= 1e-4 relative, below the 16-bit rounding of P); the tests run all of them.
@@ -86,7 +87,8 @@ int mvoc_attn_fwd(const void* q, const void* k, const void* v, void* o,
  * half the exponentials, which are what bounds a head_dim-64 attention on this chip.
  * This is the structure MVOC creates and the reference ignores: ModifiedSpaAttnProcessor writes the SAME blended
  * Q', K' into the uncond and the cond composite chunk (i2vgen-xl/pnp_utils.py:664-668) and then runs SDPA on
- * both (:684).  q, k: [B, N, H, D]; v, o: [B + pair_batches, N, H, D]; other arguments as mvoc_attn_fwd.
+ * both (:684).  q, k: [B, N, H, D]; v, o: [B + pair_batches, N, H, D]; other arguments and the stride
+ * requirements as mvoc_attn_fwd.
  */
 int mvoc_attn_pair_fwd(const void* q, const void* k, const void* v, void* o,
                        int B, int H, int Nq, int Nk, int D,
@@ -115,7 +117,8 @@ int mvoc_attn_fwd_trace(const void* q, const void* k, const void* v, void* o, in
  * q,k,v,o: [B, N, D], D == 512 innermost and contiguous; strides in ELEMENTS for (batch, token), so q/k/v may be
  * the three column slices of one fused QKV projection output [B*N, 1536].  Any N >= 1 (no multiple of 128 needed).
  * Tensor-core path (tcgen05.mma, accumulators in TMEM, operands staged by TMA); bf16 or fp16 (P is rounded to the
- * storage type).  Requirements: base pointers 16-byte aligned, strides non-negative multiples of 8.
+ * storage type).  Requirements: base pointers 16-byte aligned, strides non-negative multiples of 8, and positive
+ * along every dimension of extent > 1 (a zero q / k / v stride there returns MVOC_ERR_UNSUPPORTED).
  */
 int mvoc_attn_d512_fwd(const void* q, const void* k, const void* v, void* o, int B, int N, int D,
                        int64_t q_sb, int64_t q_sn, int64_t k_sb, int64_t k_sn,

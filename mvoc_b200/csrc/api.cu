@@ -23,6 +23,17 @@ int check_launch(const char* what) {
     return MVOC_OK;
 }
 
+int set_max_dynamic_smem(const void* kernel, int bytes, bool (&done)[64], const char* what) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    const bool tracked = dev >= 0 && dev < 64;
+    if (tracked && done[dev]) return MVOC_OK;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    MVOC_REQUIRE(e == cudaSuccess, MVOC_ERR_CUDA, "%s: cudaFuncSetAttribute: %s", what, cudaGetErrorString(e));
+    if (tracked) done[dev] = true;
+    return MVOC_OK;
+}
+
 }  // namespace mvoc
 
 extern "C" const char* mvoc_version(void) { return "mvoc_b200 0.1.0 (sm_100a)"; }

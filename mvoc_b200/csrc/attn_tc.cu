@@ -70,33 +70,6 @@ __device__ __forceinline__ void trace_at(const Params& prm, int j, int ev) {
     if (prm.trace != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0) prm.trace[j * 8 + ev] = clock64();
 }
 
-template <typename T> struct Pack2;
-template <> struct Pack2<__nv_bfloat16> {
-    static __device__ __forceinline__ uint32_t rn(float lo, float hi) {
-        __nv_bfloat162 b = __floats2bfloat162_rn(lo, hi);
-        return *reinterpret_cast<uint32_t*>(&b);
-    }
-    static __device__ __forceinline__ uint32_t scale(uint32_t v, float f) {   // bf16 = upper half of an fp32
-        return rn(__uint_as_float(v << 16) * f, __uint_as_float(v & 0xffff0000u) * f);
-    }
-};
-template <> struct Pack2<__half> {
-    static __device__ __forceinline__ uint32_t rn(float lo, float hi) {
-        __half2 b = __floats2half2_rn(lo, hi);
-        return *reinterpret_cast<uint32_t*>(&b);
-    }
-    static __device__ __forceinline__ uint32_t scale(uint32_t v, float f) {
-        const float2 x = __half22float2(*reinterpret_cast<__half2*>(&v));
-        return rn(x.x * f, x.y * f);
-    }
-};
-// kind::f16 instruction descriptor for 16-bit storage type T (fp16: format 0, bf16: format 1), fp32 accumulation
-template <typename T> __host__ __device__ constexpr uint32_t idesc_for(int M, int N, int b_mn_major) {
-    return (1u << 4) | ((std::is_same<T, __half>::value ? 0u : 1u) << 7) |
-           ((std::is_same<T, __half>::value ? 0u : 1u) << 10) | ((uint32_t)b_mn_major << 16) |
-           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
 // kEmuMask: bit (k % 8) set => the k-th pair of a score row takes the FMA-pipe exp2 instead of the MUFU.
 template <typename T, int kBN, int kNV, int kStages, uint32_t kEmuMask>
 __global__ void __launch_bounds__(THREADS, 2)
@@ -109,10 +82,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const uint32_t sbase = smem_u32(smem_raw);
     uint8_t* sgen = smem_raw;
-    if ((sbase & 1023u) != 0u) {  // 128-byte-swizzled tiles need a 1024-byte aligned base
-        if (threadIdx.x == 0) printf("mvoc attn_fwd_kernel: dynamic smem base 0x%x is not 1024-byte aligned\n", sbase);
-        __trap();
-    }
+    MVOC_REQUIRE_SMEM_1024(sbase, "attn_fwd_kernel");
 
     const uint32_t sQ = sbase + L::q_off;
     const uint32_t sK = sbase + L::k_off;
@@ -185,8 +155,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
         }
     } else if (warp == 5) {
         // ===================== MMA issuer =====================
-        constexpr uint32_t IDESC_QK = idesc_for<T>(BM, BN, 0);  // A,B K-major
-        constexpr uint32_t IDESC_PV = idesc_for<T>(BM, HD, 1);  // B (=V) MN-major
+        constexpr bool kF16 = std::is_same<T, __half>::value;
+        constexpr uint32_t IDESC_QK = ptx::idesc_f16(kF16, BM, BN, false);  // A,B K-major
+        constexpr uint32_t IDESC_PV = ptx::idesc_f16(kF16, BM, HD, true);   // B (=V) MN-major
         const uint32_t tS = tmem + COL_S, tP = tmem + COL_P, tO = tmem + COL_O;
         auto issue_qk = [&](int j) {
             const int s = j % kStages;
@@ -334,7 +305,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
                 else if ((k & 3) == 1) lb = ptx::add2(lb, p2);
                 else if ((k & 3) == 2) lc = ptx::add2(lc, p2);
                 else ld = ptx::add2(ld, p2);
-                pk[k] = Pack2<T>::rn(p0, p1);
+                pk[k] = pack2_rn<T>(p0, p1);
                 // two thirds through: poll (without blocking) whether the previous P V has completed, so that the wait
                 // in front of the P store costs nothing when it has (an mbarrier wait costs ~130 clocks even then)
                 if (k == (BN / 2) * 2 / 3 && !pv_waited && !pv_ready)
@@ -399,88 +370,47 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
 }
 
 // ------------------------------------------------------------------ host ---
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
-                                  const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres);
-        if (e == cudaSuccess && qres == cudaDriverEntryPointSuccess) fn = (EncodeTiledFn)p;
-    }
-    return fn;
-}
-
-// [B, N, H, 64] 16-bit with element strides (sb, sn, sh); box = `rows` tokens x 64 of one head.
-static int make_map(CUtensorMap* m, const void* base, int dtype, int B, int H, int N, int rows, int64_t sb, int64_t sn,
-                    int64_t sh, const char* what) {
-    EncodeTiledFn fn = get_encode_fn();
-    MVOC_REQUIRE(fn != nullptr, MVOC_ERR_DRIVER, "mvoc_attn_fwd: cuTensorMapEncodeTiled unavailable");
-    cuuint64_t dims[4] = {(cuuint64_t)HD, (cuuint64_t)H, (cuuint64_t)N, (cuuint64_t)B};
-    cuuint64_t strides[3] = {(cuuint64_t)sh * 2, (cuuint64_t)sn * 2, (cuuint64_t)sb * 2};
-    // a size-1 dimension may carry any stride; TMA still wants a non-zero multiple of 16 bytes
-    if (H == 1) strides[0] = 128;
-    if (B == 1 || strides[2] == 0) strides[2] = (cuuint64_t)sn * 2 * (cuuint64_t)N;
-    cuuint32_t box[4] = {(cuuint32_t)HD, 1, (cuuint32_t)rows, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = fn(m, dtype == MVOC_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4,
-                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MVOC_REQUIRE(r == CUDA_SUCCESS, MVOC_ERR_DRIVER,
-                 "mvoc_attn_fwd: cuTensorMapEncodeTiled(%s) failed with CUresult %d "
-                 "(B=%d H=%d N=%d strides=%lld,%lld,%lld)",
-                 what, (int)r, B, H, N, (long long)sb, (long long)sn, (long long)sh);
-    return MVOC_OK;
-}
-
 template <typename T, int kBN, int kNV, int kStages, uint32_t kEmuMask>
-static int launch(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv, const Params& prm, int B, int H,
-                  cudaStream_t s) {
+static int launch(const CUtensorMap (&m)[3], const Params& prm, int B, int H, cudaStream_t s, const char* what) {
     using L = Smem<kBN, kNV, kStages>;
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, L::alloc);
-        MVOC_REQUIRE(e == cudaSuccess, MVOC_ERR_CUDA, "mvoc_attn_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-        attr_set[dev] = true;
-    }
+    static bool smem_set[64] = {false};
+    const int rc = set_max_dynamic_smem((const void*)attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask>, L::alloc,
+                                        smem_set, what);
+    if (rc != MVOC_OK) return rc;
     dim3 grid((prm.Nq + BM - 1) / BM, H, B);
-    attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask><<<grid, THREADS, L::alloc, s>>>(mq, mk, mv, prm);
-    return check_launch("mvoc_attn_fwd");
+    attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask><<<grid, THREADS, L::alloc, s>>>(m[0], m[1], m[2], prm);
+    return check_launch(what);
 }
 
 // Common entry: kNV value tensors per softmax (1 = plain attention, 2 = the uncond/cond pair).
 static int run(const void* q, const void* k, const void* v, void* o, int B, int H, int Nq, int Nk, int D,
                const int64_t (&st)[12], int pair_batches, float scale, int dtype, int variant, void* stream,
                const char* what, long long* trace = nullptr) {
-    MVOC_REQUIRE(q && k && v && o, MVOC_ERR_INVALID_ARG, "%s: null pointer", what);
-    MVOC_REQUIRE(dtype == MVOC_BF16 || dtype == MVOC_F16, MVOC_ERR_UNSUPPORTED, "%s: dtype %d unsupported (bf16 / fp16)",
-                 what, dtype);
-    MVOC_REQUIRE(D == HD, MVOC_ERR_UNSUPPORTED, "%s: head_dim %d unsupported (64 only)", what, D);
+    int rc = check_attn_operands(q, k, v, o, dtype, D, HD, st, 12, what);
+    if (rc != MVOC_OK) return rc;
     MVOC_REQUIRE(B > 0 && H > 0 && Nq > 0 && Nk > 0, MVOC_ERR_INVALID_ARG, "%s: empty problem B=%d H=%d Nq=%d Nk=%d", what,
                  B, H, Nq, Nk);
     MVOC_REQUIRE(B <= 65535 && H <= 65535, MVOC_ERR_UNSUPPORTED, "%s: B=%d / H=%d exceed the grid limits", what, B, H);
     MVOC_REQUIRE(variant >= 0 && variant <= 5, MVOC_ERR_INVALID_ARG, "%s: unknown variant %d", what, variant);
     MVOC_REQUIRE(pair_batches >= 0, MVOC_ERR_INVALID_ARG, "%s: pair_batches=%d", what, pair_batches);
-    for (int i = 0; i < 12; ++i)
-        MVOC_REQUIRE(st[i] % 8 == 0 && st[i] >= 0, MVOC_ERR_UNSUPPORTED,
-                     "%s: stride #%d = %lld is not a non-negative multiple of 8 elements", what, i, (long long)st[i]);
-    MVOC_REQUIRE(((uintptr_t)q % 16 == 0) && ((uintptr_t)k % 16 == 0) && ((uintptr_t)v % 16 == 0) &&
-                     ((uintptr_t)o % 16 == 0),
-                 MVOC_ERR_INVALID_ARG, "%s: pointers must be 16-byte aligned", what);
     const bool pair = pair_batches > 0;
     const int kv_rows = pair ? 64 : 128;
-    CUtensorMap mq, mk, mv;
-    int rc;
-    if ((rc = make_map(&mq, q, dtype, B, H, Nq, BM, st[0], st[1], st[2], "q")) != MVOC_OK) return rc;
-    if ((rc = make_map(&mk, k, dtype, B, H, Nk, kv_rows, st[3], st[4], st[5], "k")) != MVOC_OK) return rc;
-    if ((rc = make_map(&mv, v, dtype, B + pair_batches, H, Nk, kv_rows, st[6], st[7], st[8], "v")) != MVOC_OK) return rc;
+    // q, k, v: [B, N, H, 64] viewed innermost first with element strides (sh, sn, sb); box = one head's 64 columns of
+    // `rows` tokens
+    const void* ptr[3] = {q, k, v};
+    const char* name[3] = {"q", "k", "v"};
+    const int64_t dims[3][4] = {{HD, H, Nq, B}, {HD, H, Nk, B}, {HD, H, Nk, B + pair_batches}};
+    const int64_t str[3][3] = {{st[2], st[1], st[0]}, {st[5], st[4], st[3]}, {st[8], st[7], st[6]}};
+    const int rows[3] = {BM, kv_rows, kv_rows};
+    for (int i = 0; i < 3; ++i)   // all three before the first driver call
+        if ((rc = check_map4(dims[i], str[i], what, name[i])) != MVOC_OK) return rc;
+    CUtensorMap m[3];
+    for (int i = 0; i < 3; ++i) {
+        const int box[4] = {HD, 1, rows[i], 1};
+        if ((rc = make_map4(&m[i], ptr[i], dtype, dims[i], str[i], box, CU_TENSOR_MAP_SWIZZLE_128B, what, name[i])) !=
+            MVOC_OK)
+            return rc;
+    }
     Params prm;
     prm.o = o;
     prm.o_sb = st[9];
@@ -495,7 +425,7 @@ static int run(const void* q, const void* k, const void* v, void* o, int B, int 
     // variants (same results up to the exp2 approximation; the tests run all of them):
     //   1, 2: all exponentials on the MUFU;  3 / 4 / 5: 2 / 3 / 4 of every 8 pairs on the FMA-pipe polynomial;  0: default
     const uint32_t emu = variant == 1 || variant == 2 ? 0x00u : variant == 3 ? 0x88u : variant == 5 ? 0xAAu : 0xA8u;
-#define MVOC_ATTN_LAUNCH(T, BN, NV, EMU) launch<T, BN, NV, 3, EMU>(mq, mk, mv, prm, B, H, s)
+#define MVOC_ATTN_LAUNCH(T, BN, NV, EMU) launch<T, BN, NV, 3, EMU>(m, prm, B, H, s, what)
 #define MVOC_ATTN_EMU(T, BN, NV)                                           \
     switch (emu) {                                                         \
         case 0x00u: return MVOC_ATTN_LAUNCH(T, BN, NV, 0x00u);             \
@@ -514,6 +444,22 @@ static int run(const void* q, const void* k, const void* v, void* o, int B, int 
 }
 
 }  // namespace attn
+
+int check_attn_operands(const void* q, const void* k, const void* v, const void* o, int dtype, int D, int head_dim,
+                        const int64_t* st, int n_st, const char* what) {
+    MVOC_REQUIRE(q && k && v && o, MVOC_ERR_INVALID_ARG, "%s: null pointer", what);
+    MVOC_REQUIRE(dtype == MVOC_BF16 || dtype == MVOC_F16, MVOC_ERR_UNSUPPORTED, "%s: dtype %d unsupported (bf16 / fp16)",
+                 what, dtype);
+    MVOC_REQUIRE(D == head_dim, MVOC_ERR_UNSUPPORTED, "%s: head_dim %d unsupported (%d only)", what, D, head_dim);
+    for (int i = 0; i < n_st; ++i)
+        MVOC_REQUIRE(st[i] % 8 == 0 && st[i] >= 0, MVOC_ERR_UNSUPPORTED,
+                     "%s: stride #%d = %lld is not a non-negative multiple of 8 elements", what, i, (long long)st[i]);
+    MVOC_REQUIRE(((uintptr_t)q % 16 == 0) && ((uintptr_t)k % 16 == 0) && ((uintptr_t)v % 16 == 0) &&
+                     ((uintptr_t)o % 16 == 0),
+                 MVOC_ERR_INVALID_ARG, "%s: pointers must be 16-byte aligned", what);
+    return MVOC_OK;
+}
+
 }  // namespace mvoc
 
 using namespace mvoc;

@@ -39,10 +39,6 @@ __device__ __forceinline__ void mma_bf16_16816(float (&d)[4], uint32_t a0, uint3
         : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
-__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
 // byte offset of 16-byte chunk `c` of row `r` in a 128-byte-row, XOR-swizzled tile
 __device__ __forceinline__ uint32_t swz(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
 
@@ -176,10 +172,10 @@ __global__ void __launch_bounds__(TA_WARPS * 32) attn_temporal_kernel(TAParams p
         for (int dn = 0; dn < 8; ++dn) o[dn][0] = o[dn][1] = o[dn][2] = o[dn][3] = 0.0f;
 #pragma unroll
         for (int kk = 0; kk < KT; ++kk) {
-            const uint32_t a0 = pack_bf16x2(s[2 * kk][0], s[2 * kk][1]);
-            const uint32_t a1 = pack_bf16x2(s[2 * kk][2], s[2 * kk][3]);
-            const uint32_t a2 = pack_bf16x2(s[2 * kk + 1][0], s[2 * kk + 1][1]);
-            const uint32_t a3 = pack_bf16x2(s[2 * kk + 1][2], s[2 * kk + 1][3]);
+            const uint32_t a0 = pack2_rn<__nv_bfloat16>(s[2 * kk][0], s[2 * kk][1]);
+            const uint32_t a1 = pack2_rn<__nv_bfloat16>(s[2 * kk][2], s[2 * kk][3]);
+            const uint32_t a2 = pack2_rn<__nv_bfloat16>(s[2 * kk + 1][0], s[2 * kk + 1][1]);
+            const uint32_t a3 = pack2_rn<__nv_bfloat16>(s[2 * kk + 1][2], s[2 * kk + 1][3]);
 #pragma unroll
             for (int dn = 0; dn < 8; dn += 2) {
                 uint32_t b0, b1, b2, b3;
@@ -195,9 +191,9 @@ __global__ void __launch_bounds__(TA_WARPS * 32) attn_temporal_kernel(TAParams p
 #pragma unroll
         for (int dn = 0; dn < 8; ++dn) {
             *reinterpret_cast<uint32_t*>(stage + swz(mt * 16 + g, dn) + t * 4) =
-                pack_bf16x2(o[dn][0] * i0, o[dn][1] * i0);
+                pack2_rn<__nv_bfloat16>(o[dn][0] * i0, o[dn][1] * i0);
             *reinterpret_cast<uint32_t*>(stage + swz(mt * 16 + g + 8, dn) + t * 4) =
-                pack_bf16x2(o[dn][2] * i1, o[dn][3] * i1);
+                pack2_rn<__nv_bfloat16>(o[dn][2] * i1, o[dn][3] * i1);
         }
         __syncwarp();
 #pragma unroll

@@ -56,33 +56,13 @@ struct Params {
     float scale_log2;
 };
 
-template <typename T> __device__ __forceinline__ uint32_t pack_rn(float lo, float hi);
-template <> __device__ __forceinline__ uint32_t pack_rn<__nv_bfloat16>(float lo, float hi) {
-    __nv_bfloat162 b = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&b);
-}
-template <> __device__ __forceinline__ uint32_t pack_rn<__half>(float lo, float hi) {
-    __half2 b = __floats2half2_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&b);
-}
-
-// kind::f16 instruction descriptor for 16-bit storage type T (fp16: format 0, bf16: format 1), fp32 accumulation
-template <typename T> __host__ __device__ constexpr uint32_t idesc_for(int M, int N, int b_mn_major) {
-    return (1u << 4) | ((std::is_same<T, __half>::value ? 0u : 1u) << 7) |
-           ((std::is_same<T, __half>::value ? 0u : 1u) << 10) | ((uint32_t)b_mn_major << 16) |
-           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
 template <typename T>
 __global__ void __launch_bounds__(THREADS, 1)
 attn_d512_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                  const __grid_constant__ CUtensorMap tm_v, const Params prm) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const uint32_t sbase = smem_u32(smem_raw);
-    if ((sbase & 1023u) != 0u) {  // 128-byte-swizzled tiles need a 1024-byte aligned base
-        if (threadIdx.x == 0) printf("mvoc attn_d512_kernel: dynamic smem base 0x%x is not 1024-byte aligned\n", sbase);
-        __trap();
-    }
+    MVOC_REQUIRE_SMEM_1024(sbase, "attn_d512_kernel");
     const uint32_t sQ = sbase + Q_OFF;
     const uint32_t sRing = sbase + RING_OFF;
     const uint32_t bars = sbase + BAR_OFF;
@@ -147,8 +127,9 @@ attn_d512_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
         }
     } else if (warp == 5) {
         // ===================== MMA issuer =====================
-        constexpr uint32_t IDESC_QK = idesc_for<T>(BM, BN, 0);   // A (Q), B (K) K-major
-        constexpr uint32_t IDESC_PV = idesc_for<T>(BM, BOX, 1);  // B (V) MN-major, 64 value columns per MMA
+        constexpr bool kF16 = std::is_same<T, __half>::value;
+        constexpr uint32_t IDESC_QK = ptx::idesc_f16(kF16, BM, BN, false);  // A (Q), B (K) K-major
+        constexpr uint32_t IDESC_PV = ptx::idesc_f16(kF16, BM, BOX, true);  // B (V) MN-major, 64 value columns per MMA
         const uint32_t tS = tmem + COL_S, tP = tmem + COL_P, tO = tmem + COL_O;
         int u = 0;
         auto wait_slot = [&]() {
@@ -284,7 +265,7 @@ attn_d512_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
                 const float p0 = ptx::ex2_approx(x0), p1 = ptx::ex2_approx(x1);
                 if (k & 1) lb = ptx::add2(lb, ptx::pack2(p0, p1));
                 else la = ptx::add2(la, ptx::pack2(p0, p1));
-                pk[k] = pack_rn<T>(p0, p1);
+                pk[k] = pack2_rn<T>(p0, p1);
             }
             {
                 float s0, s1;
@@ -336,59 +317,14 @@ attn_d512_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
 }
 
 // ------------------------------------------------------------------ host ---
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
-                                  const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres);
-        if (e == cudaSuccess && qres == cudaDriverEntryPointSuccess) fn = (EncodeTiledFn)p;
-    }
-    return fn;
-}
-
-// [B, N, 512] 16-bit with element strides (sb, sn), viewed as [B, N, 8, 64]; box = 128 tokens x 64 columns.
-static int make_map(CUtensorMap* m, const void* base, int dtype, int B, int N, int64_t sb, int64_t sn,
-                    const char* what) {
-    EncodeTiledFn fn = get_encode_fn();
-    MVOC_REQUIRE(fn != nullptr, MVOC_ERR_DRIVER, "mvoc_attn_d512_fwd: cuTensorMapEncodeTiled unavailable");
-    cuuint64_t dims[4] = {(cuuint64_t)BOX, (cuuint64_t)(D / BOX), (cuuint64_t)N, (cuuint64_t)B};
-    cuuint64_t strides[3] = {(cuuint64_t)BOX * 2, (cuuint64_t)sn * 2, (cuuint64_t)sb * 2};
-    // a size-1 dimension may carry any stride; TMA still wants a non-zero multiple of 16 bytes
-    if (N == 1 || strides[1] == 0) strides[1] = (cuuint64_t)D * 2;
-    if (B == 1 || strides[2] == 0) strides[2] = strides[1] * (cuuint64_t)N;
-    cuuint32_t box[4] = {(cuuint32_t)BOX, 1, (cuuint32_t)BM, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = fn(m, dtype == MVOC_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4,
-                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MVOC_REQUIRE(r == CUDA_SUCCESS, MVOC_ERR_DRIVER,
-                 "mvoc_attn_d512_fwd: cuTensorMapEncodeTiled(%s) failed with CUresult %d (B=%d N=%d strides=%lld,%lld)",
-                 what, (int)r, B, N, (long long)sb, (long long)sn);
-    return MVOC_OK;
-}
-
 template <typename T>
-static int launch(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv, const Params& prm, int B,
-                  cudaStream_t s) {
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(attn_d512_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             SMEM_BYTES);
-        MVOC_REQUIRE(e == cudaSuccess, MVOC_ERR_CUDA, "mvoc_attn_d512_fwd: cudaFuncSetAttribute: %s",
-                     cudaGetErrorString(e));
-        attr_set[dev] = true;
-    }
+static int launch(const CUtensorMap (&m)[3], const Params& prm, int B, cudaStream_t s, const char* what) {
+    static bool smem_set[64] = {false};
+    const int rc = set_max_dynamic_smem((const void*)attn_d512_kernel<T>, SMEM_BYTES, smem_set, what);
+    if (rc != MVOC_OK) return rc;
     dim3 grid((prm.N + BM - 1) / BM, 2, B);
-    attn_d512_kernel<T><<<grid, THREADS, SMEM_BYTES, s>>>(mq, mk, mv, prm);
-    return check_launch("mvoc_attn_d512_fwd");
+    attn_d512_kernel<T><<<grid, THREADS, SMEM_BYTES, s>>>(m[0], m[1], m[2], prm);
+    return check_launch(what);
 }
 
 }  // namespace attn_wide
@@ -399,32 +335,33 @@ using namespace mvoc;
 extern "C" int mvoc_attn_d512_fwd(const void* q, const void* k, const void* v, void* o, int B, int N, int D,
                                   int64_t q_sb, int64_t q_sn, int64_t k_sb, int64_t k_sn, int64_t v_sb,
                                   int64_t v_sn, int64_t o_sb, int64_t o_sn, float scale, int dtype, void* stream) {
+    using namespace attn_wide;
     const char* what = "mvoc_attn_d512_fwd";
-    MVOC_REQUIRE(q && k && v && o, MVOC_ERR_INVALID_ARG, "%s: null pointer", what);
-    MVOC_REQUIRE(dtype == MVOC_BF16 || dtype == MVOC_F16, MVOC_ERR_UNSUPPORTED, "%s: dtype %d unsupported (bf16 / fp16)",
-                 what, dtype);
-    MVOC_REQUIRE(D == attn_wide::D, MVOC_ERR_UNSUPPORTED, "%s: head_dim %d unsupported (512 only)", what, D);
+    const int64_t st[8] = {q_sb, q_sn, k_sb, k_sn, v_sb, v_sn, o_sb, o_sn};
+    int rc = check_attn_operands(q, k, v, o, dtype, D, attn_wide::D, st, 8, what);
+    if (rc != MVOC_OK) return rc;
     MVOC_REQUIRE(B > 0 && N > 0, MVOC_ERR_INVALID_ARG, "%s: empty problem B=%d N=%d", what, B, N);
     MVOC_REQUIRE(B <= 65535, MVOC_ERR_UNSUPPORTED, "%s: B=%d exceeds the grid limit", what, B);
-    const int64_t st[8] = {q_sb, q_sn, k_sb, k_sn, v_sb, v_sn, o_sb, o_sn};
-    for (int i = 0; i < 8; ++i)
-        MVOC_REQUIRE(st[i] % 8 == 0 && st[i] >= 0, MVOC_ERR_UNSUPPORTED,
-                     "%s: stride #%d = %lld is not a non-negative multiple of 8 elements", what, i, (long long)st[i]);
-    MVOC_REQUIRE(((uintptr_t)q % 16 == 0) && ((uintptr_t)k % 16 == 0) && ((uintptr_t)v % 16 == 0) &&
-                     ((uintptr_t)o % 16 == 0),
-                 MVOC_ERR_INVALID_ARG, "%s: pointers must be 16-byte aligned", what);
-    CUtensorMap mq, mk, mv;
-    int rc;
-    if ((rc = attn_wide::make_map(&mq, q, dtype, B, N, q_sb, q_sn, "q")) != MVOC_OK) return rc;
-    if ((rc = attn_wide::make_map(&mk, k, dtype, B, N, k_sb, k_sn, "k")) != MVOC_OK) return rc;
-    if ((rc = attn_wide::make_map(&mv, v, dtype, B, N, v_sb, v_sn, "v")) != MVOC_OK) return rc;
-    attn_wide::Params prm;
+    // q, k, v: [B, N, 512] viewed innermost first as [64, 8, N, B]; box = 64 columns of 128 tokens
+    const void* ptr[3] = {q, k, v};
+    const char* name[3] = {"q", "k", "v"};
+    const int64_t dims[4] = {BOX, attn_wide::D / BOX, N, B};
+    const int64_t str[3][3] = {{BOX, q_sn, q_sb}, {BOX, k_sn, k_sb}, {BOX, v_sn, v_sb}};
+    const int box[4] = {BOX, 1, BM, 1};
+    for (int i = 0; i < 3; ++i)   // all three before the first driver call
+        if ((rc = check_map4(dims, str[i], what, name[i])) != MVOC_OK) return rc;
+    CUtensorMap m[3];
+    for (int i = 0; i < 3; ++i)
+        if ((rc = make_map4(&m[i], ptr[i], dtype, dims, str[i], box, CU_TENSOR_MAP_SWIZZLE_128B, what, name[i])) !=
+            MVOC_OK)
+            return rc;
+    Params prm;
     prm.o = o;
     prm.o_sb = o_sb;
     prm.o_sn = o_sn;
     prm.N = N;
     prm.scale_log2 = scale * 1.4426950408889634f;
     cudaStream_t s = (cudaStream_t)stream;
-    if (dtype == MVOC_F16) return attn_wide::launch<__half>(mq, mk, mv, prm, B, s);
-    return attn_wide::launch<__nv_bfloat16>(mq, mk, mv, prm, B, s);
+    if (dtype == MVOC_F16) return launch<__half>(m, prm, B, s, what);
+    return launch<__nv_bfloat16>(m, prm, B, s, what);
 }

@@ -1,5 +1,6 @@
 // Shared helpers for the mvoc_b200 CUDA kernels (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -20,6 +21,24 @@ int check_launch(const char* what);
             return (code);                 \
         }                                  \
     } while (0)
+
+// cudaFuncSetAttribute(MaxDynamicSharedMemorySize, bytes) on `kernel`, once per device: `done` is the call site's
+// record of the devices already set.  MVOC_ERR_CUDA with `what` in the message on failure.
+int set_max_dynamic_smem(const void* kernel, int bytes, bool (&done)[64], const char* what);
+
+// ---- 4-D 16-bit TMA tensor maps (tensormap.cu) ----------------------------
+// dims and box innermost first, element strides of dims 1..3, zero fill out of bounds.  The stride of a dimension of
+// extent 1 is ignored and the packed value (previous stride x previous extent) is encoded; the stride of any other
+// dimension must be a positive multiple of 8 elements (16 bytes), else MVOC_ERR_UNSUPPORTED.  Messages name `what`
+// (the entry point) and `operand`.  check_map4 applies that rule without touching the driver.
+int check_map4(const int64_t (&dims)[4], const int64_t (&str)[3], const char* what, const char* operand);
+int make_map4(CUtensorMap* m, const void* base, int dtype, const int64_t (&dims)[4], const int64_t (&str)[3],
+              const int (&box)[4], CUtensorMapSwizzle swz, const char* what, const char* operand);
+
+// Operands of the tensor-core attention entry points (attn_tc.cu): q, k, v, o non-null and 16-byte aligned, dtype
+// bf16 / fp16, D == head_dim, the n_st strides non-negative multiples of 8 elements.
+int check_attn_operands(const void* q, const void* k, const void* v, const void* o, int dtype, int D, int head_dim,
+                        const int64_t* st, int n_st, const char* what);
 
 inline int num_sms() {
     static int n = 0;
@@ -57,6 +76,16 @@ __device__ __forceinline__ void unpack8(const Vec16& v, float (&f)[8]) {
     const T* p = reinterpret_cast<const T*>(&v);
 #pragma unroll
     for (int i = 0; i < 8; ++i) f[i] = Elem<T>::to_f(p[i]);
+}
+// Two fp32 values rounded to nearest into a 16-bit pair, `lo` in the low half.
+template <typename T> __device__ __forceinline__ uint32_t pack2_rn(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t pack2_rn<__nv_bfloat16>(float lo, float hi) {
+    __nv_bfloat162 b = __floats2bfloat162_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&b);
+}
+template <> __device__ __forceinline__ uint32_t pack2_rn<__half>(float lo, float hi) {
+    __half2 b = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&b);
 }
 template <typename T>
 __device__ __forceinline__ Vec16 pack8(const float (&f)[8]) {

@@ -280,12 +280,6 @@ __device__ __forceinline__ uint64_t mul_gelu_erf2(uint64_t v2, uint64_t g2) {
     return ptx::mul2(v2, gelu);
 }
 
-// Instruction descriptor kind::f16: 16-bit inputs (kF16 ? fp16 : bf16), fp32 accumulation, A and B K-major.
-__host__ __device__ constexpr uint32_t idesc_16(int M, int N, bool f16) {
-    return (1u << 4) | ((f16 ? 0u : 1u) << 7) | ((f16 ? 0u : 1u) << 10) | ((uint32_t)(N >> 3) << 17) |
-           ((uint32_t)(M >> 4) << 24);
-}
-
 struct TileCoord {
     int n_tile, c1, c2, c3;
 };
@@ -322,10 +316,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
                                                        // from the constant bank instead of a per-thread local copy
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const uint32_t sbase = smem_u32(smem_raw);
-    if ((sbase & 1023u) != 0u) {
-        if (threadIdx.x == 0) printf("mvoc gemm_tc_kernel: dynamic smem base 0x%x is not 1024-byte aligned\n", sbase);
-        __trap();
-    }
+    MVOC_REQUIRE_SMEM_1024(sbase, "gemm_tc_kernel");
     constexpr int kStages = C::kStages;
     constexpr int N_OUT = C::N_OUT;
     const uint32_t sOut = sbase + C::out_off;
@@ -422,7 +413,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
             constexpr bool kF16 = sizeof(T) == 2 && !std::is_same<T, __nv_bfloat16>::value;
             uint32_t it = 0, lt = 0;
             for (int t = first_tile; t < prm.total_tiles; t += tile_stride, ++lt) {
-                const uint32_t IDESC = idesc_16(C::kTwoCta ? 256 : 128, tile_cols<C>(prm, t % prm.n_tiles), kF16);
+                const uint32_t IDESC =
+                    ptx::idesc_f16(kF16, C::kTwoCta ? 256 : 128, tile_cols<C>(prm, t % prm.n_tiles), false);
                 const uint32_t buf = lt & 1u;
                 ptx::mbar_wait(b_acc_empty + 8 * buf, ((lt >> 1) & 1u) ^ 1u, 2);
                 ptx::tc_fence_after();
@@ -613,47 +605,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
 }
 
 // ------------------------------------------------------------------ host ---
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres);
-        if (e == cudaSuccess && qres == cudaDriverEntryPointSuccess) fn = (EncodeTiledFn)p;
-    }
-    return fn;
-}
-
-// 4-D 16-bit tensor map: dims / box innermost first, strides (elements) of dims 1..3; zero OOB fill.
-static int make_map4(CUtensorMap* m, const void* base, int dtype, const int64_t (&dims)[4], const int64_t (&str)[3],
-                     const int (&box)[4], CUtensorMapSwizzle swz, const char* what) {
-    EncodeTiledFn fn = get_encode_fn();
-    MVOC_REQUIRE(fn != nullptr, MVOC_ERR_DRIVER, "%s: cuTensorMapEncodeTiled unavailable", what);
-    cuuint64_t d[4], s[3];
-    cuuint32_t b[4], estr[4] = {1, 1, 1, 1};
-    for (int i = 0; i < 4; ++i) d[i] = (cuuint64_t)dims[i], b[i] = (cuuint32_t)box[i];
-    for (int i = 0; i < 3; ++i) {
-        s[i] = (cuuint64_t)str[i] * 2;
-        if (dims[i + 1] == 1 && (s[i] == 0 || s[i] % 16 != 0)) s[i] = (i == 0 ? d[0] * 2 : s[i - 1] * d[i]);
-        MVOC_REQUIRE(s[i] % 16 == 0, MVOC_ERR_UNSUPPORTED, "%s: stride %lld elements is not a multiple of 8", what,
-                     (long long)str[i]);
-    }
-    CUresult r = fn(m, dtype == MVOC_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4,
-                    const_cast<void*>(base), d, s, b, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
-                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    MVOC_REQUIRE(r == CUDA_SUCCESS, MVOC_ERR_DRIVER,
-                 "%s: cuTensorMapEncodeTiled failed with CUresult %d (dims %lld,%lld,%lld,%lld strides %lld,%lld,%lld "
-                 "box %d,%d,%d,%d)",
-                 what, (int)r, (long long)dims[0], (long long)dims[1], (long long)dims[2], (long long)dims[3],
-                 (long long)str[0], (long long)str[1], (long long)str[2], box[0], box[1], box[2], box[3]);
-    return MVOC_OK;
-}
-
-
 // Row box (b1, b2, b3), powers of two with product 128, that wastes the fewest zero-filled rows on the
 // (d1, d2, d3) grid; ties go to the widest box along d1 (longest contiguous runs).
 static void choose_box(int64_t d1, int64_t d2, int64_t d3, int* b1, int* b2, int* b3) {
@@ -699,26 +650,23 @@ struct Problem {
 template <typename C, typename T>
 static int launch_cfg(const Problem& pb, Params prm, int b1, int b2, int b3, cudaStream_t stream) {
     const char* what = pb.what;
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<C, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::alloc);
-        MVOC_REQUIRE(e == cudaSuccess, MVOC_ERR_CUDA, "%s: cudaFuncSetAttribute: %s", what, cudaGetErrorString(e));
-        attr_set[dev] = true;
-    }
+    static bool smem_set[64] = {false};
+    int rc = set_max_dynamic_smem((const void*)gemm_tc_kernel<C, T>, C::alloc, smem_set, what);
+    if (rc != MVOC_OK) return rc;
     CUtensorMap ma[2], mw[2], mo, mr;
-    int rc;
     for (int s = 0; s < pb.n_src; ++s) {
         const Source& sc = pb.src[s];
         const int64_t dims[4] = {sc.K, pb.d1, pb.d2, pb.d3};
         const int box[4] = {KC, b1, b2, b3};
-        if ((rc = make_map4(&ma[s], sc.a, pb.dtype, dims, sc.a_str, box, CU_TENSOR_MAP_SWIZZLE_128B, what)) != MVOC_OK)
+        if ((rc = make_map4(&ma[s], sc.a, pb.dtype, dims, sc.a_str, box, CU_TENSOR_MAP_SWIZZLE_128B, what,
+                            s ? "x2" : "x")) != MVOC_OK)
             return rc;
         const int64_t wd[4] = {sc.K, pb.w_rows, sc.taps, 1};
         const int64_t ws[3] = {sc.K, sc.K * pb.w_rows, sc.K * pb.w_rows * sc.taps};
         const int wb[4] = {KC, C::kEpi == EPI_GEGLU ? C::BN / 2 : C::B_ROWS, 1, 1};
-        if ((rc = make_map4(&mw[s], sc.w, pb.dtype, wd, ws, wb, CU_TENSOR_MAP_SWIZZLE_128B, what)) != MVOC_OK) return rc;
+        if ((rc = make_map4(&mw[s], sc.w, pb.dtype, wd, ws, wb, CU_TENSOR_MAP_SWIZZLE_128B, what, s ? "w2" : "w")) !=
+            MVOC_OK)
+            return rc;
     }
     if (pb.n_src == 1) ma[1] = ma[0], mw[1] = mw[0];
     {
@@ -727,9 +675,10 @@ static int launch_cfg(const Problem& pb, Params prm, int b1, int b2, int b3, cud
         const int64_t dims[4] = {pb.N, pb.d1, pb.d2, pb.d3};
         const int box[4] = {C::SLAB, sb1, sb2, sb3};
         const CUtensorMapSwizzle swz = C::SLAB == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-        if ((rc = make_map4(&mo, pb.out, pb.dtype, dims, pb.out_str, box, swz, what)) != MVOC_OK) return rc;
+        if ((rc = make_map4(&mo, pb.out, pb.dtype, dims, pb.out_str, box, swz, what, "out")) != MVOC_OK) return rc;
         if (pb.residual) {
-            if ((rc = make_map4(&mr, pb.residual, pb.dtype, dims, pb.res_str, box, swz, what)) != MVOC_OK) return rc;
+            if ((rc = make_map4(&mr, pb.residual, pb.dtype, dims, pb.res_str, box, swz, what, "residual")) != MVOC_OK)
+                return rc;
         } else {
             mr = mo;
         }

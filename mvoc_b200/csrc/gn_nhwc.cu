@@ -316,14 +316,12 @@ extern "C" int mvoc_groupnorm_nhwc_stats(const void* x, const void* add, void* p
     dim3 grid(p.chunks, (unsigned)N);
     const size_t smem = (2 * (size_t)p.R + 3) * (size_t)C * sizeof(float);
     MVOC_REQUIRE(smem <= 96 * 1024, MVOC_ERR_UNSUPPORTED, "mvoc_groupnorm_nhwc_stats: C=%d needs %zu B of smem", C, smem);
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaFuncSetAttribute(gnh_stats_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-        cudaFuncSetAttribute(gnh_stats_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-        attr_set = true;
-    }
+    static bool smem_set[2][64] = {};
+    const bool bf16 = dtype == MVOC_BF16;
+    const void* kernel = bf16 ? (const void*)gnh_stats_kernel<__nv_bfloat16> : (const void*)gnh_stats_kernel<__half>;
+    if ((rc = set_max_dynamic_smem(kernel, 96 * 1024, smem_set[bf16], "mvoc_groupnorm_nhwc_stats")) != MVOC_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    if (dtype == MVOC_BF16) gnh_stats_kernel<__nv_bfloat16><<<grid, threads, smem, st>>>(p);
+    if (bf16) gnh_stats_kernel<__nv_bfloat16><<<grid, threads, smem, st>>>(p);
     else gnh_stats_kernel<__half><<<grid, threads, smem, st>>>(p);
     return check_launch("mvoc_groupnorm_nhwc_stats");
 }

@@ -254,19 +254,10 @@ static int gn_launch(const void* x, void* y, const void* gamma, const void* beta
     const bool vec = (S % 8 == 0) && ((uintptr_t)x % 16 == 0) && ((uintptr_t)y % 16 == 0);
     const int64_t slab_bytes = seg * (int64_t)sizeof(T);
     if (frames == 1 && vec && slab_bytes <= GN_SMEM_SLAB_MAX && sizeof(T) == 2) {
-        static bool attr_set[2] = {false, false};
-        const int which = 0;
-        if (!attr_set[which]) {
-            cudaError_t e = cudaFuncSetAttribute(gn_slab_kernel<T>,
-                                                 cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 (int)GN_SMEM_SLAB_MAX);
-            if (e != cudaSuccess) {
-                set_error("mvoc_groupnorm_silu: cudaFuncSetAttribute failed: %s",
-                          cudaGetErrorString(e));
-                return MVOC_ERR_CUDA;
-            }
-            attr_set[which] = true;
-        }
+        static bool smem_set[64] = {false};
+        const int rc = set_max_dynamic_smem((const void*)gn_slab_kernel<T>, (int)GN_SMEM_SLAB_MAX, smem_set,
+                                            "mvoc_groupnorm_silu");
+        if (rc != MVOC_OK) return rc;
         gn_slab_kernel<T><<<(unsigned)(N * G), GN_THREADS, (size_t)slab_bytes, st>>>(
             xp, yp, gp, bp, C, S, G, eps, silu);
         return check_launch("mvoc_groupnorm_silu(slab)");

@@ -190,13 +190,24 @@ __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t addr, uint32_t lbo_
            ((uint64_t)(sbo_bytes >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
-// Instruction descriptor for kind::f16, bf16 x bf16 -> fp32.
-// [4,6) c=F32(1); [7,10) a=BF16(1); [10,13) b=BF16(1); 15 a_major; 16 b_major (1 = MN-major);
+// Instruction descriptor for kind::f16 with fp32 accumulation and A K-major; A and B both fp16 or both bf16.
+// [4,6) c=F32(1); [7,10) a, [10,13) b format (0 = fp16, 1 = bf16); 16 b_major (1 = MN-major);
 // [17,23) N>>3; [24,29) M>>4.
-__host__ __device__ constexpr uint32_t idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) |
-           ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+__host__ __device__ constexpr uint32_t idesc_f16(bool fp16, int M, int N, bool b_mn_major) {
+    return (1u << 4) | ((fp16 ? 0u : 1u) << 7) | ((fp16 ? 0u : 1u) << 10) | ((uint32_t)b_mn_major << 16) |
+           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+
+// 128-byte-swizzled tiles need a 1024-byte aligned dynamic shared-memory base: trap with a message naming the
+// kernel (a string literal) if `sbase` is not.
+#define MVOC_REQUIRE_SMEM_1024(sbase, kernel)                                                                      \
+    do {                                                                                                           \
+        if (((sbase) & 1023u) != 0u) {                                                                             \
+            if (threadIdx.x == 0)                                                                                  \
+                printf("mvoc " kernel ": dynamic smem base 0x%x is not 1024-byte aligned\n", (sbase));             \
+            __trap();                                                                                              \
+        }                                                                                                          \
+    } while (0)
 
 // ---- packed fp32x2 arithmetic (sm_100: FFMA2 / FADD2 issue two fp32 ops per slot) ----------------------
 __device__ __forceinline__ uint64_t pack2(float lo, float hi) {

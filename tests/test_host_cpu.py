@@ -76,6 +76,33 @@ def test_argument_errors_are_reported_without_a_gpu():
     assert rc == -1 and b"null pointer" in lib.mvoc_last_error()
 
 
+@pytest.mark.parametrize("operand", [0, 1, 2])
+def test_attention_rejects_zero_strides_where_the_extent_is_above_one(operand):
+    """q, k and v are read through TMA, which cannot broadcast: a zero batch stride (B = 2) or token stride (N > 1) of
+    q, k or v is refused before any CUDA call, whichever operand carries it."""
+    from mvoc_b200 import _cabi
+
+    lib = _cabi.load()
+    name = b"qkv"[operand:operand + 1]
+
+    def refused(entry):
+        err = lib.mvoc_last_error()
+        return entry in err and name + b" stride" in err
+
+    B, H, N = 2, 2, 128
+    st = [N * H * 64, H * 64, 64] * 4
+    st[3 * operand] = 0                                                  # batch stride of q, k or v
+    assert lib.mvoc_attn_fwd(16, 16, 16, 16, B, H, N, N, 64, *st, 0.125, 0, 0, None) == -2
+    assert refused(b"mvoc_attn_fwd")
+    assert lib.mvoc_attn_pair_fwd(16, 16, 16, 16, B, H, N, N, 64, *st, 1, 0.125, 0, 0, None) == -2
+    assert refused(b"mvoc_attn_pair_fwd")
+    for zero in (2 * operand, 2 * operand + 1):                          # batch, then token stride
+        st = [N * 512, 512] * 4
+        st[zero] = 0
+        assert lib.mvoc_attn_d512_fwd(16, 16, 16, 16, B, N, 512, *st, 1.0, 0, None) == -2
+        assert refused(b"mvoc_attn_d512_fwd")
+
+
 def test_gemm_tile_plan_host_logic():
     """mvoc_gemm_plan (no device call): what the GEMM entries choose.  On B200 a tcgen05.mma costs the same whatever
     N <= 256 is, so the plan minimises the NUMBER of column tiles: full 256-wide tiles plus one narrower tail tile;
