@@ -297,6 +297,18 @@ int mvoc_conv3x3_nhwc(const void* x, const void* w_taps, const void* bias, const
                       int N, int H, int W, int Cin, int Cout, int dtype, int variant, void* stream);
 
 /*
+ * 3x3 convolution, stride 2, channels-last: out[N,Ho,Wo,Cout] = conv(x[N,H,W,Cin], w) + bias, with pad_begin zero
+ * rows / columns before and pad_end after the input, each 0 or 1: Ho = (H + pad_begin + pad_end - 3) / 2 + 1, Wo
+ * likewise.  w_taps: [9, Cout, Cin] as for mvoc_conv3x3_nhwc; bias optional.  Replaces the Conv2d of the VAE
+ * encoder's Downsample2D, which pads (0, 1, 0, 1) and runs a stride-2 conv without padding (pads (0, 1);
+ * i2vgen-xl/pipelines/pipeline_i2vgen_xl.py:893-920 and :860-890 reach it through vae.encode).  torch's
+ * padding=1, as in the UNet's downsamplers, is pads (1, 1).  Cin, Cout multiples of 64; checked before any CUDA call.
+ */
+int mvoc_conv3x3_s2_nhwc(const void* x, const void* w_taps, const void* bias, void* out,
+                         int N, int H, int W, int Cin, int Cout, int pad_begin, int pad_end,
+                         int dtype, int variant, void* stream);
+
+/*
  * Temporal convolution Conv3d(kernel (3,1,1), padding (1,0,0)) on frame-major channels-last rows:
  * x [B, T, S, Cin] -> out [B, T, S, Cout] (+ bias, + residual), w_taps [3, Cout, Cin] (tap = frame offset + 1).
  * Replaces the Conv3d of TemporalConvLayer.conv1..4 and the identity add, i2vgen-xl/pnp_utils.py:1048-1053;

@@ -90,6 +90,7 @@ SIGNATURES = {
     ),
     "mvoc_conv3x3_nhwc": (
         c_int, [c_void_p] * 6 + [c_int, c_void_p] + [c_int] * 5 + [c_int, c_int, c_void_p]),
+    "mvoc_conv3x3_s2_nhwc": (c_int, [c_void_p] * 4 + [c_int] * 9 + [c_void_p]),
     "mvoc_temporal_conv3": (
         c_int, [c_void_p] * 5 + [c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_void_p]),
     "mvoc_linear": (

@@ -407,7 +407,7 @@ static int run(const void* q, const void* k, const void* v, void* o, int B, int 
     CUtensorMap m[3];
     for (int i = 0; i < 3; ++i) {
         const int box[4] = {HD, 1, rows[i], 1};
-        if ((rc = make_map4(&m[i], ptr[i], dtype, dims[i], str[i], box, CU_TENSOR_MAP_SWIZZLE_128B, what, name[i])) !=
+        if ((rc = make_map4(&m[i], ptr[i], dtype, dims[i], str[i], box, 1, CU_TENSOR_MAP_SWIZZLE_128B, what, name[i])) !=
             MVOC_OK)
             return rc;
     }

@@ -352,7 +352,7 @@ extern "C" int mvoc_attn_d512_fwd(const void* q, const void* k, const void* v, v
         if ((rc = check_map4(dims, str[i], what, name[i])) != MVOC_OK) return rc;
     CUtensorMap m[3];
     for (int i = 0; i < 3; ++i)
-        if ((rc = make_map4(&m[i], ptr[i], dtype, dims, str[i], box, CU_TENSOR_MAP_SWIZZLE_128B, what, name[i])) !=
+        if ((rc = make_map4(&m[i], ptr[i], dtype, dims, str[i], box, 1, CU_TENSOR_MAP_SWIZZLE_128B, what, name[i])) !=
             MVOC_OK)
             return rc;
     Params prm;

@@ -30,10 +30,12 @@ int set_max_dynamic_smem(const void* kernel, int bytes, bool (&done)[64], const 
 // dims and box innermost first, element strides of dims 1..3, zero fill out of bounds.  The stride of a dimension of
 // extent 1 is ignored and the packed value (previous stride x previous extent) is encoded; the stride of any other
 // dimension must be a positive multiple of 8 elements (16 bytes), else MVOC_ERR_UNSUPPORTED.  Messages name `what`
-// (the entry point) and `operand`.  check_map4 applies that rule without touching the driver.
+// (the entry point) and `operand`.  check_map4 applies that rule without touching the driver.  `elem_stride` is the
+// TMA traversal stride of dims 1 and 2: 1 loads every element of the box; 2 loads every other one, so a box of
+// {c, 2 b1, 2 b2, b3} delivers c x b1 x b2 x b3 elements (the input rows of a stride-2 convolution).
 int check_map4(const int64_t (&dims)[4], const int64_t (&str)[3], const char* what, const char* operand);
 int make_map4(CUtensorMap* m, const void* base, int dtype, const int64_t (&dims)[4], const int64_t (&str)[3],
-              const int (&box)[4], CUtensorMapSwizzle swz, const char* what, const char* operand);
+              const int (&box)[4], int elem_stride, CUtensorMapSwizzle swz, const char* what, const char* operand);
 
 // Operands of the tensor-core attention entry points (attn_tc.cu): q, k, v, o non-null and 16-byte aligned, dtype
 // bf16 / fp16, D == head_dim, the n_st strides non-negative multiples of 8 elements.

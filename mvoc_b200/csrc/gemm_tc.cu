@@ -11,6 +11,10 @@
 //   conv3x3     : [Cin, W, H, N], 9 taps shifting (d1, d2) by (-1..1, -1..1)
 //   temporal    : [Cin, S, T, B], 3 taps shifting d2 (the frame) by -1..1
 //   linear      : [K, M, 1, 1],   1 tap
+//   conv3x3 s2  : [Cout rows on the OUTPUT grid Wo, Ho, N]; the A map reads the input [Cin, W, H, N] with TMA
+//                 traversal stride 2 along (d1, d2), so a box {64, 2 b1, 2 b2, b3} delivers the b1 x b2 x b3 = 128
+//                 input pixels under the tile's output pixels, and tap (kh, kw) starts at (2 ox0 + kw - pad,
+//                 2 oy0 + kh - pad).  Tiles, MMAs and the epilogue are those of the stride-1 conv.
 // A tile of 128 rows is a TMA box {64 channels, b1, b2, b3} whose start coordinate is moved by the tap shift;
 // rows that fall outside the tensor are ZERO-FILLED by TMA, which IS the convolution's padding — no im2col
 // buffer, no halo copy.  A second (A, W) source appended to the K loop fuses the resnet's 1x1 shortcut conv
@@ -114,6 +118,7 @@ struct Params {
                                // N = tail_cols and the epilogue skips the slabs beyond it
     int gate_off;              // GEGLU: row of W where the gate half starts (F)
     int has_res;
+    int a_stride;              // A coordinate of a tile row = a_stride x its output coordinate (d1, d2) + tap shift
     int dbg;                   // timing experiments only (results are garbage): 1 = never reload the weight stage,
                                // 2 = never reload the activation stage, 4 = no TMA stores, 8 = no epilogue work at
                                // all (accumulators released at once)  (variant bits 20..23)
@@ -382,8 +387,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
                             if (!C::kTwoCta) ptx::mbar_expect_tx(full, bytes);
                             else if (leader) ptx::mbar_expect_tx(full, 2 * bytes);
                             if (!skip_a)
-                                tma_load_tile<C::kTwoCta>(sA, ma, full, kc * KC, tc.c1 + prm.off[src][tap][0],
-                                                          tc.c2 + prm.off[src][tap][1], tc.c3 + prm.off[src][tap][2]);
+                                tma_load_tile<C::kTwoCta>(sA, ma, full, kc * KC,
+                                                          prm.a_stride * tc.c1 + prm.off[src][tap][0],
+                                                          prm.a_stride * tc.c2 + prm.off[src][tap][1],
+                                                          tc.c3 + prm.off[src][tap][2]);
                             if (skip_w) continue;
                             if (C::kEpi == EPI_GEGLU) {
                                 // accumulator columns = NP value columns then NP gate columns of the same Linear
@@ -624,7 +631,9 @@ static void choose_box(int64_t d1, int64_t d2, int64_t d3, int* b1, int* b2, int
 struct Source {
     const void* a;
     int64_t K;                 // channels (multiple of 64)
+    int64_t a_dim[3];          // extents of the activation along d1, d2, d3 (the row grid unless stride > 1)
     int64_t a_str[3];          // element strides of d1, d2, d3
+    int stride;                // 1, or 2 for a stride-2 convolution (every source of a problem shares it)
     const void* w;             // [taps, n_rows, K] contiguous
     int taps;
     int8_t off[MAX_TAPS][3];
@@ -656,16 +665,16 @@ static int launch_cfg(const Problem& pb, Params prm, int b1, int b2, int b3, cud
     CUtensorMap ma[2], mw[2], mo, mr;
     for (int s = 0; s < pb.n_src; ++s) {
         const Source& sc = pb.src[s];
-        const int64_t dims[4] = {sc.K, pb.d1, pb.d2, pb.d3};
-        const int box[4] = {KC, b1, b2, b3};
-        if ((rc = make_map4(&ma[s], sc.a, pb.dtype, dims, sc.a_str, box, CU_TENSOR_MAP_SWIZZLE_128B, what,
-                            s ? "x2" : "x")) != MVOC_OK)
+        const int64_t dims[4] = {sc.K, sc.a_dim[0], sc.a_dim[1], sc.a_dim[2]};
+        const int box[4] = {KC, b1 * sc.stride, b2 * sc.stride, b3};
+        if ((rc = make_map4(&ma[s], sc.a, pb.dtype, dims, sc.a_str, box, sc.stride, CU_TENSOR_MAP_SWIZZLE_128B,
+                            what, s ? "x2" : "x")) != MVOC_OK)
             return rc;
         const int64_t wd[4] = {sc.K, pb.w_rows, sc.taps, 1};
         const int64_t ws[3] = {sc.K, sc.K * pb.w_rows, sc.K * pb.w_rows * sc.taps};
         const int wb[4] = {KC, C::kEpi == EPI_GEGLU ? C::BN / 2 : C::B_ROWS, 1, 1};
-        if ((rc = make_map4(&mw[s], sc.w, pb.dtype, wd, ws, wb, CU_TENSOR_MAP_SWIZZLE_128B, what, s ? "w2" : "w")) !=
-            MVOC_OK)
+        if ((rc = make_map4(&mw[s], sc.w, pb.dtype, wd, ws, wb, 1, CU_TENSOR_MAP_SWIZZLE_128B, what,
+                            s ? "w2" : "w")) != MVOC_OK)
             return rc;
     }
     if (pb.n_src == 1) ma[1] = ma[0], mw[1] = mw[0];
@@ -675,9 +684,10 @@ static int launch_cfg(const Problem& pb, Params prm, int b1, int b2, int b3, cud
         const int64_t dims[4] = {pb.N, pb.d1, pb.d2, pb.d3};
         const int box[4] = {C::SLAB, sb1, sb2, sb3};
         const CUtensorMapSwizzle swz = C::SLAB == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-        if ((rc = make_map4(&mo, pb.out, pb.dtype, dims, pb.out_str, box, swz, what, "out")) != MVOC_OK) return rc;
+        if ((rc = make_map4(&mo, pb.out, pb.dtype, dims, pb.out_str, box, 1, swz, what, "out")) != MVOC_OK) return rc;
         if (pb.residual) {
-            if ((rc = make_map4(&mr, pb.residual, pb.dtype, dims, pb.res_str, box, swz, what, "residual")) != MVOC_OK)
+            if ((rc = make_map4(&mr, pb.residual, pb.dtype, dims, pb.res_str, box, 1, swz, what, "residual")) !=
+                MVOC_OK)
                 return rc;
         } else {
             mr = mo;
@@ -782,6 +792,8 @@ static int run(const Problem& pb, cudaStream_t stream) {
         MVOC_REQUIRE(sc.K > 0 && sc.K % 64 == 0, MVOC_ERR_UNSUPPORTED, "%s: K=%lld must be a multiple of 64", what,
                      (long long)sc.K);
         MVOC_REQUIRE(sc.taps >= 1 && sc.taps <= MAX_TAPS, MVOC_ERR_INVALID_ARG, "%s: %d taps", what, sc.taps);
+        MVOC_REQUIRE(sc.stride == pb.src[0].stride && (sc.stride == 1 || sc.stride == 2), MVOC_ERR_UNSUPPORTED,
+                     "%s: activation stride %d (1 or 2, the same for every source)", what, sc.stride);
         prm.k_chunks[s] = (int)(sc.K / 64);
         prm.taps[s] = sc.taps;
         for (int t = 0; t < sc.taps; ++t)
@@ -794,6 +806,7 @@ static int run(const Problem& pb, cudaStream_t stream) {
     prm.t2 = (int)((pb.d2 + b2 - 1) / b2);
     prm.bias = pb.bias;
     prm.has_res = pb.residual != nullptr;
+    prm.a_stride = pb.src[0].stride;
     prm.gate_off = (int)pb.N;
     prm.dbg = (pb.variant >> 20) & 15;
     // Tile width and CTA mode.  Wide tiles win (chunk_cost above) — until the problem has fewer tiles than the chip
@@ -856,11 +869,13 @@ extern "C" int mvoc_conv3x3_nhwc(const void* x, const void* w_taps, const void* 
     pb.n_src = x2 ? 2 : 1;
     gemm::Source& s0 = pb.src[0];
     s0.a = x, s0.K = Cin, s0.w = w_taps, s0.taps = 9;
+    s0.a_dim[0] = W, s0.a_dim[1] = H, s0.a_dim[2] = N, s0.stride = 1;
     s0.a_str[0] = Cin, s0.a_str[1] = (int64_t)W * Cin, s0.a_str[2] = (int64_t)H * W * Cin;
     for (int t = 0; t < 9; ++t) s0.off[t][0] = (int8_t)(t % 3 - 1), s0.off[t][1] = (int8_t)(t / 3 - 1), s0.off[t][2] = 0;
     if (x2) {
         gemm::Source& s1 = pb.src[1];
         s1.a = x2, s1.K = Cin2, s1.w = w2, s1.taps = 1;
+        s1.a_dim[0] = W, s1.a_dim[1] = H, s1.a_dim[2] = N, s1.stride = 1;
         s1.a_str[0] = Cin2, s1.a_str[1] = (int64_t)W * Cin2, s1.a_str[2] = (int64_t)H * W * Cin2;
         s1.off[0][0] = s1.off[0][1] = s1.off[0][2] = 0;
     }
@@ -883,6 +898,7 @@ extern "C" int mvoc_temporal_conv3(const void* x, const void* w_taps, const void
     pb.n_src = 1;
     gemm::Source& s0 = pb.src[0];
     s0.a = x, s0.K = Cin, s0.w = w_taps, s0.taps = 3;
+    s0.a_dim[0] = S, s0.a_dim[1] = T, s0.a_dim[2] = B, s0.stride = 1;
     s0.a_str[0] = Cin, s0.a_str[1] = S * Cin, s0.a_str[2] = (int64_t)T * S * Cin;
     for (int t = 0; t < 3; ++t) s0.off[t][0] = 0, s0.off[t][1] = (int8_t)(t - 1), s0.off[t][2] = 0;
     pb.N = Cout, pb.w_rows = Cout;
@@ -907,6 +923,7 @@ extern "C" int mvoc_linear(const void* x, const void* w, const void* bias, const
     pb.n_src = 1;
     gemm::Source& s0 = pb.src[0];
     s0.a = x, s0.K = K, s0.w = w, s0.taps = 1;
+    s0.a_dim[0] = M, s0.a_dim[1] = 1, s0.a_dim[2] = 1, s0.stride = 1;
     s0.a_str[0] = ldx, s0.a_str[1] = 0, s0.a_str[2] = 0;
     s0.off[0][0] = s0.off[0][1] = s0.off[0][2] = 0;
     pb.N = N, pb.w_rows = N;
@@ -928,12 +945,43 @@ extern "C" int mvoc_linear_geglu(const void* x, const void* w, const void* bias,
     pb.n_src = 1;
     gemm::Source& s0 = pb.src[0];
     s0.a = x, s0.K = K, s0.w = w, s0.taps = 1;
+    s0.a_dim[0] = M, s0.a_dim[1] = 1, s0.a_dim[2] = 1, s0.stride = 1;
     s0.a_str[0] = K, s0.a_str[1] = 0, s0.a_str[2] = 0;
     s0.off[0][0] = s0.off[0][1] = s0.off[0][2] = 0;
     pb.N = F, pb.w_rows = 2 * (int64_t)F;
     pb.bias = bias, pb.residual = nullptr, pb.out = out;
     pb.out_str[0] = F, pb.out_str[1] = 0, pb.out_str[2] = 0;
     pb.geglu = 1;
+    pb.variant = variant;
+    return gemm::run(pb, (cudaStream_t)stream);
+}
+
+extern "C" int mvoc_conv3x3_s2_nhwc(const void* x, const void* w_taps, const void* bias, void* out, int N, int H, int W,
+                                    int Cin, int Cout, int pad_begin, int pad_end, int dtype, int variant,
+                                    void* stream) {
+    gemm::Problem pb{};
+    pb.what = "mvoc_conv3x3_s2_nhwc";
+    MVOC_REQUIRE(N > 0 && H > 0 && W > 0 && Cin > 0 && Cout > 0, MVOC_ERR_INVALID_ARG,
+                 "%s: empty problem N=%d H=%d W=%d Cin=%d Cout=%d", pb.what, N, H, W, Cin, Cout);
+    MVOC_REQUIRE((pad_begin == 0 || pad_begin == 1) && (pad_end == 0 || pad_end == 1), MVOC_ERR_INVALID_ARG,
+                 "%s: pad_begin=%d pad_end=%d (each 0 or 1)", pb.what, pad_begin, pad_end);
+    // output extent of a 3-tap, stride-2 window over the padded axis (0 when the window does not fit once)
+    auto out_extent = [&](int n) { return n + pad_begin + pad_end < 3 ? 0 : (n + pad_begin + pad_end - 3) / 2 + 1; };
+    const int Ho = out_extent(H), Wo = out_extent(W);
+    MVOC_REQUIRE(Ho >= 1 && Wo >= 1, MVOC_ERR_INVALID_ARG, "%s: H=%d W=%d with pads (%d, %d) leave an empty output",
+                 pb.what, H, W, pad_begin, pad_end);
+    pb.dtype = dtype;
+    pb.d1 = Wo, pb.d2 = Ho, pb.d3 = N;
+    pb.n_src = 1;
+    gemm::Source& s0 = pb.src[0];
+    s0.a = x, s0.K = Cin, s0.w = w_taps, s0.taps = 9;
+    s0.a_dim[0] = W, s0.a_dim[1] = H, s0.a_dim[2] = N, s0.stride = 2;
+    s0.a_str[0] = Cin, s0.a_str[1] = (int64_t)W * Cin, s0.a_str[2] = (int64_t)H * W * Cin;
+    for (int t = 0; t < 9; ++t)
+        s0.off[t][0] = (int8_t)(t % 3 - pad_begin), s0.off[t][1] = (int8_t)(t / 3 - pad_begin), s0.off[t][2] = 0;
+    pb.N = Cout, pb.w_rows = Cout;
+    pb.bias = bias, pb.residual = nullptr, pb.out = out;
+    pb.out_str[0] = Cout, pb.out_str[1] = (int64_t)Wo * Cout, pb.out_str[2] = (int64_t)Ho * Wo * Cout;
     pb.variant = variant;
     return gemm::run(pb, (cudaStream_t)stream);
 }

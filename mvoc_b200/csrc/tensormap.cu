@@ -28,13 +28,15 @@ int check_map4(const int64_t (&dims)[4], const int64_t (&str)[3], const char* wh
 }
 
 int make_map4(CUtensorMap* m, const void* base, int dtype, const int64_t (&dims)[4], const int64_t (&str)[3],
-              const int (&box)[4], CUtensorMapSwizzle swz, const char* what, const char* operand) {
+              const int (&box)[4], int elem_stride, CUtensorMapSwizzle swz, const char* what, const char* operand) {
     int rc = check_map4(dims, str, what, operand);
     if (rc != MVOC_OK) return rc;
+    MVOC_REQUIRE(elem_stride >= 1 && elem_stride <= 8, MVOC_ERR_UNSUPPORTED, "%s: %s element stride %d (1..8)", what,
+                 operand, elem_stride);
     EncodeTiledFn fn = get_encode_fn();
     MVOC_REQUIRE(fn != nullptr, MVOC_ERR_DRIVER, "%s: cuTensorMapEncodeTiled unavailable", what);
     cuuint64_t d[4], s[3];
-    cuuint32_t b[4], estr[4] = {1, 1, 1, 1};
+    cuuint32_t b[4], estr[4] = {1, (cuuint32_t)elem_stride, (cuuint32_t)elem_stride, 1};
     for (int i = 0; i < 4; ++i) d[i] = (cuuint64_t)dims[i], b[i] = (cuuint32_t)box[i];
     for (int i = 0; i < 3; ++i)   // bytes; an extent-1 dimension is never stepped, so it gets the packed stride
         s[i] = dims[i + 1] == 1 ? (i == 0 ? d[0] * 2 : s[i - 1] * d[i]) : (cuuint64_t)str[i] * 2;
@@ -43,9 +45,9 @@ int make_map4(CUtensorMap* m, const void* base, int dtype, const int64_t (&dims)
                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     MVOC_REQUIRE(r == CUDA_SUCCESS, MVOC_ERR_DRIVER,
                  "%s: cuTensorMapEncodeTiled(%s) failed with CUresult %d (dims %lld,%lld,%lld,%lld strides "
-                 "%lld,%lld,%lld box %d,%d,%d,%d)",
+                 "%lld,%lld,%lld box %d,%d,%d,%d element stride %d)",
                  what, operand, (int)r, (long long)dims[0], (long long)dims[1], (long long)dims[2], (long long)dims[3],
-                 (long long)str[0], (long long)str[1], (long long)str[2], box[0], box[1], box[2], box[3]);
+                 (long long)str[0], (long long)str[1], (long long)str[2], box[0], box[1], box[2], box[3], elem_stride);
     return MVOC_OK;
 }
 

@@ -11,10 +11,19 @@ loop (pipelines/pipeline_i2vgen_xl.py:1940-2000; `inverse_config.n_steps`, cfg 1
 `ddim_latents_{t}.pt` is present (the reference only tests for the directory, so a crashed or `--max_steps` run is
 never completed and composite.py later asserts on the missing timesteps).
 
-Out of scope (SURVEY §2 #9, #11): frame loading and the VAE encode of inverse.py:49-55.  The clean video
-latents / prompt / CLIP tensors are read from `--inputs file.pt` (dict: latents [1,4,T,h,w], prompt_embeds
-[1,77,1024], image_embeddings [1,1,1024], image_latents [1,4,T,h,w]; `{video_name}` in the path selects one file
-per entry).  A missing file is an error; `--synthetic` substitutes seeded synthetic tensors and random weights.
+The clean video latents / prompt / CLIP tensors are read from `--inputs file.pt` (dict: latents [1,4,T,h,w],
+prompt_embeds [1,77,1024], image_embeddings [1,1,1024], image_latents [1,4,T,h,w]; `{video_name}` in the path
+selects one file per entry).  A missing file is an error; `--synthetic` substitutes seeded synthetic tensors and
+random UNet weights.
+
+With `--vae_state_dict FILE` (a diffusers AutoencoderKL state dict) the video latents and the first-frame image
+latents are computed here, as inverse.py:143-153 and :49-55 do: the first `n_frames` .png / .jpg files of
+`<video_dir>/<video_name>/` are centre-cropped to `image_size` and encoded with one
+`torch.Generator().manual_seed(seed)` per entry, first the video (`encode_vae_video`), then the first frame
+(`prepare_image_latents`).  `--inputs` then only needs prompt_embeds and image_embeddings (CLIP stays out of scope;
+so does the reference's mp4 fallback, :154-165).  With `--synthetic` and no frame directory, seeded synthetic
+frames are encoded; the encoder weights always come from FILE.
+
 Independent videos are the unit of multi-GPU work here: with torchrun, entry i goes to rank i % world_size
 (replicas, no collective).
 """
@@ -43,8 +52,34 @@ def inversion_complete(out_dir: str, n_steps: int) -> bool:
                for t in DDIMSchedule(n_steps, inverse=True).timesteps)
 
 
+def synthetic_frames(n_frames: int, height: int, width: int, seed: int) -> torch.Tensor:
+    """Seeded uint8 noise frames as model input: [n_frames, 3, height, width] fp32 in [-1, 1]."""
+    g = torch.Generator().manual_seed(seed)
+    return torch.randint(0, 256, (n_frames, 3, height, width), generator=g, dtype=torch.uint8).float() / 127.5 - 1.0
+
+
+def encode_entry(pipe, config, idx: int, synthetic_inputs: bool, device):
+    """(video latents [1,4,T,h,w], first-frame image latents [1,4,T,h,w]) of one entry, fp32 on `device`."""
+    from .vae import load_frames
+
+    inv = config.inverse_config
+    w_px, h_px = inv.image_size
+    n_frames = int(inv.n_frames)
+    frame_dir = os.path.join(str(config.get("video_dir", ".")), str(config.video_name))
+    if os.path.isdir(frame_dir) or not synthetic_inputs:
+        frames = load_frames(frame_dir, n_frames, (int(w_px), int(h_px)))
+    else:
+        logger.info("%s not found: encoding seeded synthetic frames (--synthetic)", frame_dir)
+        frames = synthetic_frames(n_frames, int(h_px), int(w_px), 9000 + idx)
+    frames = frames.to(device)
+    generator = torch.Generator().manual_seed(int(config.get("seed", 0)))
+    latents = pipe.encode_vae_video(frames, generator)                         # inverse.py:49-55
+    image_latents = pipe.prepare_image_latents(frames[:1], n_frames, generator)   # inside invert (:860-890)
+    return latents, image_latents
+
+
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, inputs: str = None,
-         device: str = None, max_steps: int = None, synthetic_inputs: bool = False):
+         device: str = None, max_steps: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None):
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
 
@@ -62,7 +97,12 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
     elif not synthetic_inputs:
         raise FileNotFoundError("--unet_state_dict is required (pass --synthetic to run on random-init weights)")
     unet = prepare(unet.to(device=device, dtype=torch.bfloat16))
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True)
+    vae_encoder = None
+    if vae_state_dict:
+        from .vae import load_vae_encoder
+
+        vae_encoder = load_vae_encoder(vae_state_dict, device)
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae_encoder=vae_encoder)
     done = 0
     for idx, config in enumerate(cfgmod.iter_configs(template_config, configs_json)):
         if idx % world != rank:
@@ -85,9 +125,16 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
         else:
             raise FileNotFoundError("no --inputs file (VAE / CLIP outputs are inputs of this script); pass "
                                     "--synthetic for seeded synthetic tensors")
+        if vae_encoder is not None:
+            if inputs and any(k in src for k in ("latents", "image_latents")):
+                logger.info("%s: latents / image_latents of the inputs file are not read (--vae_state_dict encodes "
+                            "the frames)", config.video_name)
+            latents, image_latents = encode_entry(pipe, config, idx, synthetic_inputs, device)
+        else:
+            latents, image_latents = src["latents"].to(device).float().clone(), src["image_latents"]
         dt = unet.dtype
-        pipe.invert(src["latents"].to(device).float().clone(), src["prompt_embeds"].to(device, dt),
-                    src["image_embeddings"].to(device, dt), src["image_latents"].to(device, dt),
+        pipe.invert(latents, src["prompt_embeds"].to(device, dt),
+                    src["image_embeddings"].to(device, dt), image_latents.to(device, dt),
                     torch.full((1,), int(inv.get("target_fps", 8)), dtype=torch.int64, device=device),
                     num_inference_steps=int(inv.n_steps), guidance_scale=float(inv.cfg), output_dir=out_dir,
                     max_steps=max_steps, keep=False)
@@ -105,6 +152,9 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--max_steps", type=int, default=None)
     ap.add_argument("--synthetic", action="store_true",
                     help="substitute seeded synthetic tensors for the inputs and random-init weights")
+    ap.add_argument("--vae_state_dict", type=str, default=None,
+                    help="AutoencoderKL state dict (.safetensors or torch file): encode <video_dir>/<video_name>/ "
+                         "frames to the video and first-frame latents instead of reading them from --inputs")
     return ap
 
 
@@ -113,4 +163,4 @@ if __name__ == "__main__":
     logging.basicConfig(level=logging.INFO)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # inverse.py:134
     main(args.template_config, args.configs_json, args.unet_state_dict, args.inputs, args.device, args.max_steps,
-         args.synthetic)
+         args.synthetic, args.vae_state_dict)

@@ -729,6 +729,38 @@ def conv3x3(x: torch.Tensor, w_taps: torch.Tensor, bias: Optional[torch.Tensor] 
     return out
 
 
+def conv3x3_s2(x: torch.Tensor, w_taps: torch.Tensor, bias: Optional[torch.Tensor] = None,
+               pad: Sequence[int] = (0, 1), out: Optional[torch.Tensor] = None,
+               variant: Optional[int] = None) -> torch.Tensor:
+    """3x3 / stride 2 convolution on channels-last x [N, H, W, Cin] with w_taps [9, Cout, Cin] (+ bias) ->
+    [N, Ho, Wo, Cout], Ho = (H + pad[0] + pad[1] - 3) // 2 + 1.  pad = (zeros before, zeros after) each axis:
+    (0, 1) is the VAE's Downsample2D (F.pad (0, 1, 0, 1), then an unpadded conv), (1, 1) torch's padding=1."""
+    _need_cuda(x, w_taps, bias, out)
+    if x.dim() != 4 or not x.is_contiguous():
+        raise ValueError(f"conv3x3_s2: need contiguous [N, H, W, Cin], got {tuple(x.shape)}")
+    N, H, W, ci = x.shape
+    if w_taps.dim() != 3 or w_taps.shape[0] != 9 or w_taps.shape[2] != ci or not w_taps.is_contiguous():
+        raise ValueError(f"conv3x3_s2: w_taps must be contiguous [9, Cout, {ci}], got {tuple(w_taps.shape)}")
+    pb, pe = (int(p) for p in pad)
+    if pb not in (0, 1) or pe not in (0, 1):
+        raise ValueError(f"conv3x3_s2: pad {tuple(pad)} must be (0 or 1, 0 or 1)")
+    Ho, Wo = ((n + pb + pe - 3) // 2 + 1 for n in (H, W))
+    if Ho < 1 or Wo < 1:
+        raise ValueError(f"conv3x3_s2: {H}x{W} with pad {tuple(pad)} leaves an empty output")
+    co = w_taps.shape[1]
+    if out is None:
+        out = torch.empty((N, Ho, Wo, co), dtype=x.dtype, device=x.device)
+    elif tuple(out.shape) != (N, Ho, Wo, co) or not out.is_contiguous():
+        raise ValueError(f"conv3x3_s2: out must be contiguous [{N}, {Ho}, {Wo}, {co}]")
+    v = GEMM_VARIANT if variant is None else variant
+    with _Timed(("gemm", "conv3x3_s2", N * Ho * Wo, 9 * ci, co), 2.0 * N * Ho * Wo * co * 9 * ci):
+        rc = _cabi.load().mvoc_conv3x3_s2_nhwc(x.data_ptr(), w_taps.data_ptr(), _ptr(bias), out.data_ptr(), N, H, W,
+                                               ci, co, pb, pe, _dt(x), int(v), _stream())
+    _cabi.check(rc, "mvoc_conv3x3_s2_nhwc")
+    _count()
+    return out
+
+
 def temporal_conv3(x: torch.Tensor, w_taps: torch.Tensor, bias: Optional[torch.Tensor], videos: int, frames: int,
                    residual: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
                    variant: Optional[int] = None) -> torch.Tensor:

@@ -5,9 +5,10 @@ hot path:
   * ``sample_with_pnp_pipeline_with_edit_prompt_extraction_with_attn_injection``  (:1220-1748,
     loop :1636-1734) — 50-step DDIM composition with source-branch feature injection;
   * ``invert``  (:1752-2018, loop :1940-2000) — DDIM inversion writing ``ddim_latents_{t}.pt``.
-VAE / CLIP / PIL work around the loops (:1356-1541, :1739-1748) is out of scope (SURVEY §2 #9): the
-methods take the tensors those stages produce (prompt embeds, CLIP image embeds, first-frame image
-latents, masks, inverted latents).  INTEGRATION.md shows the seam.
+CLIP / PIL work around the loops (:1356-1541, :1739-1748) is out of scope (SURVEY §2 #9): the loops take
+the tensors those stages produce (prompt embeds, CLIP image embeds, first-frame image latents, masks,
+inverted latents).  The VAE runs here when the pipeline is given one: ``decode_latents`` (decoder),
+``encode_vae_video`` and ``prepare_image_latents`` (encoder).  INTEGRATION.md shows the seam.
 
 Per step the reference launches ~6 elementwise kernels per object for the fusion, a torch.cat, the
 CFG combine and ~10 scheduler kernels, reloads the source latents from disk and syncs twice
@@ -98,11 +99,13 @@ class Conditioning:
 
 
 class I2VGenXLPipeline:
-    def __init__(self, unet, device="cuda", parallel=None, use_cuda_graphs: bool = False, vae=None):
+    def __init__(self, unet, device="cuda", parallel=None, use_cuda_graphs: bool = False, vae=None,
+                 vae_encoder=None):
         from .parallel import FrameParallel
 
         self.unet = unet
         self.vae = vae             # mvoc_b200.vae.AutoencoderKLDecoder for decode_latents, or None
+        self.vae_encoder = vae_encoder   # mvoc_b200.vae.AutoencoderKLEncoder for encode_vae_video, or None
         self.device = torch.device(device)
         self.parallel = parallel or FrameParallel.single(self.device)
         # A UNet forward is ~2700 launches; enqueuing them from Python takes about as long as the GPU needs
@@ -134,6 +137,47 @@ class I2VGenXLPipeline:
         frames = [self.vae(flat[i:i + decode_chunk_size]) for i in range(0, flat.shape[0], decode_chunk_size)]
         image = torch.cat(frames, dim=0)
         return image.reshape((b, f) + image.shape[1:]).permute(0, 2, 1, 3, 4).float()
+
+    @torch.no_grad()
+    def _vae_latents(self, images: torch.Tensor, generator: Optional[torch.Generator] = None,
+                     encode_chunk_size: int = 4) -> torch.Tensor:
+        """images [n, 3, H, W] in [-1, 1] -> scaled latents [n, 4, H/8, W/8] fp32: vae.encode(x).latent_dist.sample()
+        x scaling_factor.  The frames are encoded `encode_chunk_size` at a time (which bounds the encoder's activation
+        memory); the noise of the sample is ONE torch.randn((n, 4, h, w)) in fp32 on the generator's device, so the
+        chunk size changes nothing else.  Both encode_vae_video and prepare_image_latents go through here."""
+        from .vae import SCALING_FACTOR, DiagonalGaussian
+
+        if self.vae_encoder is None:
+            raise RuntimeError("encoding frames: this pipeline was built without a VAE encoder (vae_encoder=None)")
+        if encode_chunk_size < 1:
+            raise ValueError(f"encode_chunk_size={encode_chunk_size} must be >= 1")
+        moments = torch.cat([self.vae_encoder(images[i:i + encode_chunk_size])
+                             for i in range(0, images.shape[0], encode_chunk_size)])
+        post = DiagonalGaussian(moments)
+        noise = torch.randn(tuple(post.mean.shape), generator=generator, dtype=torch.float32,
+                            device=generator.device if generator is not None else post.mean.device)
+        return post.sample(noise.to(post.mean.device)) * SCALING_FACTOR
+
+    def encode_vae_video(self, frames: torch.Tensor, generator: Optional[torch.Generator] = None,
+                         encode_chunk_size: int = 4) -> torch.Tensor:
+        """pipelines/pipeline_i2vgen_xl.py:893-920: frames [T, 3, H, W] in [-1, 1] -> latents [1, 4, T, H/8, W/8]
+        fp32, a sample of the posterior (not its mode) times the scaling factor.  Sample or mode could not be read
+        off the reference here; the sample is what its prepare_image_latents takes (diffusers 0.27.2), and this
+        method follows it."""
+        lat = self._vae_latents(frames, generator, encode_chunk_size)
+        return lat.permute(1, 0, 2, 3).unsqueeze(0).contiguous()
+
+    def prepare_image_latents(self, image: torch.Tensor, num_frames: int,
+                              generator: Optional[torch.Generator] = None) -> torch.Tensor:
+        """pipelines/pipeline_i2vgen_xl.py:860-890 (diffusers 0.27.2) at one video per prompt and guidance 1, the
+        only case inversion uses: image [1, 3, H, W] -> [1, 4, T, H/8, W/8] fp32.  Frame 0 is the encoded, scaled
+        image; frames 1..T-1 are constant planes i / (T - 1), the position mask of the later frames."""
+        lat = self._vae_latents(image, generator).unsqueeze(2)
+        if num_frames > 1:
+            pos = torch.arange(1, num_frames, dtype=torch.float32, device=lat.device) / (num_frames - 1)
+            pos = pos.view(1, 1, -1, 1, 1).expand(lat.shape[0], lat.shape[1], -1, lat.shape[3], lat.shape[4])
+            lat = torch.cat([lat, pos], dim=2)
+        return lat
 
     def drop_graphs(self) -> None:
         """Forget every captured graph.  The private pool goes with them: torch asserts when a capture re-uses a
