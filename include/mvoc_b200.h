@@ -126,6 +126,26 @@ int mvoc_attn_d512_fwd(const void* q, const void* k, const void* v, void* o, int
                        float scale, int dtype, void* stream);
 
 /*
+ * Dense non-causal attention forward at head_dim 80, O = softmax(Q K^T * scale) V.
+ * Replaces the self-attention of transformers' CLIPAttention in the CLIP image tower (ViT-H/14: 16 heads of 80 over
+ * 257 tokens), reached from I2VGenXLPipeline._encode_image, i2vgen-xl/pipelines/pipeline_i2vgen_xl.py:1391-1541
+ * (the per-branch, per-frame image embeddings).
+ *
+ * Arguments and strides as mvoc_attn_fwd: q,o [B, Nq, H, D], k,v [B, Nk, H, D], D == 80 innermost and contiguous,
+ * strides in ELEMENTS for (batch, token, head), so q/k/v may be the three column slices of one fused QKV projection
+ * output [B*N, 3*H*80].  Any Nq, Nk >= 1.  Tensor-core path (tcgen05.mma, accumulators in TMEM, operands staged by
+ * TMA); bf16 or fp16 (P is rounded to the storage type).  Requirements: base pointers 16-byte aligned, strides
+ * non-negative multiples of 8, and positive along every dimension of extent > 1 (MVOC_ERR_UNSUPPORTED otherwise).
+ */
+int mvoc_attn_d80_fwd(const void* q, const void* k, const void* v, void* o,
+                      int B, int H, int Nq, int Nk, int D,
+                      int64_t q_sb, int64_t q_sn, int64_t q_sh,
+                      int64_t k_sb, int64_t k_sn, int64_t k_sh,
+                      int64_t v_sb, int64_t v_sn, int64_t v_sh,
+                      int64_t o_sb, int64_t o_sn, int64_t o_sh,
+                      float scale, int dtype, void* stream);
+
+/*
  * Short-sequence attention (tokens = frames), one warp per (pixel, head).
  * Replaces F.scaled_dot_product_attention at i2vgen-xl/pnp_utils.py:862-864
  * (injected temporal attn1) and the stock processor on the temporal attn2,
@@ -334,6 +354,15 @@ int mvoc_linear(const void* x, const void* w, const void* bias, const void* resi
  */
 int mvoc_linear_geglu(const void* x, const void* w, const void* bias, void* out, int64_t M, int K, int F,
                       int dtype, int variant, void* stream);
+
+/*
+ * Linear with the exact (erf) GELU in the epilogue: out[M, N] = gelu(x[M, K] . w[N, K]^T + bias[N]); row strides
+ * ldx / ldo in elements (multiples of 8); bias may be null.  The erf GELU is the GEGLU epilogue's.  Replaces mlp.fc1 +
+ * activation_fn ("gelu") of every CLIPEncoderLayer of the CLIP image tower (transformers' CLIPMLP), reached from
+ * I2VGenXLPipeline._encode_image, i2vgen-xl/pipelines/pipeline_i2vgen_xl.py:1391-1541.  K, N multiples of 64.
+ */
+int mvoc_linear_gelu(const void* x, const void* w, const void* bias, void* out, int64_t M, int K, int N,
+                     int64_t ldx, int64_t ldo, int dtype, int variant, void* stream);
 
 /*
  * ---- frame-shard <-> pixel-shard exchange over NVLink peer memory (csrc/exchange.cu) ----------------------

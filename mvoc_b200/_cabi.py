@@ -40,6 +40,8 @@ SIGNATURES = {
         c_int, [c_void_p] * 4 + [c_int] * 5 + [ctypes.POINTER(c_int64), c_int, c_float, c_int, c_int, c_void_p, c_void_p]),
     "mvoc_attn_d512_fwd": (
         c_int, [c_void_p] * 4 + [c_int] * 3 + [c_int64] * 8 + [c_float, c_int, c_void_p]),
+    "mvoc_attn_d80_fwd": (
+        c_int, [c_void_p] * 4 + [c_int] * 5 + [c_int64] * 12 + [c_float, c_int, c_void_p]),
     "mvoc_attn_temporal_fwd": (
         c_int,
         [c_void_p] * 4 + [c_int64, c_int, c_int, c_int] + [c_int64] * 12 + [c_float, c_int, c_void_p],
@@ -96,6 +98,7 @@ SIGNATURES = {
     "mvoc_linear": (
         c_int, [c_void_p] * 5 + [c_int64, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
     "mvoc_linear_geglu": (c_int, [c_void_p] * 4 + [c_int64, c_int, c_int, c_int, c_int, c_void_p]),
+    "mvoc_linear_gelu": (c_int, [c_void_p] * 4 + [c_int64, c_int, c_int, c_int64, c_int64, c_int, c_int, c_void_p]),
     "mvoc_exchange_header_bytes": (c_int64, []),
     "mvoc_exchange_max_sites": (c_int, []),
     "mvoc_exchange_arena_create": (c_int, [c_int64, ctypes.POINTER(c_void_p), c_void_p]),

@@ -23,6 +23,13 @@ With `--vae_state_dict` (a diffusers AutoencoderKL state dict, .safetensors or a
 also decoded (decode_latents, pipelines/pipeline_i2vgen_xl.py:771-791) and written as one PNG per frame to
 `<output_dir>/composite_frames/` (`composite_frames.synthetic/` under `--synthetic`).  `--synthetic` never invents
 decoder weights: without the flag nothing is decoded.
+
+With `--image_encoder_state_dict FILE` (a transformers CLIPVisionModelWithProjection state dict) `image_embeddings`
+[n+3,T,1024] is computed here in the branch order [bg, objs..., zeros, main] (pipelines/pipeline_i2vgen_xl.py:766-767)
+from `edited_contorl_frame_path_background`, `edited_contorl_frame_path[j]` and `edited_contorl_frame_path_main` (the
+first frame when a path is a directory), each centre-cropped to (width, width), resized to 224 x 224 and
+CLIP-normalised.  Every other conditioning key still comes from `--conditioning`.  A missing control frame is an
+error; only `--synthetic` substitutes a seeded synthetic frame for it.
 """
 from __future__ import annotations
 
@@ -127,8 +134,37 @@ def run_entry(pipe, config, device, conditioning=None, allow_synthetic: bool = F
         obj_ddim_latents_idx_offset=list(config.obj_ddim_latents_idx_offset)[:n_obj] or None)
 
 
+def branch_image_embeddings(pipe, config, allow_synthetic: bool = False) -> torch.Tensor:
+    """image_embeddings [n+3, T, 1024] of one entry in the branch order [bg, objs..., zeros, main] (SURVEY Appendix B
+    #9; pipelines/pipeline_i2vgen_xl.py:766-767).  The reference encodes every frame of every branch, T x (n+2) CLIP
+    calls, but the UNet reads only image_embeddings[:, 0:1] (mvoc_b200/unet3d.py, I2VGenXLUNet.context), so ONE
+    embedding per branch from its control frame, repeated over T, gives the UNet the same input with n+2 calls."""
+    from PIL import Image
+
+    from .clip import clip_image_input, first_frame
+
+    T = int(config.n_frames)
+    w_px, h_px = (int(v) for v in config.image_size)
+    paths = ([config.edited_contorl_frame_path_background] + list(config.edited_contorl_frame_path)
+             + [config.edited_contorl_frame_path_main])
+    images = []
+    for i, p in enumerate(paths):
+        if os.path.exists(p):
+            images.append(first_frame(p))
+            continue
+        if not allow_synthetic:
+            raise FileNotFoundError(f"control frame {p!r} not found (pass --synthetic for a synthetic frame)")
+        logger.warning("control frame %s not found: using a seeded synthetic frame (--synthetic)", p)
+        g = torch.Generator().manual_seed(7000 + i)
+        images.append(Image.fromarray(torch.randint(0, 256, (h_px, w_px, 3), generator=g, dtype=torch.uint8).numpy()))
+    emb = pipe.encode_image(clip_image_input(images, w_px))                      # [n+2, 1, 1024]
+    emb = torch.cat([emb[:-1], torch.zeros_like(emb[:1]), emb[-1:]])           # [bg, objs, zeros, main]
+    return emb.expand(-1, T, -1).contiguous()
+
+
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, conditioning: str = None,
-         device: str = None, max_entries: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None):
+         device: str = None, max_entries: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None,
+         image_encoder_state_dict: str = None):
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
     from .vae import load_vae_decoder, save_frames
@@ -145,7 +181,12 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
         raise FileNotFoundError("--unet_state_dict is required (pass --synthetic to run on random-init weights)")
     unet = prepare(unet.to(device=device, dtype=torch.bfloat16))
     vae = load_vae_decoder(vae_state_dict, device) if vae_state_dict else None
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae=vae)
+    image_encoder = None
+    if image_encoder_state_dict:
+        from .clip import load_clip_image_encoder
+
+        image_encoder = load_clip_image_encoder(image_encoder_state_dict, device)
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae=vae, image_encoder=image_encoder)
     done = 0
     for config in cfgmod.iter_configs(template_config, configs_json):
         config = resolve_paths(config)
@@ -156,6 +197,16 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
             if not os.path.exists(cpath):
                 raise FileNotFoundError(f"conditioning file {cpath!r} not found")
             cond = torch.load(cpath, map_location="cpu")
+        if image_encoder is not None:
+            if cond is not None and "image_embeddings" in cond:
+                logger.info("%s: image_embeddings of the conditioning file is not read (--image_encoder_state_dict "
+                            "encodes the control frames)", config.video_name)
+            if cond is None and synthetic_inputs:   # the other keys stay synthetic
+                T, h, w = latent_geometry(config)
+                cond = synthetic.make_inputs(synthetic.Workload(config.video_name, "full", T, h, w,
+                                                                len(config.obj_mask_path)), [], None)
+            if cond is not None:
+                cond = dict(cond, image_embeddings=branch_image_embeddings(pipe, config, synthetic_inputs))
         latents = run_entry(pipe, config, device, cond, allow_synthetic=synthetic_inputs)
         os.makedirs(config.output_dir, exist_ok=True)
         out = os.path.join(config.output_dir,
@@ -181,6 +232,9 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--conditioning", type=str, default=None)
     ap.add_argument("--vae_state_dict", type=str, default=None,
                     help="diffusers AutoencoderKL state dict: also decode the latents and write PNG frames")
+    ap.add_argument("--image_encoder_state_dict", type=str, default=None,
+                    help="CLIPVisionModelWithProjection state dict: encode the control frames to image_embeddings "
+                         "instead of reading them from --conditioning")
     ap.add_argument("--device", type=str, default=None)
     ap.add_argument("--max_entries", type=int, default=None)
     ap.add_argument("--synthetic", action="store_true",
@@ -193,4 +247,4 @@ if __name__ == "__main__":
     logging.basicConfig(level=logging.INFO)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # composite.py:246
     main(args.template_config, args.configs_json, args.unet_state_dict, args.conditioning, args.device,
-         args.max_entries, args.synthetic, args.vae_state_dict)
+         args.max_entries, args.synthetic, args.vae_state_dict, args.image_encoder_state_dict)

@@ -5,6 +5,7 @@
 //   TemporalConvLayer conv1..4 (+ identity)                 i2vgen-xl/pnp_utils.py:1048-1053
 //   to_q / to_k / to_v / to_out, proj_in / proj_out         i2vgen-xl/pnp_utils.py:604-612, :692, :191, :206, :432, :503
 //   GEGLU feed-forward                                      i2vgen-xl/pnp_utils.py:335
+//   CLIP image tower mlp.fc1 + GELU (Linear with the exact GELU in the epilogue; mvoc_b200/clip.py)
 //
 // Formulation.  out[row, n] = sum_{src, tap, k} A_src[row + shift(tap), k] * W_src[tap, n, k]  (+ bias[n]) (+ residual)
 // where the rows of A are the pixels of a channels-last activation viewed as a 4-D tensor [K, d1, d2, d3]:
@@ -60,7 +61,7 @@ constexpr int SMEM_LIMIT = 232448;         // 227 KB per CTA
 constexpr uint32_t TMEM_COLS = 512;
 constexpr int MAX_TAPS = 9;
 
-enum Epilogue { EPI_LINEAR = 0, EPI_GEGLU = 1 };
+enum Epilogue { EPI_LINEAR = 0, EPI_GEGLU = 1, EPI_GELU = 2 };   // GELU: the Linear's tile, then gelu(out)
 
 template <int BN_, bool kTwoCta_, int kEpi_>
 struct Cfg {
@@ -308,7 +309,7 @@ __device__ __forceinline__ TileCoord decode_tile(const Params& p, int t, uint32_
 // accumulator columns in use for column tile n_tile
 template <typename C>
 __device__ __forceinline__ int tile_cols(const Params& p, int n_tile) {
-    if (C::kEpi == EPI_LINEAR && p.tail_cols > 0 && n_tile == p.n_tiles - 1) return p.tail_cols;
+    if (C::kEpi != EPI_GEGLU && p.tail_cols > 0 && n_tile == p.n_tiles - 1) return p.tail_cols;
     return C::BN;
 }
 
@@ -540,6 +541,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
                             ptx::unpack2(mul_gelu_erf2(ptx::pack2(f[e], f[e + 1]), ptx::pack2(gv[e], gv[e + 1])), f[e],
                                          f[e + 1]);
                     }
+                    if constexpr (C::kEpi == EPI_GELU) {   // gelu(acc + bias) = 1 x gelu(acc + bias): the GEGLU gate code
+#pragma unroll
+                        for (int e = 0; e < 8; e += 2)
+                            ptx::unpack2(mul_gelu_erf2(ptx::pack2(1.0f, 1.0f), ptx::pack2(f[e], f[e + 1])), f[e], f[e + 1]);
+                    }
                     const uint32_t addr = sbuf + (((uint32_t)c ^ sw) << 4);
                     if (prm.has_res) add8<T>(f, lds16(addr));
                     sts16(addr, pack8<T>(f));
@@ -652,6 +658,7 @@ struct Problem {
     void* out;
     int64_t out_str[3];
     int geglu;
+    int gelu;                  // exact GELU on the Linear's output (EPI_GELU)
     int variant;               // bit 0: CTA pairs; bit 1: no tail tiles; bits 8..16: BN override (0 = auto)
     const char* what;
 };
@@ -695,7 +702,7 @@ static int launch_cfg(const Problem& pb, Params prm, int b1, int b2, int b3, cud
     }
     prm.n_tiles = (int)((pb.N + C::OUT_COLS - 1) / C::OUT_COLS);
     prm.tail_cols = (int)(pb.N % C::OUT_COLS);
-    MVOC_REQUIRE(prm.tail_cols == 0 || (C::kEpi == EPI_LINEAR && prm.tail_cols % 64 == 0),
+    MVOC_REQUIRE(prm.tail_cols == 0 || (C::kEpi != EPI_GEGLU && prm.tail_cols % 64 == 0),
                  MVOC_ERR_UNSUPPORTED, "%s: N=%lld does not tile by %d columns", what, (long long)pb.N, C::OUT_COLS);
     const int64_t m_tiles = (int64_t)prm.t1 * prm.t2 * ((pb.d3 + b3 - 1) / b3);
     const int64_t units = C::kTwoCta ? (m_tiles + 1) / 2 : m_tiles;
@@ -823,6 +830,16 @@ static int run(const Problem& pb, cudaStream_t stream) {
     if (pb.geglu) {
         if (BN == 256) return launch_bn<256, EPI_GEGLU>(pb, prm, b1, b2, b3, stream, two);
         return launch_bn<128, EPI_GEGLU>(pb, prm, b1, b2, b3, stream, two);
+    }
+    if (pb.gelu) {
+        switch (BN) {
+            case 256: return launch_bn<256, EPI_GELU>(pb, prm, b1, b2, b3, stream, two);
+            case 192: return launch_bn<192, EPI_GELU>(pb, prm, b1, b2, b3, stream, two);
+            case 160: return launch_bn<160, EPI_GELU>(pb, prm, b1, b2, b3, stream, two);
+            case 128: return launch_bn<128, EPI_GELU>(pb, prm, b1, b2, b3, stream, two);
+            case 64: return launch_bn<64, EPI_GELU>(pb, prm, b1, b2, b3, stream, two);
+            default: break;
+        }
     }
     switch (BN) {
         case 256: return launch_bn<256, EPI_LINEAR>(pb, prm, b1, b2, b3, stream, two);
@@ -982,6 +999,30 @@ extern "C" int mvoc_conv3x3_s2_nhwc(const void* x, const void* w_taps, const voi
     pb.N = Cout, pb.w_rows = Cout;
     pb.bias = bias, pb.residual = nullptr, pb.out = out;
     pb.out_str[0] = Cout, pb.out_str[1] = (int64_t)Wo * Cout, pb.out_str[2] = (int64_t)Ho * Wo * Cout;
+    pb.variant = variant;
+    return gemm::run(pb, (cudaStream_t)stream);
+}
+
+extern "C" int mvoc_linear_gelu(const void* x, const void* w, const void* bias, void* out, int64_t M, int K, int N,
+                                int64_t ldx, int64_t ldo, int dtype, int variant, void* stream) {
+    gemm::Problem pb{};
+    pb.what = "mvoc_linear_gelu";
+    MVOC_REQUIRE(M > 0 && K > 0 && N > 0, MVOC_ERR_INVALID_ARG, "%s: empty problem M=%lld K=%d N=%d", pb.what,
+                 (long long)M, K, N);
+    MVOC_REQUIRE(ldx >= K && ldo >= N, MVOC_ERR_INVALID_ARG, "%s: leading dimensions ldx=%lld ldo=%lld too small for K=%d N=%d",
+                 pb.what, (long long)ldx, (long long)ldo, K, N);
+    pb.dtype = dtype;
+    pb.d1 = M, pb.d2 = 1, pb.d3 = 1;
+    pb.n_src = 1;
+    gemm::Source& s0 = pb.src[0];
+    s0.a = x, s0.K = K, s0.w = w, s0.taps = 1;
+    s0.a_dim[0] = M, s0.a_dim[1] = 1, s0.a_dim[2] = 1, s0.stride = 1;
+    s0.a_str[0] = ldx, s0.a_str[1] = 0, s0.a_str[2] = 0;
+    s0.off[0][0] = s0.off[0][1] = s0.off[0][2] = 0;
+    pb.N = N, pb.w_rows = N;
+    pb.bias = bias, pb.residual = nullptr, pb.out = out;
+    pb.out_str[0] = ldo, pb.out_str[1] = 0, pb.out_str[2] = 0;
+    pb.gelu = 1;
     pb.variant = variant;
     return gemm::run(pb, (cudaStream_t)stream);
 }

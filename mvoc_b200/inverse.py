@@ -24,6 +24,12 @@ latents are computed here, as inverse.py:143-153 and :49-55 do: the first `n_fra
 so does the reference's mp4 fallback, :154-165).  With `--synthetic` and no frame directory, seeded synthetic
 frames are encoded; the encoder weights always come from FILE.
 
+With `--image_encoder_state_dict FILE` (a transformers CLIPVisionModelWithProjection state dict) `image_embeddings`
+[1,1,1024] is computed here from the first frame of the same directory: centre-cropped to (width, width), resized to
+224 x 224 and CLIP-normalised (mvoc_b200.clip.clip_image_input), then encoded on the library's kernels.  It works with
+or without `--vae_state_dict`; with both, `--inputs` only needs prompt_embeds.  `--synthetic` without a frame
+directory encodes the first seeded synthetic frame.
+
 Independent videos are the unit of multi-GPU work here: with torchrun, entry i goes to rank i % world_size
 (replicas, no collective).
 """
@@ -78,8 +84,27 @@ def encode_entry(pipe, config, idx: int, synthetic_inputs: bool, device):
     return latents, image_latents
 
 
+def image_embeddings_entry(pipe, config, idx: int, synthetic_inputs: bool) -> torch.Tensor:
+    """CLIP image_embeddings [1,1,1024] of one entry's first frame (the frame directory of encode_entry)."""
+    from PIL import Image
+
+    from .clip import clip_image_input, first_frame
+
+    inv = config.inverse_config
+    w_px, h_px = (int(v) for v in inv.image_size)
+    frame_dir = os.path.join(str(config.get("video_dir", ".")), str(config.video_name))
+    if os.path.isdir(frame_dir) or not synthetic_inputs:
+        image = first_frame(frame_dir)
+    else:
+        logger.info("%s not found: encoding the first seeded synthetic frame (--synthetic)", frame_dir)
+        f0 = synthetic_frames(1, h_px, w_px, 9000 + idx)[0]
+        image = Image.fromarray(((f0 + 1.0) * 127.5).round().to(torch.uint8).permute(1, 2, 0).numpy())
+    return pipe.encode_image(clip_image_input(image, w_px))
+
+
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, inputs: str = None,
-         device: str = None, max_steps: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None):
+         device: str = None, max_steps: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None,
+         image_encoder_state_dict: str = None):
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
 
@@ -102,7 +127,12 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
         from .vae import load_vae_encoder
 
         vae_encoder = load_vae_encoder(vae_state_dict, device)
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae_encoder=vae_encoder)
+    image_encoder = None
+    if image_encoder_state_dict:
+        from .clip import load_clip_image_encoder
+
+        image_encoder = load_clip_image_encoder(image_encoder_state_dict, device)
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae_encoder=vae_encoder, image_encoder=image_encoder)
     done = 0
     for idx, config in enumerate(cfgmod.iter_configs(template_config, configs_json)):
         if idx % world != rank:
@@ -132,9 +162,16 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
             latents, image_latents = encode_entry(pipe, config, idx, synthetic_inputs, device)
         else:
             latents, image_latents = src["latents"].to(device).float().clone(), src["image_latents"]
+        if image_encoder is not None:
+            if inputs and "image_embeddings" in src:
+                logger.info("%s: image_embeddings of the inputs file is not read (--image_encoder_state_dict encodes "
+                            "the first frame)", config.video_name)
+            image_embeddings = image_embeddings_entry(pipe, config, idx, synthetic_inputs)
+        else:
+            image_embeddings = src["image_embeddings"]
         dt = unet.dtype
         pipe.invert(latents, src["prompt_embeds"].to(device, dt),
-                    src["image_embeddings"].to(device, dt), image_latents.to(device, dt),
+                    image_embeddings.to(device, dt), image_latents.to(device, dt),
                     torch.full((1,), int(inv.get("target_fps", 8)), dtype=torch.int64, device=device),
                     num_inference_steps=int(inv.n_steps), guidance_scale=float(inv.cfg), output_dir=out_dir,
                     max_steps=max_steps, keep=False)
@@ -155,6 +192,9 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--vae_state_dict", type=str, default=None,
                     help="AutoencoderKL state dict (.safetensors or torch file): encode <video_dir>/<video_name>/ "
                          "frames to the video and first-frame latents instead of reading them from --inputs")
+    ap.add_argument("--image_encoder_state_dict", type=str, default=None,
+                    help="CLIPVisionModelWithProjection state dict (.safetensors or torch file): encode the first "
+                         "frame of <video_dir>/<video_name>/ to image_embeddings instead of reading it from --inputs")
     return ap
 
 
@@ -163,4 +203,4 @@ if __name__ == "__main__":
     logging.basicConfig(level=logging.INFO)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # inverse.py:134
     main(args.template_config, args.configs_json, args.unet_state_dict, args.inputs, args.device, args.max_steps,
-         args.synthetic, args.vae_state_dict)
+         args.synthetic, args.vae_state_dict, args.image_encoder_state_dict)

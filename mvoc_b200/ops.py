@@ -185,6 +185,42 @@ def attention_d512(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: Opt
     return out
 
 
+CLIP_HEAD_DIM = 80
+
+
+def _bnh80_strides(t: torch.Tensor, what: str, heads: int):
+    """(batch, token, head) element strides of a [B, N, heads*80] view with a contiguous last dim."""
+    if t.dim() != 3 or t.shape[-1] != heads * CLIP_HEAD_DIM or t.stride(-1) != 1:
+        raise ValueError(f"attention_d80: {what} must be [B, N, {heads}*{CLIP_HEAD_DIM}] with a contiguous last dim, "
+                         f"got {tuple(t.shape)} strides {t.stride()}")
+    return t.stride(0), t.stride(1), CLIP_HEAD_DIM
+
+
+def attention_d80(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, scale: Optional[float] = None,
+                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """softmax(Q K^T * scale) V with head_dim 80 (the CLIP image tower's self-attention, mvoc_attn_d80_fwd):
+    q [B, Nq, H*80], k / v [B, Nk, H*80] (any batch / token strides, e.g. column slices of a fused QKV output)
+    -> [B, Nq, H*80]."""
+    _need_cuda(q, k, v, out)
+    if q.dim() != 3 or k.dim() != 3 or k.shape[0] != q.shape[0] or v.shape != k.shape:
+        raise ValueError(f"attention_d80: q {tuple(q.shape)} k {tuple(k.shape)} v {tuple(v.shape)} mismatch")
+    B, Nq, C = q.shape
+    Nk = k.shape[1]
+    if out is None:
+        out = torch.empty((B, Nq, C), dtype=q.dtype, device=q.device)
+    if tuple(out.shape) != (B, Nq, C) or out.dtype != q.dtype:
+        raise ValueError(f"attention_d80: out {tuple(out.shape)} {out.dtype} does not match q {tuple(q.shape)}")
+    st = [s for t, nm in ((q, "q"), (k, "k"), (v, "v"), (out, "out")) for s in _bnh80_strides(t, nm, heads)]
+    if scale is None:
+        scale = CLIP_HEAD_DIM ** -0.5
+    with _Timed(("attn_d80", B, heads, Nq, Nk), 4.0 * B * heads * Nq * Nk * CLIP_HEAD_DIM):
+        rc = _cabi.load().mvoc_attn_d80_fwd(q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), B, heads, Nq,
+                                            Nk, CLIP_HEAD_DIM, *st, float(scale), _dt(q), _stream())
+    _cabi.check(rc, "mvoc_attn_d80_fwd")
+    _count()
+    return out
+
+
 def temporal_attention(
     q: torch.Tensor,
     k: torch.Tensor,
@@ -676,6 +712,29 @@ def linear_geglu(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Ten
         rc = _cabi.load().mvoc_linear_geglu(x.data_ptr(), weight.data_ptr(), _ptr(bias), out.data_ptr(), M, K, F,
                                             _dt(x), int(v), _stream())
     _cabi.check(rc, "mvoc_linear_geglu")
+    _count()
+    return out
+
+
+def linear_gelu(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor] = None,
+                out: Optional[torch.Tensor] = None, variant: Optional[int] = None) -> torch.Tensor:
+    """out[..., N] = gelu(x[..., K] @ weight[N, K]^T (+ bias)) with the exact (erf) GELU in the tcgen05 GEMM epilogue
+    (mvoc_linear_gelu): the CLIP image tower's mlp.fc1 + activation."""
+    _need_cuda(x, weight, bias, out)
+    N, K = weight.shape
+    if x.shape[-1] != K or not weight.is_contiguous():
+        raise ValueError(f"linear_gelu: x {tuple(x.shape)} vs contiguous weight {tuple(weight.shape)}")
+    M, ldx = _rows(x, "linear_gelu x")
+    if out is None:
+        out = torch.empty(x.shape[:-1] + (N,), dtype=x.dtype, device=x.device)
+    Mo, ldo = _rows(out, "linear_gelu out")
+    if Mo != M or out.shape[-1] != N:
+        raise ValueError(f"linear_gelu: out {tuple(out.shape)} does not match [{M}, {N}]")
+    v = GEMM_VARIANT if variant is None else variant
+    with _Timed(("gemm", "gelu", M, K, N), 2.0 * M * K * N):
+        rc = _cabi.load().mvoc_linear_gelu(x.data_ptr(), weight.data_ptr(), _ptr(bias), out.data_ptr(), M, K, N, ldx,
+                                           ldo, _dt(x), int(v), _stream())
+    _cabi.check(rc, "mvoc_linear_gelu")
     _count()
     return out
 

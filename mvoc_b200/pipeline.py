@@ -8,7 +8,8 @@ hot path:
 CLIP / PIL work around the loops (:1356-1541, :1739-1748) is out of scope (SURVEY §2 #9): the loops take
 the tensors those stages produce (prompt embeds, CLIP image embeds, first-frame image latents, masks,
 inverted latents).  The VAE runs here when the pipeline is given one: ``decode_latents`` (decoder),
-``encode_vae_video`` and ``prepare_image_latents`` (encoder).  INTEGRATION.md shows the seam.
+``encode_vae_video`` and ``prepare_image_latents`` (encoder); so does the CLIP image tower (``encode_image``).
+INTEGRATION.md shows the seam.
 
 Per step the reference launches ~6 elementwise kernels per object for the fusion, a torch.cat, the
 CFG combine and ~10 scheduler kernels, reloads the source latents from disk and syncs twice
@@ -100,12 +101,13 @@ class Conditioning:
 
 class I2VGenXLPipeline:
     def __init__(self, unet, device="cuda", parallel=None, use_cuda_graphs: bool = False, vae=None,
-                 vae_encoder=None):
+                 vae_encoder=None, image_encoder=None):
         from .parallel import FrameParallel
 
         self.unet = unet
         self.vae = vae             # mvoc_b200.vae.AutoencoderKLDecoder for decode_latents, or None
         self.vae_encoder = vae_encoder   # mvoc_b200.vae.AutoencoderKLEncoder for encode_vae_video, or None
+        self.image_encoder = image_encoder   # mvoc_b200.clip.CLIPVisionEncoder for encode_image, or None
         self.device = torch.device(device)
         self.parallel = parallel or FrameParallel.single(self.device)
         # A UNet forward is ~2700 launches; enqueuing them from Python takes about as long as the GPU needs
@@ -178,6 +180,22 @@ class I2VGenXLPipeline:
             pos = pos.view(1, 1, -1, 1, 1).expand(lat.shape[0], lat.shape[1], -1, lat.shape[3], lat.shape[4])
             lat = torch.cat([lat, pos], dim=2)
         return lat
+
+    @torch.no_grad()
+    def encode_image(self, frames: torch.Tensor, encode_chunk_size: int = 64) -> torch.Tensor:
+        """I2VGenXLPipeline._encode_image (diffusers 0.27.2, called from pipelines/pipeline_i2vgen_xl.py:1391-1541):
+        CLIP-normalised images [B, 3, 224, 224] (mvoc_b200.clip.clip_image_input) -> image_embeds.unsqueeze(1)
+        [B, 1, 1024] in the encoder's dtype, `encode_chunk_size` images at a time (which bounds the activation
+        memory).  Every kernel of the tower computes an image's rows from that image alone and the GEMM's K order
+        does not depend on its tile plan, so the result is bit-identical for every chunk size (tested on the GPU)."""
+        if self.image_encoder is None:
+            raise RuntimeError("encode_image: this pipeline was built without a CLIP image encoder (image_encoder=None)")
+        if encode_chunk_size < 1:
+            raise ValueError(f"encode_image: encode_chunk_size={encode_chunk_size} must be >= 1")
+        frames = frames.to(self.device)
+        emb = torch.cat([self.image_encoder(frames[i:i + encode_chunk_size])
+                         for i in range(0, frames.shape[0], encode_chunk_size)])
+        return emb.unsqueeze(1)
 
     def drop_graphs(self) -> None:
         """Forget every captured graph.  The private pool goes with them: torch asserts when a capture re-uses a

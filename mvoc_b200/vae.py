@@ -224,11 +224,12 @@ def _read_state_dict(path: str) -> dict:
     return torch.load(path, map_location="cpu", weights_only=True)
 
 
-def _load_part(path: str, model_cls, part: str, ignore: tuple, device, dtype):
-    """One side of a diffusers AutoencoderKL state dict into `model_cls()`: keys under `ignore` (the other side) are
-    skipped; a missing or unexpected key, or a tensor of the wrong shape, raises an error that names it."""
+def _load_part(path: str, model_cls, part: str, ignore: tuple, device, dtype, kind: str = "VAE"):
+    """One side of a diffusers AutoencoderKL state dict (or another `kind` of checkpoint) into `model_cls()`: keys
+    under `ignore` (the other side) are skipped; a missing or unexpected key, or a tensor of the wrong shape, raises an
+    error that names it."""
     if not os.path.exists(path):
-        raise FileNotFoundError(f"VAE state dict {path!r} not found")
+        raise FileNotFoundError(f"{kind} state dict {path!r} not found")
     sd = _read_state_dict(path)
     with torch.device("meta"):
         model = model_cls()
