@@ -88,7 +88,8 @@ int mvoc_attn_fwd(const void* q, const void* k, const void* v, void* o,
  * This is the structure MVOC creates and the reference ignores: ModifiedSpaAttnProcessor writes the SAME blended
  * Q', K' into the uncond and the cond composite chunk (i2vgen-xl/pnp_utils.py:664-668) and then runs SDPA on
  * both (:684).  q, k: [B, N, H, D]; v, o: [B + pair_batches, N, H, D]; other arguments and the stride
- * requirements as mvoc_attn_fwd.
+ * requirements as mvoc_attn_fwd.  pair_batches >= B (MVOC_ERR_INVALID_ARG otherwise): with fewer, output batch
+ * b + pair_batches < B would be written by two CTAs.  Output batches in [B, pair_batches) are not written.
  */
 int mvoc_attn_pair_fwd(const void* q, const void* k, const void* v, void* o,
                        int B, int H, int Nq, int Nk, int D,

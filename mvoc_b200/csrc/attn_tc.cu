@@ -404,6 +404,8 @@ static int run(const void* q, const void* k, const void* v, void* o, int B, int 
     const int rows[3] = {BM, kv_rows, kv_rows};
     for (int i = 0; i < 3; ++i)   // all three before the first driver call
         if ((rc = check_map4(dims[i], str[i], what, name[i])) != MVOC_OK) return rc;
+    // CTA b writes O[b] and O[b + pair_batches]: below B, a second output batch is also written by another CTA
+    MVOC_REQUIRE(!pair || pair_batches >= B, MVOC_ERR_INVALID_ARG, "%s: pair_batches=%d < B=%d", what, pair_batches, B);
     CUtensorMap m[3];
     for (int i = 0; i < 3; ++i) {
         const int box[4] = {HD, 1, rows[i], 1};

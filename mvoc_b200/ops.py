@@ -120,6 +120,18 @@ def _bnc_strides(t: torch.Tensor, heads: int):
     return t.stride(0), t.stride(1), HEAD_DIM
 
 
+def _check_io(what: str, out: torch.Tensor, shape, *inputs: torch.Tensor) -> None:
+    """The kernels take one dtype code (q's) for every operand and write `shape` through `out`'s strides: inputs and
+    out must share q's dtype, and out must be exactly `shape` with a contiguous last dim."""
+    dt = inputs[0].dtype
+    for name, t in zip(("q", "k", "v", "out"), (*inputs, out)):
+        if t.dtype != dt:
+            raise ValueError(f"{what}: {name} is {t.dtype}, q is {dt}")
+    if tuple(out.shape) != tuple(shape) or out.stride(-1) != 1:
+        raise ValueError(f"{what}: out must be {tuple(shape)} with a contiguous last dim, got {tuple(out.shape)} "
+                         f"strides {out.stride()}")
+
+
 def attention(
     q: torch.Tensor,
     k: torch.Tensor,
@@ -137,6 +149,7 @@ def attention(
         raise ValueError(f"attention: q {tuple(q.shape)} k {tuple(k.shape)} v {tuple(v.shape)} mismatch")
     if out is None:
         out = torch.empty((B, Nq, C), dtype=q.dtype, device=q.device)
+    _check_io("attention", out, (B, Nq, C), q, k, v)
     if scale is None:
         scale = HEAD_DIM ** -0.5
     lib = _cabi.load()
@@ -174,6 +187,7 @@ def attention_d512(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: Opt
     B, N = q.shape[0], q.shape[1]
     if out is None:
         out = torch.empty((B, N, WIDE_HEAD_DIM), dtype=q.dtype, device=q.device)
+    _check_io("attention_d512", out, (B, N, WIDE_HEAD_DIM), q, k, v)
     st = [s for t, nm in ((q, "q"), (k, "k"), (v, "v"), (out, "out")) for s in _bn_strides(t, nm, B, N)]
     if scale is None:
         scale = WIDE_HEAD_DIM ** -0.5
@@ -208,8 +222,7 @@ def attention_d80(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int,
     Nk = k.shape[1]
     if out is None:
         out = torch.empty((B, Nq, C), dtype=q.dtype, device=q.device)
-    if tuple(out.shape) != (B, Nq, C) or out.dtype != q.dtype:
-        raise ValueError(f"attention_d80: out {tuple(out.shape)} {out.dtype} does not match q {tuple(q.shape)}")
+    _check_io("attention_d80", out, (B, Nq, C), q, k, v)
     st = [s for t, nm in ((q, "q"), (k, "k"), (v, "v"), (out, "out")) for s in _bnh80_strides(t, nm, heads)]
     if scale is None:
         scale = CLIP_HEAD_DIM ** -0.5
@@ -236,6 +249,7 @@ def temporal_attention(
         raise ValueError("temporal_attention: q, k, v must have the same shape")
     if out is None:
         out = torch.empty((P, T, C), dtype=q.dtype, device=q.device)
+    _check_io("temporal_attention", out, (P, T, C), q, k, v)
     if scale is None:
         scale = HEAD_DIM ** -0.5
     lib = _cabi.load()
@@ -288,14 +302,17 @@ def qk_blend_(
 def attention_pair(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, pair_batches: int,
                    scale: Optional[float] = None, out: Optional[torch.Tensor] = None, variant: int = 0) -> torch.Tensor:
     """Two branches that share Q and K (mvoc_attn_pair_fwd): q, k [B, N, H*64]; v [B + pair_batches, N, H*64];
-    out[b] = softmax(q[b] k[b]^T) v[b], out[b + pair_batches] = the same softmax times v[b + pair_batches]."""
+    out[b] = softmax(q[b] k[b]^T) v[b], out[b + pair_batches] = the same softmax times v[b + pair_batches].
+    pair_batches >= B (fewer would make two CTAs write one output batch); out batches [B, pair_batches) are not
+    written."""
     _need_cuda(q, k, v, out)
     B, Nq, C = q.shape
     Nk = k.shape[1]
-    if k.shape[0] != B or v.shape[0] != B + pair_batches or v.shape[1] != Nk or pair_batches < 1:
+    if k.shape[0] != B or v.shape[0] != B + pair_batches or v.shape[1] != Nk or pair_batches < B:
         raise ValueError(f"attention_pair: q {tuple(q.shape)} k {tuple(k.shape)} v {tuple(v.shape)} pair {pair_batches}")
     if out is None:
         out = torch.empty((B + pair_batches, Nq, C), dtype=q.dtype, device=q.device)
+    _check_io("attention_pair", out, (B + pair_batches, Nq, C), q, k, v)
     if scale is None:
         scale = HEAD_DIM ** -0.5
     with _Timed(("attn_pair", B, heads, Nq, Nk), 2 * 4.0 * B * heads * Nq * Nk * HEAD_DIM):
@@ -342,6 +359,7 @@ def attention_inject_(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mask: t
         raise ValueError(f"attention_inject_: mask must be contiguous [{n_obj}, {frames * pixels}]")
     if out is None:
         out = torch.empty((nb * frames, pixels, C), dtype=q.dtype, device=q.device)
+    _check_io("attention_inject_", out, (nb * frames, pixels, C), q, k, v)
     lds = [_token_rows(t, nm, nb * frames, pixels, C) for t, nm in ((q, "q"), (k, "k"), (v, "v"), (out, "out"))]
     if scale is None:
         scale = HEAD_DIM ** -0.5
@@ -632,6 +650,7 @@ def temporal_attention_frames(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
             raise ValueError(f"temporal_attention_frames: expected [{rows}, {C}] row-major views, got {tuple(t.shape)}")
     if out is None:
         out = torch.empty((rows, C), dtype=q.dtype, device=q.device)
+    _check_io("temporal_attention_frames", out, (rows, C), q, k, v)
     if scale is None:
         scale = HEAD_DIM ** -0.5
     st = []

@@ -1,5 +1,5 @@
-"""CLIP image tower on the GPU: mvoc_attn_d80_fwd against float64 attention, every compiled mvoc_linear_gelu kernel
-element by element against float64, the full-width encoder against transformers' CLIPVisionModelWithProjection in
+"""CLIP image tower on the GPU: mvoc_attn_d80_fwd's error codes, every compiled mvoc_linear_gelu kernel element by
+element against float64, the full-width encoder against transformers' CLIPVisionModelWithProjection in
 fp32 on the same random weights, chunk invariance, and the scripts' embeddings."""
 import json
 import os
@@ -23,47 +23,7 @@ def rel_l2(a, b):
 
 
 # ------------------------------------------------------------------ mvoc_attn_d80_fwd
-# Bars against float64 attention of the same 16-bit inputs: P is rounded to the storage type before P V and the output
-# once more, so the error is a few units of the storage type's rounding: relative L2 <= 8 u, and every element within
-# 32 u of the largest |ref| of its (batch, head) row block.
-ATTN_RTOL = {torch.bfloat16: 8 * 2.0 ** -8, torch.float16: 8 * 2.0 ** -11}
-ATTN_NS = [1, 77, 127, 128, 129, 257, 1024, 4096]
-ATTN_BH = {1: (3, 16), 77: (2, 5), 127: (1, 3), 128: (2, 2), 129: (3, 1), 257: (4, 16), 1024: (1, 4), 4096: (1, 2)}
-
-
-@pytest.mark.parametrize("fused", [False, True], ids=["separate", "fused_qkv"])
-@pytest.mark.parametrize("N", ATTN_NS)
-@pytest.mark.parametrize("dt", list(DTYPES))
-def test_attention_d80_vs_float64(cuda_device, dt, N, fused):
-    from mvoc_b200 import ops
-
-    dtype = DTYPES[dt]
-    B, H = ATTN_BH[N]
-    C = H * 80
-    torch.manual_seed(N + H + fused)
-    if fused:   # q, k, v: column slices of one [B, N, 3C] projection output; out: a column slice too (NaN beside it)
-        qkv = (torch.randn(B, N, 3 * C, device=cuda_device) * 1.5).to(dtype)
-        q, k, v = qkv[..., :C], qkv[..., C:2 * C], qkv[..., 2 * C:]
-        buf = torch.full((B, N, C + 64), float("nan"), dtype=dtype, device=cuda_device)
-        out = buf[..., :C]
-    else:
-        q, k, v = ((torch.randn(B, N, C, device=cuda_device) * 1.5).to(dtype) for _ in range(3))
-        buf, out = None, None
-    o = ops.attention_d80(q, k, v, H, out=out)
-    torch.cuda.synchronize()
-    sp = lambda t: t.double().reshape(B, N, H, 80).transpose(1, 2)
-    ref = F.scaled_dot_product_attention(sp(q), sp(k), sp(v), scale=80 ** -0.5).transpose(1, 2).reshape(B, N, C)
-    assert o.shape == (B, N, C) and o.dtype == dtype and torch.isfinite(o).all()
-    if buf is not None:
-        assert torch.isnan(buf[..., C:]).all(), "a write beside the output"
-    u = UNIT[dtype]
-    err = rel_l2(o, ref)
-    assert err <= ATTN_RTOL[dtype], f"rel L2 {err:.3e} > {ATTN_RTOL[dtype]:.3e}"
-    peak = ref.abs().reshape(B, N, H, 80).amax(dim=(1, 3), keepdim=True)
-    worst = float(((o.double() - ref).abs().reshape(B, N, H, 80) / peak).max())
-    assert worst <= 32 * u, f"max |err| / row-block peak {worst:.3e} > {32 * u:.3e}"
-
-
+# (element by element against float64 attention: tests/test_attention_matrix_gpu.py)
 def test_attention_d80_error_codes(cuda_device):
     from mvoc_b200 import _cabi, ops
 

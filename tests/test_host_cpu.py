@@ -103,6 +103,22 @@ def test_attention_rejects_zero_strides_where_the_extent_is_above_one(operand):
         assert refused(b"mvoc_attn_d512_fwd")
 
 
+def test_attention_pair_rejects_pair_batches_below_batches():
+    """CTA b writes output batches b and b + pair_batches, so pair_batches < B would make two CTAs write one output
+    batch: refused before any CUDA call by the pair entry and by the trace entry in pair mode."""
+    from mvoc_b200 import _cabi
+
+    lib = _cabi.load()
+    B, H, N = 3, 2, 128
+    st = [N * H * 64, H * 64, 64] * 4
+    for pb in (1, 2):
+        assert lib.mvoc_attn_pair_fwd(16, 16, 16, 16, B, H, N, N, 64, *st, pb, 0.125, 0, 0, None) == -1
+        assert b"mvoc_attn_pair_fwd: pair_batches" in lib.mvoc_last_error()
+        strides = (ctypes.c_int64 * 12)(*st)
+        assert lib.mvoc_attn_fwd_trace(16, 16, 16, 16, B, H, N, N, 64, strides, pb, 0.125, 0, 0, 16, None) == -1
+        assert b"mvoc_attn_fwd_trace: pair_batches" in lib.mvoc_last_error()
+
+
 def test_gemm_tile_plan_host_logic():
     """mvoc_gemm_plan (no device call): what the GEMM entries choose.  On B200 a tcgen05.mma costs the same whatever
     N <= 256 is, so the plan minimises the NUMBER of column tiles: full 256-wide tiles plus one narrower tail tile;
