@@ -100,6 +100,28 @@ int mvoc_attn_pair_fwd(const void* q, const void* k, const void* v, void* o,
                        int pair_batches, float scale, int dtype, int variant, void* stream);
 
 /*
+ * Causal attention forward at head_dim 64: O[r] = softmax(Q[r] K[0..r]^T * scale) V[0..r] for query row r.
+ * Replaces the self-attention of transformers' CLIPAttention with the causal mask in the CLIP text tower (16 heads of
+ * 64 over 77 tokens), reached from I2VGenXLPipeline.encode_prompt (diffusers 0.27.2) for the prompt, the negative
+ * prompt and the inversion prompt (no attention mask is passed: the pad positions are encoded too).
+ *
+ * Arguments and strides as mvoc_attn_fwd: q,o [B, Nq, H, D], k,v [B, Nk, H, D], D == 64 innermost and contiguous,
+ * strides in ELEMENTS for (batch, token, head), so q/k/v may be the three column slices of one fused QKV projection
+ * output [B*N, 3*H*64].  Nq == Nk (top-left and bottom-right alignment are then the same and no row is empty;
+ * MVOC_ERR_UNSUPPORTED otherwise), any N >= 1.  Key blocks above the diagonal are skipped, so the work is about half
+ * that of mvoc_attn_fwd at long N.  Tensor-core path; bf16 or fp16 (P is rounded to the storage type); the exp2 split
+ * of mvoc_attn_fwd's default variant.  Requirements and error codes as mvoc_attn_fwd: base pointers 16-byte aligned,
+ * strides non-negative multiples of 8, and positive along every dimension of extent > 1 (MVOC_ERR_UNSUPPORTED).
+ */
+int mvoc_attn_causal_fwd(const void* q, const void* k, const void* v, void* o,
+                         int B, int H, int Nq, int Nk, int D,
+                         int64_t q_sb, int64_t q_sn, int64_t q_sh,
+                         int64_t k_sb, int64_t k_sn, int64_t k_sh,
+                         int64_t v_sb, int64_t v_sn, int64_t v_sh,
+                         int64_t o_sb, int64_t o_sn, int64_t o_sh,
+                         float scale, int dtype, void* stream);
+
+/*
  * Diagnostics: mvoc_attn_fwd (pair_batches == 0) or mvoc_attn_pair_fwd with clock64() time stamps of CTA (0,0,0)
  * written to trace[key block * 8 + event] (device memory, int64): 0 softmax starts waiting for S, 1 S ready,
  * 2 row maximum known, 3 exponentials done, 4 P buffer free, 5 P published; 6 Q K^T issued, 7 P V issued.

@@ -36,6 +36,8 @@ SIGNATURES = {
         c_int,
         [c_void_p] * 4 + [c_int] * 5 + [c_int64] * 12 + [c_float, c_int, c_int, c_void_p],
     ),
+    "mvoc_attn_causal_fwd": (
+        c_int, [c_void_p] * 4 + [c_int] * 5 + [c_int64] * 12 + [c_float, c_int, c_void_p]),
     "mvoc_attn_fwd_trace": (
         c_int, [c_void_p] * 4 + [c_int] * 5 + [ctypes.POINTER(c_int64), c_int, c_float, c_int, c_int, c_void_p, c_void_p]),
     "mvoc_attn_d512_fwd": (

@@ -77,11 +77,14 @@ class CLIPVisionEmbeddings(nn.Module):
 
 
 class CLIPAttention(nn.Module):
-    def __init__(self, cfg: CLIPVisionConfig):
+    """Self-attention of both CLIP towers: dense at head_dim 80 (image) or causal at head_dim 64 (text, `causal`)."""
+
+    def __init__(self, cfg, causal: bool = False):
         super().__init__()
         d = cfg.hidden_size
         self.heads = cfg.num_attention_heads
         self.head_dim = d // self.heads
+        self.causal = causal
         self.k_proj = nn.Linear(d, d)
         self.v_proj = nn.Linear(d, d)
         self.q_proj = nn.Linear(d, d)
@@ -94,13 +97,13 @@ class CLIPAttention(nn.Module):
         w_qkv = derived(self, "w_qkv", ws, lambda: torch.cat(ws, dim=0).contiguous())
         b_qkv = derived(self, "b_qkv", bs, lambda: torch.cat(bs, dim=0).contiguous())
         qkv = ops.linear(h, w_qkv, b_qkv)
-        a = ops.attention_d80(qkv[..., :d], qkv[..., d:2 * d], qkv[..., 2 * d:], self.heads,
-                              scale=self.head_dim ** -0.5)
+        attend = ops.attention_causal if self.causal else ops.attention_d80
+        a = attend(qkv[..., :d], qkv[..., d:2 * d], qkv[..., 2 * d:], self.heads, scale=self.head_dim ** -0.5)
         return ops.linear(a, self.out_proj.weight, self.out_proj.bias, residual)
 
 
 class CLIPMLP(nn.Module):
-    def __init__(self, cfg: CLIPVisionConfig):
+    def __init__(self, cfg):
         super().__init__()
         self.fc1 = nn.Linear(cfg.hidden_size, cfg.intermediate_size)
         self.fc2 = nn.Linear(cfg.intermediate_size, cfg.hidden_size)
@@ -114,9 +117,9 @@ def _layernorm(ln: nn.LayerNorm, x: torch.Tensor) -> torch.Tensor:
 
 
 class CLIPEncoderLayer(nn.Module):
-    def __init__(self, cfg: CLIPVisionConfig):
+    def __init__(self, cfg, causal: bool = False):
         super().__init__()
-        self.self_attn = CLIPAttention(cfg)
+        self.self_attn = CLIPAttention(cfg, causal)
         self.layer_norm1 = nn.LayerNorm(cfg.hidden_size, eps=cfg.layer_norm_eps)
         self.mlp = CLIPMLP(cfg)
         self.layer_norm2 = nn.LayerNorm(cfg.hidden_size, eps=cfg.layer_norm_eps)
@@ -127,9 +130,9 @@ class CLIPEncoderLayer(nn.Module):
 
 
 class CLIPEncoder(nn.Module):
-    def __init__(self, cfg: CLIPVisionConfig):
+    def __init__(self, cfg, causal: bool = False):
         super().__init__()
-        self.layers = nn.ModuleList([CLIPEncoderLayer(cfg) for _ in range(cfg.num_hidden_layers)])
+        self.layers = nn.ModuleList([CLIPEncoderLayer(cfg, causal) for _ in range(cfg.num_hidden_layers)])
 
 
 class CLIPVisionTransformer(nn.Module):

@@ -30,6 +30,12 @@ from `edited_contorl_frame_path_background`, `edited_contorl_frame_path[j]` and 
 first frame when a path is a directory), each centre-cropped to (width, width), resized to 224 x 224 and
 CLIP-normalised.  Every other conditioning key still comes from `--conditioning`.  A missing control frame is an
 error; only `--synthetic` substitutes a seeded synthetic frame for it.
+
+With `--text_encoder_state_dict FILE` (a transformers CLIPTextModel state dict) and `--tokenizer_dir DIR` (the
+checkpoint's tokenizer/ folder) `prompt_embeds` [n+3,77,1024] is computed here from the entry's `prompt`,
+`negative_prompt` and `ddim_inv_prompt` in the branch order [inv x (n+1), negative, prompt] (SURVEY Appendix B #9),
+each distinct string encoded once.  The two flags go together; `--synthetic` never invents text weights or a
+vocabulary.  `image_latents_first` / `image_latents` still come from `--conditioning`.
 """
 from __future__ import annotations
 
@@ -162,12 +168,24 @@ def branch_image_embeddings(pipe, config, allow_synthetic: bool = False) -> torc
     return emb.expand(-1, T, -1).contiguous()
 
 
+def branch_prompt_embeds(pipe, config) -> torch.Tensor:
+    """prompt_embeds [n+3, 77, 1024] of one entry: encode_prompt of [ddim_inv_prompt x (n+1), negative_prompt,
+    prompt], each distinct string encoded once."""
+    from .clip_text import composition_prompt_embeds
+
+    return composition_prompt_embeds(pipe.encode_prompt, len(config.obj_mask_path), config.get("prompt", ""),
+                                     config.get("negative_prompt", ""), config.get("ddim_inv_prompt", ""))
+
+
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, conditioning: str = None,
          device: str = None, max_entries: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None,
-         image_encoder_state_dict: str = None):
+         image_encoder_state_dict: str = None, text_encoder_state_dict: str = None, tokenizer_dir: str = None):
+    from .clip_text import check_text_flags, load_text_tower
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
     from .vae import load_vae_decoder, save_frames
+
+    check_text_flags(text_encoder_state_dict, tokenizer_dir)
 
     template = cfgmod.load_template(template_config)
     device = torch.device(device or template.get("device", "cuda:0"))
@@ -186,7 +204,9 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
         from .clip import load_clip_image_encoder
 
         image_encoder = load_clip_image_encoder(image_encoder_state_dict, device)
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae=vae, image_encoder=image_encoder)
+    text_encoder, tokenizer = load_text_tower(text_encoder_state_dict, tokenizer_dir, device)
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae=vae, image_encoder=image_encoder,
+                            text_encoder=text_encoder, tokenizer=tokenizer)
     done = 0
     for config in cfgmod.iter_configs(template_config, configs_json):
         config = resolve_paths(config)
@@ -197,16 +217,20 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
             if not os.path.exists(cpath):
                 raise FileNotFoundError(f"conditioning file {cpath!r} not found")
             cond = torch.load(cpath, map_location="cpu")
-        if image_encoder is not None:
-            if cond is not None and "image_embeddings" in cond:
-                logger.info("%s: image_embeddings of the conditioning file is not read (--image_encoder_state_dict "
-                            "encodes the control frames)", config.video_name)
+        if image_encoder is not None or text_encoder is not None:
+            for key, flag, enc in (("image_embeddings", "--image_encoder_state_dict", image_encoder),
+                                   ("prompt_embeds", "--text_encoder_state_dict", text_encoder)):
+                if enc is not None and cond is not None and key in cond:
+                    logger.info("%s: %s of the conditioning file is not read (%s computes it)", config.video_name,
+                                key, flag)
             if cond is None and synthetic_inputs:   # the other keys stay synthetic
                 T, h, w = latent_geometry(config)
                 cond = synthetic.make_inputs(synthetic.Workload(config.video_name, "full", T, h, w,
                                                                 len(config.obj_mask_path)), [], None)
-            if cond is not None:
+            if cond is not None and image_encoder is not None:
                 cond = dict(cond, image_embeddings=branch_image_embeddings(pipe, config, synthetic_inputs))
+            if cond is not None and text_encoder is not None:
+                cond = dict(cond, prompt_embeds=branch_prompt_embeds(pipe, config))
         latents = run_entry(pipe, config, device, cond, allow_synthetic=synthetic_inputs)
         os.makedirs(config.output_dir, exist_ok=True)
         out = os.path.join(config.output_dir,
@@ -235,6 +259,12 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--image_encoder_state_dict", type=str, default=None,
                     help="CLIPVisionModelWithProjection state dict: encode the control frames to image_embeddings "
                          "instead of reading them from --conditioning")
+    ap.add_argument("--text_encoder_state_dict", type=str, default=None,
+                    help="CLIPTextModel state dict: encode the entry's prompt, negative_prompt and ddim_inv_prompt to "
+                         "prompt_embeds instead of reading them from --conditioning (needs --tokenizer_dir)")
+    ap.add_argument("--tokenizer_dir", type=str, default=None,
+                    help="the checkpoint's tokenizer/ folder (vocab.json, merges.txt, tokenizer_config.json / "
+                         "special_tokens_map.json) for --text_encoder_state_dict")
     ap.add_argument("--device", type=str, default=None)
     ap.add_argument("--max_entries", type=int, default=None)
     ap.add_argument("--synthetic", action="store_true",
@@ -247,4 +277,5 @@ if __name__ == "__main__":
     logging.basicConfig(level=logging.INFO)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # composite.py:246
     main(args.template_config, args.configs_json, args.unet_state_dict, args.conditioning, args.device,
-         args.max_entries, args.synthetic, args.vae_state_dict, args.image_encoder_state_dict)
+         args.max_entries, args.synthetic, args.vae_state_dict, args.image_encoder_state_dict,
+         args.text_encoder_state_dict, args.tokenizer_dir)

@@ -3,6 +3,11 @@
 // and inside diffusers' AttnProcessor2_0 (reached through attention_forward,
 // i2vgen-xl/pnp_utils.py:348-385) — non-causal, no mask, no dropout, D = 64.
 //
+// Causal mode (kCausal, mvoc_attn_causal_fwd; the CLIP text tower's self-attention): Nq == Nk, query row r sees keys
+// 0..r.  Query tile m needs key blocks 0..m only (BM == BN), so the producer, MMA and softmax warps all run
+// min(ceil(Nk/128), m + 1) blocks: blocks above the diagonal are never loaded, multiplied or exponentiated.  In the
+// diagonal block, columns past the row are set to -inf by the same register select as the tail mask.
+//
 // Pair mode (kNV = 2): MVOC writes the SAME blended Q', K' to the uncond and cond composite slots
 // (i2vgen-xl/pnp_utils.py:664-668), so their score matrices are identical: one CTA computes S and the softmax once
 // and multiplies P with BOTH value tiles (two O accumulators) — half the exponentials for those two branches.  It
@@ -71,7 +76,7 @@ __device__ __forceinline__ void trace_at(const Params& prm, int j, int ev) {
 }
 
 // kEmuMask: bit (k % 8) set => the k-th pair of a score row takes the FMA-pipe exp2 instead of the MUFU.
-template <typename T, int kBN, int kNV, int kStages, uint32_t kEmuMask>
+template <typename T, int kBN, int kNV, int kStages, uint32_t kEmuMask, bool kCausal>
 __global__ void __launch_bounds__(THREADS, 2)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                 const __grid_constant__ CUtensorMap tm_v, const Params prm) {
@@ -96,7 +101,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int m_blk = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
-    const int n_blocks = (prm.Nk + BN - 1) / BN;
+    static_assert(!kCausal || (kBN == BM && kNV == 1), "causal mode: plain attention on 128-key blocks");
+    // causal: query tile m_blk needs key blocks 0..m_blk only (the host checks Nq == Nk)
+    const int n_blocks = kCausal ? min((prm.Nk + BN - 1) / BN, m_blk + 1) : (prm.Nk + BN - 1) / BN;
 
     if (warp == 4 && lane == 0) {
         ptx::prefetch_tensormap(&tm_q);
@@ -218,7 +225,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
         float m_used = -INFINITY, l_sum = 0.0f;
         bool s_ready = false;   // S of the next block already seen complete by a non-blocking poll
         for (int j = 0; j < n_blocks; ++j) {
-            const int valid = min(BN, prm.Nk - j * BN);
+            // causal: in the diagonal block, column i is key m_blk*BM + i and must not exceed query row m_blk*BM + row
+            const int valid = kCausal && j == m_blk ? min(min(BN, prm.Nk - j * BN), row + 1) : min(BN, prm.Nk - j * BN);
             const bool tail = valid < BN;
             if (threadIdx.x == 0) trace_at(prm, j, 0);   // softmax of block j starts waiting for S
             if (!s_ready) ptx::mbar_wait(b_s_full, (uint32_t)j & 1u, 9);
@@ -237,7 +245,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
             ptx::tc_fence_before();
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(b_s_free);
-            if (tail) {  // keys past Nk (zero-filled by TMA) must not take part: exp2(-inf) = 0
+            if (tail) {  // keys past Nk (zero-filled by TMA) or, causal, past the row must not take part: exp2(-inf) = 0
 #pragma unroll
                 for (int i = 0; i < BN; ++i)
                     if (i >= valid) r[i] = 0xff800000u;
@@ -370,22 +378,23 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
 }
 
 // ------------------------------------------------------------------ host ---
-template <typename T, int kBN, int kNV, int kStages, uint32_t kEmuMask>
+template <typename T, int kBN, int kNV, int kStages, uint32_t kEmuMask, bool kCausal = false>
 static int launch(const CUtensorMap (&m)[3], const Params& prm, int B, int H, cudaStream_t s, const char* what) {
     using L = Smem<kBN, kNV, kStages>;
     static bool smem_set[64] = {false};
-    const int rc = set_max_dynamic_smem((const void*)attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask>, L::alloc,
+    const int rc = set_max_dynamic_smem((const void*)attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask, kCausal>, L::alloc,
                                         smem_set, what);
     if (rc != MVOC_OK) return rc;
     dim3 grid((prm.Nq + BM - 1) / BM, H, B);
-    attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask><<<grid, THREADS, L::alloc, s>>>(m[0], m[1], m[2], prm);
+    attn_fwd_kernel<T, kBN, kNV, kStages, kEmuMask, kCausal><<<grid, THREADS, L::alloc, s>>>(m[0], m[1], m[2], prm);
     return check_launch(what);
 }
 
 // Common entry: kNV value tensors per softmax (1 = plain attention, 2 = the uncond/cond pair).
+// causal: plain attention only (pair_batches == 0, variant 0), Nq == Nk.
 static int run(const void* q, const void* k, const void* v, void* o, int B, int H, int Nq, int Nk, int D,
                const int64_t (&st)[12], int pair_batches, float scale, int dtype, int variant, void* stream,
-               const char* what, long long* trace = nullptr) {
+               const char* what, long long* trace = nullptr, bool causal = false) {
     int rc = check_attn_operands(q, k, v, o, dtype, D, HD, st, 12, what);
     if (rc != MVOC_OK) return rc;
     MVOC_REQUIRE(B > 0 && H > 0 && Nq > 0 && Nk > 0, MVOC_ERR_INVALID_ARG, "%s: empty problem B=%d H=%d Nq=%d Nk=%d", what,
@@ -393,6 +402,8 @@ static int run(const void* q, const void* k, const void* v, void* o, int B, int 
     MVOC_REQUIRE(B <= 65535 && H <= 65535, MVOC_ERR_UNSUPPORTED, "%s: B=%d / H=%d exceed the grid limits", what, B, H);
     MVOC_REQUIRE(variant >= 0 && variant <= 5, MVOC_ERR_INVALID_ARG, "%s: unknown variant %d", what, variant);
     MVOC_REQUIRE(pair_batches >= 0, MVOC_ERR_INVALID_ARG, "%s: pair_batches=%d", what, pair_batches);
+    MVOC_REQUIRE(!causal || Nq == Nk, MVOC_ERR_UNSUPPORTED, "%s: causal attention needs Nq == Nk, got Nq=%d Nk=%d",
+                 what, Nq, Nk);
     const bool pair = pair_batches > 0;
     const int kv_rows = pair ? 64 : 128;
     // q, k, v: [B, N, H, 64] viewed innermost first with element strides (sh, sn, sb); box = one head's 64 columns of
@@ -424,6 +435,10 @@ static int run(const void* q, const void* k, const void* v, void* o, int B, int 
     prm.scale_log2 = scale * 1.4426950408889634f;
     prm.trace = trace;
     cudaStream_t s = (cudaStream_t)stream;
+    if (causal) {
+        if (dtype == MVOC_F16) return launch<__half, 128, 1, 3, 0xA8u, true>(m, prm, B, H, s, what);
+        return launch<__nv_bfloat16, 128, 1, 3, 0xA8u, true>(m, prm, B, H, s, what);
+    }
     // variants (same results up to the exp2 approximation; the tests run all of them):
     //   1, 2: all exponentials on the MUFU;  3 / 4 / 5: 2 / 3 / 4 of every 8 pairs on the FMA-pipe polynomial;  0: default
     const uint32_t emu = variant == 1 || variant == 2 ? 0x00u : variant == 3 ? 0x88u : variant == 5 ? 0xAAu : 0xA8u;
@@ -473,6 +488,15 @@ extern "C" int mvoc_attn_fwd(const void* q, const void* k, const void* v, void* 
                              int dtype, int variant, void* stream) {
     const int64_t st[12] = {q_sb, q_sn, q_sh, k_sb, k_sn, k_sh, v_sb, v_sn, v_sh, o_sb, o_sn, o_sh};
     return attn::run(q, k, v, o, B, H, Nq, Nk, D, st, 0, scale, dtype, variant, stream, "mvoc_attn_fwd");
+}
+
+extern "C" int mvoc_attn_causal_fwd(const void* q, const void* k, const void* v, void* o, int B, int H, int Nq,
+                                    int Nk, int D, int64_t q_sb, int64_t q_sn, int64_t q_sh, int64_t k_sb, int64_t k_sn,
+                                    int64_t k_sh, int64_t v_sb, int64_t v_sn, int64_t v_sh, int64_t o_sb, int64_t o_sn,
+                                    int64_t o_sh, float scale, int dtype, void* stream) {
+    const int64_t st[12] = {q_sb, q_sn, q_sh, k_sb, k_sn, k_sh, v_sb, v_sn, v_sh, o_sb, o_sn, o_sh};
+    return attn::run(q, k, v, o, B, H, Nq, Nk, D, st, 0, scale, dtype, 0, stream, "mvoc_attn_causal_fwd", nullptr,
+                     true);
 }
 
 extern "C" int mvoc_attn_pair_fwd(const void* q, const void* k, const void* v, void* o, int B, int H,

@@ -20,15 +20,20 @@ With `--vae_state_dict FILE` (a diffusers AutoencoderKL state dict) the video la
 latents are computed here, as inverse.py:143-153 and :49-55 do: the first `n_frames` .png / .jpg files of
 `<video_dir>/<video_name>/` are centre-cropped to `image_size` and encoded with one
 `torch.Generator().manual_seed(seed)` per entry, first the video (`encode_vae_video`), then the first frame
-(`prepare_image_latents`).  `--inputs` then only needs prompt_embeds and image_embeddings (CLIP stays out of scope;
-so does the reference's mp4 fallback, :154-165).  With `--synthetic` and no frame directory, seeded synthetic
-frames are encoded; the encoder weights always come from FILE.
+(`prepare_image_latents`).  `--inputs` then only needs prompt_embeds and image_embeddings (unless the CLIP flags
+below compute them; the reference's mp4 fallback, :154-165, stays out of scope).  With `--synthetic` and no frame
+directory, seeded synthetic frames are encoded; the encoder weights always come from FILE.
 
 With `--image_encoder_state_dict FILE` (a transformers CLIPVisionModelWithProjection state dict) `image_embeddings`
 [1,1,1024] is computed here from the first frame of the same directory: centre-cropped to (width, width), resized to
 224 x 224 and CLIP-normalised (mvoc_b200.clip.clip_image_input), then encoded on the library's kernels.  It works with
 or without `--vae_state_dict`; with both, `--inputs` only needs prompt_embeds.  `--synthetic` without a frame
 directory encodes the first seeded synthetic frame.
+
+With `--text_encoder_state_dict FILE` (a transformers CLIPTextModel state dict) and `--tokenizer_dir DIR` (the
+checkpoint's tokenizer/ folder) `prompt_embeds` [1,77,1024] is `encode_prompt(inverse_config.prompt)` (batch 1: the
+inversion runs at cfg 1.0).  The two flags go together; `--synthetic` never invents text weights or a vocabulary.
+With the VAE, image and text flags all given, every input is computed here and `--inputs` is not needed.
 
 Independent videos are the unit of multi-GPU work here: with torchrun, entry i goes to rank i % world_size
 (replicas, no collective).
@@ -104,9 +109,12 @@ def image_embeddings_entry(pipe, config, idx: int, synthetic_inputs: bool) -> to
 
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, inputs: str = None,
          device: str = None, max_steps: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None,
-         image_encoder_state_dict: str = None):
+         image_encoder_state_dict: str = None, text_encoder_state_dict: str = None, tokenizer_dir: str = None):
+    from .clip_text import check_text_flags, load_text_tower
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
+
+    check_text_flags(text_encoder_state_dict, tokenizer_dir)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -132,7 +140,10 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
         from .clip import load_clip_image_encoder
 
         image_encoder = load_clip_image_encoder(image_encoder_state_dict, device)
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae_encoder=vae_encoder, image_encoder=image_encoder)
+    text_encoder, tokenizer = load_text_tower(text_encoder_state_dict, tokenizer_dir, device)
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae_encoder=vae_encoder, image_encoder=image_encoder,
+                            text_encoder=text_encoder, tokenizer=tokenizer)
+    computes_all = vae_encoder is not None and image_encoder is not None and text_encoder is not None
     done = 0
     for idx, config in enumerate(cfgmod.iter_configs(template_config, configs_json)):
         if idx % world != rank:
@@ -150,11 +161,14 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
             if not os.path.exists(ipath):
                 raise FileNotFoundError(f"inversion inputs {ipath!r} not found")
             src = torch.load(ipath, map_location="cpu")
+        elif computes_all:
+            src = {}                                                            # every input is computed below
         elif synthetic_inputs:
             src = synthetic.make_inversion_inputs(wl, idx)
         else:
-            raise FileNotFoundError("no --inputs file (VAE / CLIP outputs are inputs of this script); pass "
-                                    "--synthetic for seeded synthetic tensors")
+            raise FileNotFoundError("no --inputs file (VAE / CLIP outputs are inputs of this script unless "
+                                    "--vae_state_dict, --image_encoder_state_dict and --text_encoder_state_dict with "
+                                    "--tokenizer_dir compute them all); pass --synthetic for seeded synthetic tensors")
         if vae_encoder is not None:
             if inputs and any(k in src for k in ("latents", "image_latents")):
                 logger.info("%s: latents / image_latents of the inputs file are not read (--vae_state_dict encodes "
@@ -169,8 +183,15 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
             image_embeddings = image_embeddings_entry(pipe, config, idx, synthetic_inputs)
         else:
             image_embeddings = src["image_embeddings"]
+        if text_encoder is not None:
+            if inputs and "prompt_embeds" in src:
+                logger.info("%s: prompt_embeds of the inputs file is not read (--text_encoder_state_dict encodes "
+                            "inverse_config.prompt)", config.video_name)
+            prompt_embeds = pipe.encode_prompt([inv.get("prompt", "")])           # [1, 77, 1024]
+        else:
+            prompt_embeds = src["prompt_embeds"]
         dt = unet.dtype
-        pipe.invert(latents, src["prompt_embeds"].to(device, dt),
+        pipe.invert(latents, prompt_embeds.to(device, dt),
                     image_embeddings.to(device, dt), image_latents.to(device, dt),
                     torch.full((1,), int(inv.get("target_fps", 8)), dtype=torch.int64, device=device),
                     num_inference_steps=int(inv.n_steps), guidance_scale=float(inv.cfg), output_dir=out_dir,
@@ -195,6 +216,12 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--image_encoder_state_dict", type=str, default=None,
                     help="CLIPVisionModelWithProjection state dict (.safetensors or torch file): encode the first "
                          "frame of <video_dir>/<video_name>/ to image_embeddings instead of reading it from --inputs")
+    ap.add_argument("--text_encoder_state_dict", type=str, default=None,
+                    help="CLIPTextModel state dict (.safetensors or torch file): encode inverse_config.prompt to "
+                         "prompt_embeds instead of reading it from --inputs (needs --tokenizer_dir)")
+    ap.add_argument("--tokenizer_dir", type=str, default=None,
+                    help="the checkpoint's tokenizer/ folder (vocab.json, merges.txt, tokenizer_config.json / "
+                         "special_tokens_map.json) for --text_encoder_state_dict")
     return ap
 
 
@@ -203,4 +230,5 @@ if __name__ == "__main__":
     logging.basicConfig(level=logging.INFO)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # inverse.py:134
     main(args.template_config, args.configs_json, args.unet_state_dict, args.inputs, args.device, args.max_steps,
-         args.synthetic, args.vae_state_dict, args.image_encoder_state_dict)
+         args.synthetic, args.vae_state_dict, args.image_encoder_state_dict, args.text_encoder_state_dict,
+         args.tokenizer_dir)

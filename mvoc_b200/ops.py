@@ -166,6 +166,31 @@ def attention(
     return out
 
 
+def attention_causal(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, scale: Optional[float] = None,
+                     out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Causal softmax(Q K^T * scale) V with head_dim 64 (the CLIP text tower's self-attention, mvoc_attn_causal_fwd):
+    query row r attends to keys 0..r.  q, k, v [B, N, H*64] (any batch / token strides, e.g. column slices of a fused
+    QKV output) -> [B, N, H*64]."""
+    _need_cuda(q, k, v, out)
+    if q.dim() != 3 or q.shape != k.shape or v.shape != k.shape:
+        raise ValueError(f"attention_causal: q {tuple(q.shape)} k {tuple(k.shape)} v {tuple(v.shape)} must be one "
+                         "[B, N, H*64] shape")
+    B, N, C = q.shape
+    if out is None:
+        out = torch.empty((B, N, C), dtype=q.dtype, device=q.device)
+    _check_io("attention_causal", out, (B, N, C), q, k, v)
+    if scale is None:
+        scale = HEAD_DIM ** -0.5
+    with _Timed(("attn_causal", B, heads, N), 2.0 * B * heads * N * (N + 1) * HEAD_DIM):
+        rc = _cabi.load().mvoc_attn_causal_fwd(
+            q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), B, heads, N, N, HEAD_DIM,
+            *_bnc_strides(q, heads), *_bnc_strides(k, heads), *_bnc_strides(v, heads), *_bnc_strides(out, heads),
+            float(scale), _dt(q), _stream())
+    _cabi.check(rc, "mvoc_attn_causal_fwd")
+    _count()
+    return out
+
+
 WIDE_HEAD_DIM = 512
 
 

@@ -101,13 +101,15 @@ class Conditioning:
 
 class I2VGenXLPipeline:
     def __init__(self, unet, device="cuda", parallel=None, use_cuda_graphs: bool = False, vae=None,
-                 vae_encoder=None, image_encoder=None):
+                 vae_encoder=None, image_encoder=None, text_encoder=None, tokenizer=None):
         from .parallel import FrameParallel
 
         self.unet = unet
         self.vae = vae             # mvoc_b200.vae.AutoencoderKLDecoder for decode_latents, or None
         self.vae_encoder = vae_encoder   # mvoc_b200.vae.AutoencoderKLEncoder for encode_vae_video, or None
         self.image_encoder = image_encoder   # mvoc_b200.clip.CLIPVisionEncoder for encode_image, or None
+        self.text_encoder = text_encoder     # mvoc_b200.clip_text.CLIPTextEncoder for encode_prompt, or None
+        self.tokenizer = tokenizer           # mvoc_b200.clip_text.CLIPTokenizer for encode_prompt, or None
         self.device = torch.device(device)
         self.parallel = parallel or FrameParallel.single(self.device)
         # A UNet forward is ~2700 launches; enqueuing them from Python takes about as long as the GPU needs
@@ -196,6 +198,23 @@ class I2VGenXLPipeline:
         emb = torch.cat([self.image_encoder(frames[i:i + encode_chunk_size])
                          for i in range(0, frames.shape[0], encode_chunk_size)])
         return emb.unsqueeze(1)
+
+    @torch.no_grad()
+    def encode_prompt(self, prompts, encode_chunk_size: int = 64) -> torch.Tensor:
+        """I2VGenXLPipeline.encode_prompt (diffusers 0.27.2) for one prompt list, clip_skip None: each prompt (None
+        becomes "") is tokenized to 77 ids (padding "max_length", truncation) and encoded by the text tower without an
+        attention mask -> last_hidden_state [n, 77, 1024] in the encoder's dtype, `encode_chunk_size` prompts at a time.
+        As in encode_image, every kernel computes a prompt's rows from that prompt alone, so the result is
+        bit-identical for every chunk size (tested on the GPU)."""
+        if self.text_encoder is None or self.tokenizer is None:
+            raise RuntimeError("encode_prompt: this pipeline was built without a CLIP text encoder and tokenizer "
+                               "(text_encoder=None or tokenizer=None)")
+        if encode_chunk_size < 1:
+            raise ValueError(f"encode_prompt: encode_chunk_size={encode_chunk_size} must be >= 1")
+        prompts = [prompts] if prompts is None or isinstance(prompts, str) else list(prompts)
+        ids = self.tokenizer(["" if p is None else p for p in prompts]).to(self.device)
+        return torch.cat([self.text_encoder(ids[i:i + encode_chunk_size])
+                          for i in range(0, ids.shape[0], encode_chunk_size)])
 
     def drop_graphs(self) -> None:
         """Forget every captured graph.  The private pool goes with them: torch asserts when a capture re-uses a
