@@ -311,6 +311,13 @@ int mvoc_geglu(const void* x, void* y, int64_t M, int F, int dtype, void* stream
 int mvoc_upsample_nearest2x_nhwc(const void* x, void* y, int64_t N, int H, int W, int C, int dtype, void* stream);
 
 /*
+ * Channel concatenation of two channels-last activations a [rows, CA], b [rows, CB] -> y [rows, CA + CB]: the
+ * skip-connection torch.cat before every resnet of the up blocks (diffusers UNet3D up blocks, reached from
+ * i2vgen-xl/pipelines/pipeline_i2vgen_xl.py:318-350).  A copy, bit-identical to torch.cat.  CA, CB % 8 == 0.
+ */
+int mvoc_concat_lastdim(const void* a, const void* b, void* y, int64_t rows, int CA, int CB, int dtype, void* stream);
+
+/*
  * ---- dense work on tcgen05 tensor cores (csrc/gemm_tc.cu) ------------------------------------------------
  * One persistent implicit-GEMM kernel: 128-row activation tiles are TMA boxes of the channels-last tensor
  * (shifted per filter tap, zero-filled outside = the padding), weights are K-major [tap, Cout, Cin], fp32

@@ -65,6 +65,7 @@ SIGNATURES = {
     "mvoc_gemm_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, ctypes.POINTER(c_int), ctypes.POINTER(c_int),
                                ctypes.POINTER(c_int)]),
     "mvoc_upsample_nearest2x_nhwc": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p]),
+    "mvoc_concat_lastdim": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]),
     "mvoc_layernorm": (c_int, [c_void_p] * 4 + [c_int64, c_int, c_float, c_int, c_void_p]),
     "mvoc_qk_blend": (
         c_int,

@@ -35,6 +35,16 @@ checkpoint's tokenizer/ folder) `prompt_embeds` [1,77,1024] is `encode_prompt(in
 inversion runs at cfg 1.0).  The two flags go together; `--synthetic` never invents text weights or a vocabulary.
 With the VAE, image and text flags all given, every input is computed here and `--inputs` is not needed.
 
+With `recon_config.enable_recon: true` an entry is also reconstructed after its inversion (also when the inversion was
+skipped as complete), the reference's sanity check (inverse.py:192-227): the noisiest stored latents of
+`recon_config.ddim_latents_path` (utils.load_ddim_latents_at_T) are sampled back with the plain I2VGenXL loop
+(`I2VGenXLPipeline.sample`, `recon_config.n_steps` steps, guidance `recon_config.cfg`) under the entry's own
+conditioning, and the result is written to `<recon_config.output_dir>/recon_latents.pt`.  Under guidance the negative
+prompt is `encode_prompt(inverse_config.negative_prompt)` with the text flags, else `negative_prompt_embeds` of
+`--inputs` (seeded under `--synthetic`).  With `--vae_state_dict` the result is also decoded to `recon_frames/NNN.png`
+(the decoder is read from the same file as the encoder).  `--synthetic` writes `.synthetic` names, and `--max_steps`
+caps the sampling loop as it caps the inversion.
+
 Independent videos are the unit of multi-GPU work here: with torchrun, entry i goes to rank i % world_size
 (replicas, no collective).
 """
@@ -50,6 +60,11 @@ from . import config as cfgmod
 from . import synthetic
 
 logger = logging.getLogger(__name__)
+
+# recon_config defaults when the merged entry lacks the keys: diffusers' I2VGenXLPipeline.__call__ defaults (the
+# reference's own values could not be read); the template states them and an entry overrides them
+RECON_STEPS = 50
+RECON_CFG = 9.0
 
 
 def inversion_complete(out_dir: str, n_steps: int) -> bool:
@@ -141,8 +156,8 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
 
         image_encoder = load_clip_image_encoder(image_encoder_state_dict, device)
     text_encoder, tokenizer = load_text_tower(text_encoder_state_dict, tokenizer_dir, device)
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae_encoder=vae_encoder, image_encoder=image_encoder,
-                            text_encoder=text_encoder, tokenizer=tokenizer)
+    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=device.type == "cuda", vae_encoder=vae_encoder,
+                            image_encoder=image_encoder, text_encoder=text_encoder, tokenizer=tokenizer)
     computes_all = vae_encoder is not None and image_encoder is not None and text_encoder is not None
     done = 0
     for idx, config in enumerate(cfgmod.iter_configs(template_config, configs_json)):
@@ -150,9 +165,13 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
             continue                                                            # one video per GPU
         inv = config.inverse_config
         out_dir = inv.output_dir
-        if inversion_complete(out_dir, int(inv.n_steps)) and not config.get("force_recompute_latents", False):
+        recon = config.get("recon_config") or {}
+        do_recon = bool(recon.get("enable_recon", False))
+        skip = inversion_complete(out_dir, int(inv.n_steps)) and not config.get("force_recompute_latents", False)
+        if skip:
             logger.info("%s is complete: skipping (force_recompute_latents is false)", out_dir)   # inverse.py:181-183
-            continue
+            if not do_recon:
+                continue
         w_px, h_px = inv.image_size
         wl = synthetic.Workload(config.video_name, "full", int(inv.n_frames), int(h_px) // 8, int(w_px) // 8, 0,
                                 inversion_steps=int(inv.n_steps))
@@ -191,13 +210,57 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, i
         else:
             prompt_embeds = src["prompt_embeds"]
         dt = unet.dtype
-        pipe.invert(latents, prompt_embeds.to(device, dt),
-                    image_embeddings.to(device, dt), image_latents.to(device, dt),
-                    torch.full((1,), int(inv.get("target_fps", 8)), dtype=torch.int64, device=device),
-                    num_inference_steps=int(inv.n_steps), guidance_scale=float(inv.cfg), output_dir=out_dir,
-                    max_steps=max_steps, keep=False)
-        done += 1
+        prompt_embeds, image_embeddings = prompt_embeds.to(device, dt), image_embeddings.to(device, dt)
+        image_latents = image_latents.to(device, dt)
+        fps = torch.full((1,), int(inv.get("target_fps", 8)), dtype=torch.int64, device=device)
+        negative = None
+        if do_recon and float(recon.get("cfg", RECON_CFG)) > 1.0:    # checked before the inversion is spent
+            if text_encoder is not None:
+                negative = pipe.encode_prompt([inv.get("negative_prompt", "")])
+            elif "negative_prompt_embeds" in src:
+                negative = src["negative_prompt_embeds"].to(device, dt)
+            else:
+                raise KeyError(f"{config.video_name}: recon_config.cfg > 1 (classifier-free guidance) needs "
+                               "negative_prompt_embeds in the --inputs file, or --text_encoder_state_dict with "
+                               "--tokenizer_dir to encode inverse_config.negative_prompt")
+        if not skip:
+            pipe.invert(latents, prompt_embeds, image_embeddings, image_latents, fps,
+                        num_inference_steps=int(inv.n_steps), guidance_scale=float(inv.cfg), output_dir=out_dir,
+                        max_steps=max_steps, keep=False)
+            done += 1
+        if do_recon:
+            reconstruct(pipe, recon, prompt_embeds, negative, image_embeddings, image_latents, fps, device,
+                        vae_state_dict, synthetic_inputs, max_steps)
     return done
+
+
+def reconstruct(pipe, recon, prompt_embeds, negative_prompt_embeds, image_embeddings, image_latents, fps, device,
+                vae_state_dict: str = None, synthetic_inputs: bool = False, max_steps: int = None) -> torch.Tensor:
+    """The reconstruction check of one entry (the reference's inverse.py:192-227): plain sampling (pipe.sample) from
+    the noisiest stored latents of `recon.ddim_latents_path` with `recon.n_steps` and guidance `recon.cfg`; writes
+    `<recon.output_dir>/recon_latents.pt` and, with a VAE file, the decoded frames to `recon_frames/` (`.synthetic`
+    names under --synthetic, as composite.py does).  Returns the final latents."""
+    from .utils import load_ddim_latents_at_T
+
+    x_T = load_ddim_latents_at_T(recon.ddim_latents_path).float()              # utils.py:39-45, fp16 on disk
+    latents = pipe.sample(prompt_embeds, negative_prompt_embeds, image_embeddings, image_latents, fps,
+                          num_inference_steps=int(recon.get("n_steps", RECON_STEPS)),
+                          guidance_scale=float(recon.get("cfg", RECON_CFG)), latents=x_T, max_steps=max_steps)
+    out_dir = recon.get("output_dir") or os.path.join(os.path.dirname(os.path.normpath(recon.ddim_latents_path)),
+                                                      "recon")
+    os.makedirs(out_dir, exist_ok=True)
+    out = os.path.join(out_dir, "recon_latents.synthetic.pt" if synthetic_inputs else "recon_latents.pt")
+    torch.save(latents.detach().cpu(), out)
+    logger.info("saved %s", out)
+    if vae_state_dict:
+        from .vae import load_vae_decoder, save_frames
+
+        if pipe.vae is None:
+            pipe.vae = load_vae_decoder(vae_state_dict, device)                 # the same file as the encoder's
+        frames_dir = os.path.join(out_dir, "recon_frames.synthetic" if synthetic_inputs else "recon_frames")
+        save_frames(pipe.decode_latents(latents)[0], frames_dir)
+        logger.info("saved %s", frames_dir)
+    return latents
 
 
 def build_parser() -> argparse.ArgumentParser:

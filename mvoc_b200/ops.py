@@ -643,6 +643,25 @@ def upsample_nearest2x(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> t
     return out
 
 
+def concat_lastdim(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    """torch.cat([a, b], dim=-1) of two contiguous channels-last tensors [..., CA], [..., CB] (the up blocks' skip
+    connections): one library copy kernel, bit-identical to torch.cat."""
+    _need_cuda(a, b)
+    if not (a.is_contiguous() and b.is_contiguous()) or a.shape[:-1] != b.shape[:-1] or a.dtype != b.dtype:
+        raise ValueError(f"concat_lastdim: need contiguous tensors of one dtype with equal leading dims, got "
+                         f"{tuple(a.shape)} {a.dtype} and {tuple(b.shape)} {b.dtype}")
+    CA, CB = a.shape[-1], b.shape[-1]
+    out = torch.empty(tuple(a.shape[:-1]) + (CA + CB,), dtype=a.dtype, device=a.device)
+    rows = a.numel() // CA
+    if rows == 0:
+        return out                    # nothing to copy (an empty tensor has no data pointer to hand the kernel)
+    with _Timed(("concat_lastdim", rows, CA, CB), 2.0 * out.numel() * out.element_size()):
+        _cabi.check(_cabi.load().mvoc_concat_lastdim(a.data_ptr(), b.data_ptr(), out.data_ptr(), rows, CA, CB, _dt(a),
+                                                     _stream()), "mvoc_concat_lastdim")
+    _count()
+    return out
+
+
 def layernorm(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, eps: float,
               out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Row-wise LayerNorm over the last dim of a contiguous [..., C] tensor (warp per row)."""

@@ -123,7 +123,7 @@ class I2VGenXLPipeline:
         self._static_in = {}
         self.scheduler: Optional[DDIMSchedule] = None
         self._cond_caches = {}     # id(cond) -> {"key": cond (strong ref), "ctx", "il", "fps_emb"}; a few conditionings
-
+        self._plain_in = {}        # latent shape -> 4-slot input buffer of `sample`
 
     @torch.no_grad()
     def decode_latents(self, latents: torch.Tensor, decode_chunk_size: int = 4) -> torch.Tensor:
@@ -450,6 +450,90 @@ class I2VGenXLPipeline:
             if on_step is not None:
                 on_step(t, x)
         return saved
+
+    # ------------------------------------------------------------------ plain sampling
+    def _plain_input(self, latents: torch.Tensor, nb: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(4-slot buffer, UNet input [nb, 4, T, h, w]) of `sample` (nb = 2 under guidance, else 1).  The input is
+        the tail of a persistent 4-slot buffer that ONE mvoc_latent_composite launch fills from the fp32 latents
+        (background, one source branch, uncond, cond: all four are the latents), so the cast and the batch copy are
+        a library kernel.  The tail is registered as the static input of its shape: captured graphs read it
+        without a further copy."""
+        shape = tuple(latents.shape[1:])
+        buf = self._plain_in.get(shape)
+        if buf is None:
+            buf = torch.empty((4,) + shape, dtype=self.unet.dtype, device=latents.device)
+            self._plain_in[shape] = buf
+        view = buf[4 - nb:]
+        key = (nb,) + shape
+        old = self._static_in.get(key)
+        if old is None or old.data_ptr() != view.data_ptr():
+            if old is not None:
+                self.drop_graphs()       # graphs captured on the old buffer would read stale input
+            self._static_in[key] = view
+        return buf, self._static_in[key]
+
+    @torch.no_grad()
+    def sample(
+        self,
+        prompt_embeds: torch.Tensor,
+        negative_prompt_embeds: Optional[torch.Tensor],
+        image_embeddings: torch.Tensor,
+        image_latents: torch.Tensor,
+        fps: torch.Tensor,
+        num_inference_steps: int = 50,
+        guidance_scale: float = 9.0,
+        latents: Optional[torch.Tensor] = None,
+        generator: Optional[torch.Generator] = None,
+        max_steps: Optional[int] = None,
+        callback: Optional[Callable] = None,
+    ) -> torch.Tensor:
+        """Plain I2VGenXL sampling, diffusers 0.27.2 ``I2VGenXLPipeline.__call__`` steps 3-7 (the reference's
+        pipelines/pipeline_i2vgen_xl.py:980-1216 derives from it): stock UNet, classifier-free guidance, DDIM.
+
+        Tensors come in the shapes `invert` takes: prompt / negative embeds [1,77,1024], CLIP image embeddings
+        [1,1,1024], first-frame image latents [1,4,T,h,w], fps [1].  Guidance is on when guidance_scale > 1; the
+        UNet batch is then [uncond, cond]: prompt embeds [negative, prompt], image embeddings [zeros, emb]
+        (_encode_image), the image latents and fps twice.  At guidance_scale <= 1 it is batch 1, like `invert`.
+        `latents` [1,4,T,h,w] is the start (used as fp32; the caller's tensor is not modified); None draws
+        torch.randn((1,4,T,h,w)) in fp32 on the generator's device.  Either is scaled by init_noise_sigma
+        (prepare_latents; 1.0 for DDIM).
+        Returns the final latents [1,4,T,h,w] fp32.  The plain path is the stock forward: MVOC injection hooks
+        installed on the UNet are an error, not something to fire silently."""
+        if any(pnp_utils.injection_installed(self.unet)):
+            raise ValueError("sample: MVOC injection hooks are installed on this UNet (init_pnp / register_*); the "
+                             "plain sampling loop runs the stock forward, so use a pipeline without them")
+        cfg = guidance_scale > 1.0                                              # do_classifier_free_guidance
+        if cfg and negative_prompt_embeds is None:
+            raise ValueError(f"sample: guidance_scale={guidance_scale} > 1 needs negative_prompt_embeds")
+        dev, dt = self.device, self.unet.dtype
+        sched = DDIMSchedule(num_inference_steps)
+        b, c, T, h, w = image_latents.shape
+        if latents is None:                                                     # prepare_latents
+            latents = torch.randn((1, 4, T, h, w), generator=generator, dtype=torch.float32,
+                                  device=generator.device if generator is not None else dev)
+        x = latents.to(dev, torch.float32) * sched.init_noise_sigma             # scales given latents too (a copy)
+        prompt_embeds, image_embeddings = prompt_embeds.to(dev, dt), image_embeddings.to(dev, dt)
+        image_latents, fps = image_latents.to(dev, dt), fps.to(dev)
+        if cfg:
+            prompt_embeds = torch.cat([negative_prompt_embeds.to(dev, dt), prompt_embeds])
+            image_embeddings = torch.cat([torch.zeros_like(image_embeddings), image_embeddings])
+            image_latents = torch.cat([image_latents, image_latents])
+            fps = torch.cat([fps, fps])
+        cond = Conditioning(prompt_embeds, image_embeddings, image_latents, image_latents, fps)
+        slots, unet_in = self._plain_input(x, 2 if cfg else 1)
+        for i, t in enumerate(sched.timesteps):
+            if max_steps is not None and i >= max_steps:
+                break
+            # slots <- [x, x, x, x] in the UNet dtype.  z, bg and objs alias one buffer, which the kernel's __restrict__
+            # pointers allow only because it never writes z when do_fusion is off (csrc/latent.cu): keep that so.
+            ops.latent_composite_(x, x, x, None, slots, 0.0, False)
+            noise_pred = self._unet_forward(unet_in, t, cond)
+            pred = self._gather_prediction(noise_pred)
+            a_t, a_prev = sched.step_alphas(t)
+            ops.cfg_ddim_step_(pred[0], pred[1] if cfg else None, x, guidance_scale, a_t, a_prev)
+            if callback is not None:
+                callback(i, t, x)
+        return x
 
 
 # --------------------------------------------------------------------------

@@ -319,18 +319,35 @@ def register_time_all(model, t, mask):
         setattr(m, "mask", mask)
 
 
-def hook_signature(unet) -> tuple:
-    """Which hooks fire at the `t` last pushed by register_time_all — the control-flow key of one UNet
-    forward (CUDA-graph capture in mvoc_b200.pipeline is keyed on it)."""
+def _hook_sites(unet, pred) -> tuple:
+    """One bool per hook site, in one fixed order: whether the site carries an injection hook and `pred(site)`."""
     sig = []
     blk = unet.up_blocks[-1]
     for m in list(blk.resnets) + list(blk.temp_convs) + [unet.conv_out]:
-        sig.append(getattr(m, "feature_hook", None) is not None and hasattr(m, "t") and _fires(m))
+        sig.append(getattr(m, "feature_hook", None) is not None and pred(m))
     for bi, li in injected_attention_sites(unet):
         for grp in ("attentions", "temp_attentions"):
             p = getattr(unet.up_blocks[bi], grp)[li].transformer_blocks[0].attn1.processor
-            sig.append(isinstance(p, _InjectingProcessor) and hasattr(p, "t") and _fires(p))
+            sig.append(isinstance(p, _InjectingProcessor) and pred(p))
     return tuple(sig)
+
+
+def hook_signature(unet) -> tuple:
+    """Which hooks fire at the `t` last pushed by register_time_all — the control-flow key of one UNet
+    forward (CUDA-graph capture in mvoc_b200.pipeline is keyed on it)."""
+    return _hook_sites(unet, lambda m: hasattr(m, "t") and _fires(m))
+
+
+def _scheduled(obj) -> bool:
+    sched = getattr(obj, "injection_schedule", None)
+    return sched is not None and len(sched) > 0
+
+
+def injection_installed(unet) -> tuple:
+    """Per hook site of hook_signature (the same walk, the same order): whether an injection hook with a non-empty
+    schedule is installed, whatever `t` was pushed last.  The plain sampling loop (I2VGenXLPipeline.sample) refuses a
+    UNet where any is."""
+    return _hook_sites(unet, _scheduled)
 
 
 def register_time(model, t):

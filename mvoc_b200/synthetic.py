@@ -135,7 +135,8 @@ def make_inputs(wl: Workload, timesteps: List[int], alphas_cumprod) -> dict:
 
 def make_inversion_inputs(wl: Workload, video_index: int = 0) -> dict:
     """Inputs of pipe.invert for one synthetic source video (inverse.py:48-76): clean latents x0,
-    empty-prompt embeds, one CLIP embedding, first-frame image latents; batch 1 (cfg 1.0 => no CFG)."""
+    empty-prompt embeds, one CLIP embedding, first-frame image latents; batch 1 (cfg 1.0 => no CFG).  The negative
+    prompt embeds are read only by the guided reconstruction (recon_config)."""
     T, h, w = wl.n_frames, wl.latent_h, wl.latent_w
     return {
         "latents": _randn((1, 4, T, h, w), 3000 + video_index) * 0.18215 * 4.0,
@@ -143,4 +144,5 @@ def make_inversion_inputs(wl: Workload, video_index: int = 0) -> dict:
         "image_embeddings": _randn((1, 1, 1024), 3200 + video_index),
         "image_latents": _image_latents(2, T, h, w, 33 + video_index)[:1],
         "fps": torch.full((1,), wl.target_fps, dtype=torch.int64),
+        "negative_prompt_embeds": _randn((1, 77, 1024), 3300 + video_index),
     }

@@ -86,12 +86,31 @@ class _Ctx:
     def __init__(self):
         self.parallel = None   # mvoc_b200.parallel.FrameParallel or None
         self.full_hw = None    # (h, w) of the un-sharded frame while a temporal operator runs on pixel shards
+        self.temb_act = None   # (emb, SiLU(emb)) of the running forward: every resnet's time_emb_proj reads the same
 
 
 # MVOC_DENSE=lib sends the dense work to cuDNN / cuBLAS instead of this repo's tcgen05 kernels: the A/B baseline
 # of bench.py (recorded in its `switches`), never the product configuration.
 _DENSE_TC = os.environ.get("MVOC_DENSE", "tc") != "lib"
 _TC_DTYPES = (torch.bfloat16, torch.float16)
+
+
+def _temb_act(ctx: Optional[_Ctx], temb: torch.Tensor) -> torch.Tensor:
+    """SiLU(temb) of a resnet's time_emb_proj (pnp_utils.py:941-948).  Every resnet of one UNet forward gets the same
+    temb, so I2VGenXLUNet.body computes the SiLU once and the resnets read it (the same values: one launch instead of
+    one per resnet)."""
+    act = ctx.temb_act if ctx is not None else None
+    return act[1] if act is not None and act[0] is temb else F.silu(temb)
+
+
+def cat_channels(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    """torch.cat([a, b], dim=-1) of two channels-last activations (the up blocks' skip connections): the library's
+    copy kernel (mvoc_concat_lastdim, bit-identical) on the bf16 / fp16 product path, like Upsample2D's; the fp32
+    host-layer tests run torch.cat."""
+    if a.dtype in _TC_DTYPES and a.is_contiguous() and b.is_contiguous() and a.shape[-1] % 8 == 0 \
+            and b.shape[-1] % 8 == 0:
+        return ops.concat_lastdim(a, b)
+    return torch.cat([a, b], dim=-1)
 
 
 def derived(module: nn.Module, name: str, sources, build):
@@ -459,7 +478,7 @@ class ResnetBlock2D(nn.Module):
         n, H, W, cin = input_tensor.shape
         h = self.norm1(input_tensor, silu=True)                                 # :909-910
         h = conv_nhwc(h, self.conv1)                                            # :939
-        t = None if self.time_emb_proj is None else self.time_emb_proj(F.silu(temb))   # :941-948
+        t = None if self.time_emb_proj is None else self.time_emb_proj(_temb_act(self.ctx, temb))   # :941-948
         h = self.norm2(h, silu=True, add=t, out=h)                              # `+ temb` :952 fused into norm2 :953, :965
         if self.conv_shortcut is None:
             if self.feature_hook is None:
@@ -689,7 +708,7 @@ class CrossAttnUpBlock3D(_Block3D):
                                                       self.temp_attentions):
             res = res_hidden_states_tuple[-1]
             res_hidden_states_tuple = res_hidden_states_tuple[:-1]
-            hidden_states = torch.cat([hidden_states, res], dim=-1)
+            hidden_states = cat_channels(hidden_states, res)
             hidden_states = resnet(hidden_states, temb)
             hidden_states = temp_conv(hidden_states, num_frames=num_frames)
             hidden_states = attn(hidden_states, encoder_hidden_states=encoder_hidden_states)[0]
@@ -710,7 +729,7 @@ class UpBlock3D(_Block3D):
         for resnet, temp_conv in zip(self.resnets, self.temp_convs):
             res = res_hidden_states_tuple[-1]
             res_hidden_states_tuple = res_hidden_states_tuple[:-1]
-            hidden_states = torch.cat([hidden_states, res], dim=-1)
+            hidden_states = cat_channels(hidden_states, res)
             hidden_states = resnet(hidden_states, temb)
             hidden_states = temp_conv(hidden_states, num_frames=num_frames)
         if self.upsamplers is not None:
@@ -869,6 +888,13 @@ class I2VGenXLUNet(nn.Module):
     def body(self, sample, emb, context_emb, num_frames, forward_upsample_size):
         """down / mid / up / out, pipeline_i2vgen_xl.py:292-357, on channels-last [(b t), h, w, C].
         Returns the noise prediction as [(b t), 4, h, w] (contiguous NCHW)."""
+        self.ctx.temb_act = (emb, F.silu(emb))                                  # read by every resnet
+        try:
+            return self._body(sample, emb, context_emb, num_frames, forward_upsample_size)
+        finally:
+            self.ctx.temb_act = None
+
+    def _body(self, sample, emb, context_emb, num_frames, forward_upsample_size):
         upsample_size = None
         res_samples = (sample,)
         for blk in self.down_blocks:
