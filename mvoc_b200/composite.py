@@ -10,10 +10,9 @@ masks (utils.mask_preprocess) and runs the 50-step composition loop
 (pipelines/pipeline_i2vgen_xl.py:1636-1734) on the GPU.  The final latents are written to
 `<output_dir>/composite_latents.pt`.
 
-Out of scope here (SURVEY §2 #9, #10): CLIP / VAE encode.  The tensors those stages produce are read from
-`--conditioning file.pt` (a dict with prompt_embeds [n+3,77,1024], image_embeddings [n+3,T,1024],
-image_latents_first / image_latents [n+3,4,T,h,w]); the path may contain `{video_name}` / `{edited_video_name}`
-so that every config entry gets its own file.  Missing inverted latents, masks or conditioning are ERRORS, like
+The conditioning tensors not computed by the flags below are read from `--conditioning file.pt` (a dict with
+prompt_embeds [n+3,77,1024], image_embeddings [n+3,T,1024], image_latents_first / image_latents [n+3,4,T,h,w]); the
+path may contain `{video_name}` / `{edited_video_name}` so that every config entry gets its own file.  Missing inverted latents, masks or conditioning are ERRORS, like
 the reference's asserts (utils.py:34, composite.py:246).  Only with `--synthetic` are seeded synthetic tensors
 of the right shape substituted (mvoc_b200.synthetic) — the offline end-to-end exercise of the config → hooks →
 loop path; the output is then written as `composite_latents.synthetic.pt`.  UNet weights come from
@@ -28,14 +27,35 @@ With `--image_encoder_state_dict FILE` (a transformers CLIPVisionModelWithProjec
 [n+3,T,1024] is computed here in the branch order [bg, objs..., zeros, main] (pipelines/pipeline_i2vgen_xl.py:766-767)
 from `edited_contorl_frame_path_background`, `edited_contorl_frame_path[j]` and `edited_contorl_frame_path_main` (the
 first frame when a path is a directory), each centre-cropped to (width, width), resized to 224 x 224 and
-CLIP-normalised.  Every other conditioning key still comes from `--conditioning`.  A missing control frame is an
-error; only `--synthetic` substitutes a seeded synthetic frame for it.
+CLIP-normalised.  A missing control frame is an error; only `--synthetic` substitutes a seeded synthetic frame for
+it.
 
 With `--text_encoder_state_dict FILE` (a transformers CLIPTextModel state dict) and `--tokenizer_dir DIR` (the
 checkpoint's tokenizer/ folder) `prompt_embeds` [n+3,77,1024] is computed here from the entry's `prompt`,
 `negative_prompt` and `ddim_inv_prompt` in the branch order [inv x (n+1), negative, prompt] (SURVEY Appendix B #9),
 each distinct string encoded once.  The two flags go together; `--synthetic` never invents text weights or a
-vocabulary.  `image_latents_first` / `image_latents` still come from `--conditioning`.
+vocabulary.
+
+With `--encode_image_latents` (needs `--vae_state_dict`, whose encoder half is then loaded too) `image_latents_first`
+= `image_latents` [n+3,4,T,h,w] are computed here in the branch order [bg, objs..., main, main] from the first frame of
+the same control-frame paths: each centre-cropped to image_size, encoded together by prepare_image_latents under one
+`torch.Generator().manual_seed(seed)`.  The flag is opt-in: `--vae_state_dict` alone only decodes.  A key computed
+here replaces the conditioning file's (logged).  With `--encode_image_latents`, `--image_encoder_state_dict` and the
+text flags together every conditioning key is computed and `--conditioning` is not needed (fps comes from the
+config's target_fps); otherwise a missing key is an error that names it.
+
+Frame-parallel over the GPUs of one node, every active entry in turn over all ranks:
+
+    python -m torch.distributed.run --nproc-per-node N -m mvoc_b200.composite --template_config ... --configs_json ...
+
+Every rank owns n_frames / N frames of all n+3 branches (mvoc_b200.parallel.FrameParallel, the NVLink peer exchange
+around the temporal operators); n_frames must divide by N, which is checked on every rank before any collective.
+Every rank reads the same inputs and computes the same conditioning; under `--synthetic` rank 0's random-init UNet
+weights are broadcast to the others.  The prediction is all-gathered before each DDIM update, so every rank ends with
+the full latents; rank 0 writes composite_latents.pt, and with `--vae_state_dict` every rank decodes and writes its own
+frames under their global numbers.  The peer-exchange arena is sized for the largest entry
+(parallel.exchange_arena_mb; MVOC_EXCHANGE_ARENA_MB overrides it).  Without torchrun (or with N = 1) nothing of this
+runs.
 """
 from __future__ import annotations
 
@@ -140,16 +160,15 @@ def run_entry(pipe, config, device, conditioning=None, allow_synthetic: bool = F
         obj_ddim_latents_idx_offset=list(config.obj_ddim_latents_idx_offset)[:n_obj] or None)
 
 
-def branch_image_embeddings(pipe, config, allow_synthetic: bool = False) -> torch.Tensor:
-    """image_embeddings [n+3, T, 1024] of one entry in the branch order [bg, objs..., zeros, main] (SURVEY Appendix B
-    #9; pipelines/pipeline_i2vgen_xl.py:766-767).  The reference encodes every frame of every branch, T x (n+2) CLIP
-    calls, but the UNet reads only image_embeddings[:, 0:1] (mvoc_b200/unet3d.py, I2VGenXLUNet.context), so ONE
-    embedding per branch from its control frame, repeated over T, gives the UNet the same input with n+2 calls."""
+def control_frames(config, allow_synthetic: bool = False) -> list:
+    """The first frame (PIL, RGB) of each branch's control frames in the order [bg, objs..., main]:
+    `edited_contorl_frame_path_background`, `edited_contorl_frame_path[j]` and `edited_contorl_frame_path_main`, each a
+    file or a directory of frames.  A missing one raises FileNotFoundError unless allow_synthetic, which substitutes a
+    seeded uint8 noise frame of `image_size`."""
     from PIL import Image
 
-    from .clip import clip_image_input, first_frame
+    from .clip import first_frame
 
-    T = int(config.n_frames)
     w_px, h_px = (int(v) for v in config.image_size)
     paths = ([config.edited_contorl_frame_path_background] + list(config.edited_contorl_frame_path)
              + [config.edited_contorl_frame_path_main])
@@ -163,9 +182,38 @@ def branch_image_embeddings(pipe, config, allow_synthetic: bool = False) -> torc
         logger.warning("control frame %s not found: using a seeded synthetic frame (--synthetic)", p)
         g = torch.Generator().manual_seed(7000 + i)
         images.append(Image.fromarray(torch.randint(0, 256, (h_px, w_px, 3), generator=g, dtype=torch.uint8).numpy()))
+    return images
+
+
+def branch_image_embeddings(pipe, config, allow_synthetic: bool = False) -> torch.Tensor:
+    """image_embeddings [n+3, T, 1024] of one entry in the branch order [bg, objs..., zeros, main] (SURVEY Appendix B
+    #9; pipelines/pipeline_i2vgen_xl.py:766-767).  The reference encodes every frame of every branch, T x (n+2) CLIP
+    calls, but the UNet reads only image_embeddings[:, 0:1] (mvoc_b200/unet3d.py, I2VGenXLUNet.context), so ONE
+    embedding per branch from its control frame, repeated over T, gives the UNet the same input with n+2 calls."""
+    from .clip import clip_image_input
+
+    T = int(config.n_frames)
+    w_px = int(config.image_size[0])
+    images = control_frames(config, allow_synthetic)
     emb = pipe.encode_image(clip_image_input(images, w_px))                      # [n+2, 1, 1024]
     emb = torch.cat([emb[:-1], torch.zeros_like(emb[:1]), emb[-1:]])           # [bg, objs, zeros, main]
     return emb.expand(-1, T, -1).contiguous()
+
+
+def branch_image_latents(pipe, config, allow_synthetic: bool = False) -> torch.Tensor:
+    """image_latents [n+3, 4, T, h, w] fp32 of one entry in the branch order [bg, objs..., main, main] (SURVEY
+    Appendix B #9; the CFG doubling duplicates main; the composition uses the same tensor as image_latents_first).
+    Each branch's first control frame is centre-cropped to image_size (center_crop_wide) and the n+2 distinct frames
+    go through prepare_image_latents together, under one torch.Generator().manual_seed(seed): one posterior noise
+    draw over the n+2 images in branch order."""
+    from .vae import center_crop_wide, pil_to_model_input
+
+    T = int(config.n_frames)
+    size = tuple(int(v) for v in config.image_size)
+    images = [center_crop_wide(im, size) for im in control_frames(config, allow_synthetic)]
+    x = pil_to_model_input(images).to(pipe.device)
+    lat = pipe.prepare_image_latents(x, T, torch.Generator().manual_seed(int(config.seed)))   # [n+2, 4, T, h, w]
+    return torch.cat([lat, lat[-1:]])
 
 
 def branch_prompt_embeds(pipe, config) -> torch.Tensor:
@@ -177,39 +225,94 @@ def branch_prompt_embeds(pipe, config) -> torch.Tensor:
                                      config.get("negative_prompt", ""), config.get("ddim_inv_prompt", ""))
 
 
+CONDITIONING_KEYS = ("prompt_embeds", "image_embeddings", "image_latents_first", "image_latents")
+
+
+def check_frame_split(configs, world: int) -> None:
+    """Frame-parallel composition gives every rank n_frames / world frames of an entry: an entry whose n_frames the
+    rank count does not divide is an error, raised on every rank (they all read the same configs) before any
+    collective, so that no rank waits for another."""
+    for config in configs:
+        T = int(config.n_frames)
+        if T % world != 0:
+            raise ValueError(f"{config.video_name}: n_frames={T} is not divisible by WORLD_SIZE={world} (every rank "
+                             "composes n_frames / WORLD_SIZE frames)")
+
+
 def main(template_config: str, configs_json: str, unet_state_dict: str = None, conditioning: str = None,
          device: str = None, max_entries: int = None, synthetic_inputs: bool = False, vae_state_dict: str = None,
-         image_encoder_state_dict: str = None, text_encoder_state_dict: str = None, tokenizer_dir: str = None):
-    from .clip_text import check_text_flags, load_text_tower
+         image_encoder_state_dict: str = None, text_encoder_state_dict: str = None, tokenizer_dir: str = None,
+         encode_image_latents: bool = False):
+    from .clip_text import check_text_flags
+    from .parallel import FrameParallel, exchange_arena_mb
+
+    check_text_flags(text_encoder_state_dict, tokenizer_dir)
+    if encode_image_latents and not vae_state_dict:
+        raise ValueError("--encode_image_latents needs --vae_state_dict: the VAE encoder is read from that file")
+
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    local = int(os.environ.get("LOCAL_RANK", "0"))
+    template = cfgmod.load_template(template_config)
+    device = torch.device(device or (f"cuda:{local}" if world > 1 else template.get("device", "cuda:0")))
+    configs = [resolve_paths(c) for c in cfgmod.iter_configs(template_config, configs_json)]
+    if max_entries is not None:
+        configs = configs[:max_entries]
+    if device.type == "cuda":
+        torch.cuda.set_device(device)      # the C-ABI launches on the current device (mvoc_b200.ops._need_cuda)
+    arena_mb = None
+    if world > 1:
+        check_frame_split(configs, world)
+        arena_mb = max((exchange_arena_mb(len(c.obj_mask_path) + 3, *latent_geometry(c), world) for c in configs),
+                       default=None)
+    par = FrameParallel.from_env(device, arena_mb=arena_mb)            # world_size 1 => no process group
+    try:
+        return _run(configs, par, device, unet_state_dict, conditioning, synthetic_inputs, vae_state_dict,
+                    image_encoder_state_dict, text_encoder_state_dict, tokenizer_dir, encode_image_latents)
+    finally:
+        par.shutdown()                     # no process group or IPC mapping outlives the run
+
+
+def _run(configs, par, device, unet_state_dict, conditioning, synthetic_inputs, vae_state_dict,
+         image_encoder_state_dict, text_encoder_state_dict, tokenizer_dir, encode_image_latents) -> int:
+    from .clip_text import load_text_tower
     from .pipeline import I2VGenXLPipeline
     from .unet3d import I2VGenXLUNet, UNetConfig, prepare
     from .vae import load_vae_decoder, save_frames
 
-    check_text_flags(text_encoder_state_dict, tokenizer_dir)
-
-    template = cfgmod.load_template(template_config)
-    device = torch.device(device or template.get("device", "cuda:0"))
-    if device.type == "cuda":
-        torch.cuda.set_device(device)      # the C-ABI launches on the current device (mvoc_b200.ops._need_cuda)
     torch.set_grad_enabled(False)                                               # composite.py:253
     unet = I2VGenXLUNet(UNetConfig.full()).eval().requires_grad_(False)
     if unet_state_dict:
         unet.load_state_dict(torch.load(unet_state_dict, map_location="cpu"), strict=True)
     elif not synthetic_inputs:
         raise FileNotFoundError("--unet_state_dict is required (pass --synthetic to run on random-init weights)")
-    unet = prepare(unet.to(device=device, dtype=torch.bfloat16))
+    unet = unet.to(device=device, dtype=torch.bfloat16)
+    if not unet_state_dict:
+        par.broadcast_module(unet)         # random-init weights: rank 0's on every rank
+    unet = prepare(unet)
     vae = load_vae_decoder(vae_state_dict, device) if vae_state_dict else None
+    vae_encoder = None
+    if encode_image_latents:
+        from .vae import load_vae_encoder
+
+        vae_encoder = load_vae_encoder(vae_state_dict, device)
     image_encoder = None
     if image_encoder_state_dict:
         from .clip import load_clip_image_encoder
 
         image_encoder = load_clip_image_encoder(image_encoder_state_dict, device)
     text_encoder, tokenizer = load_text_tower(text_encoder_state_dict, tokenizer_dir, device)
-    pipe = I2VGenXLPipeline(unet, device, use_cuda_graphs=True, vae=vae, image_encoder=image_encoder,
-                            text_encoder=text_encoder, tokenizer=tokenizer)
+    pipe = I2VGenXLPipeline(unet, device, parallel=par, use_cuda_graphs=device.type == "cuda", vae=vae,
+                            vae_encoder=vae_encoder, image_encoder=image_encoder, text_encoder=text_encoder,
+                            tokenizer=tokenizer)
+    computes = {}                          # conditioning key -> the flag that computes it
+    if image_encoder is not None:
+        computes["image_embeddings"] = "--image_encoder_state_dict"
+    if text_encoder is not None:
+        computes["prompt_embeds"] = "--text_encoder_state_dict"
+    if vae_encoder is not None:
+        computes.update(image_latents_first="--encode_image_latents", image_latents="--encode_image_latents")
     done = 0
-    for config in cfgmod.iter_configs(template_config, configs_json):
-        config = resolve_paths(config)
+    for config in configs:
         logger.info("Processing %s / %s", config.video_name, config.edited_video_name)
         cond = None
         if conditioning:
@@ -217,34 +320,47 @@ def main(template_config: str, configs_json: str, unet_state_dict: str = None, c
             if not os.path.exists(cpath):
                 raise FileNotFoundError(f"conditioning file {cpath!r} not found")
             cond = torch.load(cpath, map_location="cpu")
-        if image_encoder is not None or text_encoder is not None:
-            for key, flag, enc in (("image_embeddings", "--image_encoder_state_dict", image_encoder),
-                                   ("prompt_embeds", "--text_encoder_state_dict", text_encoder)):
-                if enc is not None and cond is not None and key in cond:
+        if computes:
+            for key, flag in computes.items():
+                if cond is not None and key in cond:
                     logger.info("%s: %s of the conditioning file is not read (%s computes it)", config.video_name,
                                 key, flag)
-            if cond is None and synthetic_inputs:   # the other keys stay synthetic
-                T, h, w = latent_geometry(config)
-                cond = synthetic.make_inputs(synthetic.Workload(config.video_name, "full", T, h, w,
-                                                                len(config.obj_mask_path)), [], None)
-            if cond is not None and image_encoder is not None:
+            if cond is None:
+                if synthetic_inputs:       # the keys not computed stay synthetic
+                    T, h, w = latent_geometry(config)
+                    cond = synthetic.make_inputs(synthetic.Workload(config.video_name, "full", T, h, w,
+                                                                    len(config.obj_mask_path)), [], None)
+                elif len(computes) == len(CONDITIONING_KEYS):
+                    cond = {}              # every key is computed below; fps comes from the config
+                else:
+                    missing = [k for k in CONDITIONING_KEYS if k not in computes]
+                    raise FileNotFoundError(f"no --conditioning file for {config.video_name}, and no flag computes "
+                                            f"{', '.join(missing)} (image_embeddings: --image_encoder_state_dict; "
+                                            "prompt_embeds: --text_encoder_state_dict with --tokenizer_dir; "
+                                            "image_latents_first / image_latents: --encode_image_latents)")
+            if image_encoder is not None:
                 cond = dict(cond, image_embeddings=branch_image_embeddings(pipe, config, synthetic_inputs))
-            if cond is not None and text_encoder is not None:
+            if text_encoder is not None:
                 cond = dict(cond, prompt_embeds=branch_prompt_embeds(pipe, config))
+            if vae_encoder is not None:
+                il = branch_image_latents(pipe, config, synthetic_inputs)
+                cond = dict(cond, image_latents_first=il, image_latents=il)
         latents = run_entry(pipe, config, device, cond, allow_synthetic=synthetic_inputs)
-        os.makedirs(config.output_dir, exist_ok=True)
-        out = os.path.join(config.output_dir,
-                           "composite_latents.synthetic.pt" if synthetic_inputs else "composite_latents.pt")
-        torch.save(latents.detach().cpu(), out)
-        logger.info("saved %s", out)
+        if par.rank == 0:
+            os.makedirs(config.output_dir, exist_ok=True)
+            out = os.path.join(config.output_dir,
+                               "composite_latents.synthetic.pt" if synthetic_inputs else "composite_latents.pt")
+            torch.save(latents.detach().cpu(), out)
+            logger.info("saved %s", out)
         if vae is not None:
+            # every rank decodes and writes its own frames, under their global numbers
             frames_dir = os.path.join(config.output_dir,
                                       "composite_frames.synthetic" if synthetic_inputs else "composite_frames")
-            save_frames(pipe.decode_latents(latents)[0], frames_dir)
+            f0, f1 = par.frame_range(latents.shape[2])
+            save_frames(pipe.decode_latents(latents[:, :, f0:f1])[0], frames_dir, first_index=f0)
             logger.info("saved %s", frames_dir)
         done += 1
-        if max_entries is not None and done >= max_entries:
-            break
+    par.barrier()                          # every rank's frames are on disk when the command returns
     return done
 
 
@@ -265,6 +381,9 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--tokenizer_dir", type=str, default=None,
                     help="the checkpoint's tokenizer/ folder (vocab.json, merges.txt, tokenizer_config.json / "
                          "special_tokens_map.json) for --text_encoder_state_dict")
+    ap.add_argument("--encode_image_latents", action="store_true",
+                    help="encode each branch's first control frame with the VAE encoder of --vae_state_dict to "
+                         "image_latents_first / image_latents instead of reading them from --conditioning")
     ap.add_argument("--device", type=str, default=None)
     ap.add_argument("--max_entries", type=int, default=None)
     ap.add_argument("--synthetic", action="store_true",
@@ -274,8 +393,9 @@ def build_parser() -> argparse.ArgumentParser:
 
 if __name__ == "__main__":
     args = build_parser().parse_args()
-    logging.basicConfig(level=logging.INFO)
+    # under torchrun only rank 0 logs progress; the other ranks report errors only
+    logging.basicConfig(level=logging.INFO if int(os.environ.get("RANK", "0")) == 0 else logging.ERROR)
     assert os.path.exists(args.template_config) and os.path.exists(args.configs_json)   # composite.py:246
     main(args.template_config, args.configs_json, args.unet_state_dict, args.conditioning, args.device,
          args.max_entries, args.synthetic, args.vae_state_dict, args.image_encoder_state_dict,
-         args.text_encoder_state_dict, args.tokenizer_dir)
+         args.text_encoder_state_dict, args.tokenizer_dir, args.encode_image_latents)

@@ -161,6 +161,18 @@ class PeerExchange:
             self.base = None
 
 
+def exchange_arena_mb(n_branches: int, n_frames: int, latent_h: int, latent_w: int, world: int) -> int:
+    """MiB of peer-exchange arena a composition of this geometry needs on each of `world` ranks.  Every temporal
+    operator of a forward bump-allocates two buffers of (tensor / P) bytes, about 60 tensors of the first level's
+    size (n_branches x n_frames x h x w x 320 channels, bf16); clamped to [4096, 32768].  MVOC_EXCHANGE_ARENA_MB,
+    when set, wins."""
+    env = os.environ.get("MVOC_EXCHANGE_ARENA_MB")
+    if env:
+        return int(env)
+    l0 = n_branches * n_frames * latent_h * latent_w * 320 * 2
+    return int(min(32768, max(4096, 60 * l0 / world / 2 ** 20)))
+
+
 class FrameParallel:
     def __init__(self, group=None, world: int = 1, rank: int = 0, device=None):
         self.group = group
@@ -175,7 +187,9 @@ class FrameParallel:
         return cls(None, 1, 0, device)
 
     @classmethod
-    def from_env(cls, device=None, backend: Optional[str] = None) -> "FrameParallel":
+    def from_env(cls, device=None, backend: Optional[str] = None, arena_mb: Optional[int] = None) -> "FrameParallel":
+        """The partition torchrun's environment describes.  The peer-exchange arena is `arena_mb` MiB
+        (exchange_arena_mb), or MVOC_EXCHANGE_ARENA_MB / 6144 when it is not given."""
         world = int(os.environ.get("WORLD_SIZE", "1"))
         if world == 1:
             return cls.single(device)
@@ -188,7 +202,7 @@ class FrameParallel:
         # MVOC_EXCHANGE=nccl keeps the NCCL all-to-all / all-gather exchange (the A/B baseline of bench.py)
         if (device is not None and torch.device(device).type == "cuda"
                 and os.environ.get("MVOC_EXCHANGE", "peer") != "nccl"):
-            mb = int(os.environ.get("MVOC_EXCHANGE_ARENA_MB", "6144"))
+            mb = arena_mb if arena_mb is not None else int(os.environ.get("MVOC_EXCHANGE_ARENA_MB", "6144"))
             fp.peer = PeerExchange(fp.group, fp.world, fp.rank, device, mb << 20)
         return fp
 
@@ -217,6 +231,14 @@ class FrameParallel:
     def barrier(self) -> None:
         if self.world > 1:
             dist.barrier(group=self.group)
+
+    def broadcast_module(self, module: torch.nn.Module, src: int = 0) -> None:
+        """Overwrite every parameter and buffer of `module` in place with rank `src`'s (random-init weights are
+        then the same on every rank, however much of its RNG each rank has drawn)."""
+        if self.world == 1:
+            return
+        for t in module.state_dict().values():
+            dist.broadcast(t, src=src, group=self.group)
 
     def max_over_ranks(self, value: float) -> float:
         if self.world == 1:

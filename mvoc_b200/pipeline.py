@@ -173,9 +173,11 @@ class I2VGenXLPipeline:
 
     def prepare_image_latents(self, image: torch.Tensor, num_frames: int,
                               generator: Optional[torch.Generator] = None) -> torch.Tensor:
-        """pipelines/pipeline_i2vgen_xl.py:860-890 (diffusers 0.27.2) at one video per prompt and guidance 1, the
-        only case inversion uses: image [1, 3, H, W] -> [1, 4, T, H/8, W/8] fp32.  Frame 0 is the encoded, scaled
-        image; frames 1..T-1 are constant planes i / (T - 1), the position mask of the later frames."""
+        """pipelines/pipeline_i2vgen_xl.py:860-890 (diffusers 0.27.2) at one video per prompt and guidance 1: images
+        [n, 3, H, W] -> [n, 4, T, H/8, W/8] fp32, one row per image (inversion passes one image, a composition the
+        first control frame of each branch).  Frame 0 is the encoded, scaled image; frames 1..T-1 are constant
+        planes i / (T - 1), the position mask of the later frames.  The posterior noise is one draw over the n
+        images (see _vae_latents)."""
         lat = self._vae_latents(image, generator).unsqueeze(2)
         if num_frames > 1:
             pos = torch.arange(1, num_frames, dtype=torch.float32, device=lat.device) / (num_frames - 1)

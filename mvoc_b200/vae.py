@@ -315,14 +315,15 @@ def frames_to_uint8(video: torch.Tensor) -> torch.Tensor:
     return (x * 255).round().to(torch.uint8).permute(1, 2, 3, 0).contiguous()
 
 
-def save_frames(video: torch.Tensor, out_dir: str) -> list:
-    """One RGB PNG per frame of a [3, T, H, W] video: out_dir/000.png, 001.png, ..."""
+def save_frames(video: torch.Tensor, out_dir: str, first_index: int = 0) -> list:
+    """One RGB PNG per frame of a [3, T, H, W] video: out_dir/000.png, 001.png, ...  The files are numbered from
+    `first_index`, so that a slice of a longer video keeps its frames' numbers."""
     from PIL import Image
 
     os.makedirs(out_dir, exist_ok=True)
     paths = []
     for i, frame in enumerate(frames_to_uint8(video).numpy()):
-        p = os.path.join(out_dir, f"{i:03d}.png")
+        p = os.path.join(out_dir, f"{first_index + i:03d}.png")
         Image.fromarray(frame).save(p)
         paths.append(p)
     return paths
